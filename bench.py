@@ -12,6 +12,7 @@ GPU) is measured in the same run and reported under the key "pma".  Other worklo
 (--workload sfma|sr|q) print their own line with the same schema.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload dynaq|pma|sfma|sr|q]
+                  [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  DESIGN.md "Measurement" documents every field.
 """
@@ -35,6 +36,7 @@ if ROOT not in sys.path:
 import numpy as np  # noqa: E402
 
 SEED = 0x5EED
+DUMP_BYTES = 60 * 1024 * 1024     # --dump-outputs: all arrays of one run together (under 64 MB with the .npy headers)
 
 # Workloads.  bytes_per_unit = algorithmic bytes per unit (SURVEY.md section 8d, DESIGN.md).
 WORKLOADS = {
@@ -414,6 +416,10 @@ class Job:
         tr = wl['trials']
         self.host_out = {'trial_steps': torch.empty((n_local, tr), dtype=torch.int32).pin_memory(),
                          'trial_reward': torch.empty((n_local, tr), dtype=torch.float64).pin_memory()}
+        # the agent's tables after train(): what a caller reads back (a compact SR agent's are not all reset per step)
+        a = self.agent
+        self.tables = (dict(SRc=a._SRc, visited=a._visited, n_visited=a._n_visited, rew=a._rewards, model=a._model)
+                       if name == 'sr100' else self.state)
         key = 'Q' if 'Q' in self.state else ('rew' if 'rew' in self.state else 'n_visited')
         self.out_key = key
         self.host_out[key] = torch.empty(self.state[key].shape, dtype=self.state[key].dtype).pin_memory()
@@ -447,6 +453,25 @@ class Job:
         self.host_out['trial_reward'].copy_(res['trial_reward'], non_blocking=True)
         return res
 
+    def outputs(self, res, budget):
+        """The result of one train() and the agent's tables, on the host as float32 / float64 (integers exactly), for
+        a fixed, seeded sample of this rank's agents sized to stay within ``budget`` bytes."""
+        torch = self.torch
+        n = self.stream.n_agents
+        arrs = {k: v for k, v in res.items() if torch.is_tensor(v)}
+        assert not set(arrs) & set(self.tables)
+        arrs.update(self.tables)
+        size = lambda v: 4 if v.dtype == torch.float32 else 8
+        per_agent = 8 + sum(v[0].numel() * size(v) for v in arrs.values())     # + the agent id
+        m = int(min(n, max(1, budget // per_agent)))
+        ids = np.sort(np.random.default_rng(SEED).choice(n, m, replace=False))
+        idx = torch.as_tensor(ids, device=self.dev)
+        out = {'agents': (ids + self.stream.agent_id_base).astype(np.float64)}
+        for k, v in arrs.items():
+            a = v.index_select(0, idx).cpu().numpy()
+            out[k] = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        return out
+
     def h2d_bytes(self):
         return sum(v.numel() * v.element_size() for v in list(self.host_in.values()) + list(self.host_big.values()) + [self.host_draws])
 
@@ -454,8 +479,9 @@ class Job:
         return sum(v.numel() * v.element_size() for v in self.host_out.values())
 
 
-def measure(job, k, warmup, cdist, dev, flush, e2e=True, n_total=None):
-    """Returns dict(ms kernel-only, ms e2e, per-rank units of one step, launches, wall)."""
+def measure(job, k, warmup, cdist, dev, flush, e2e=True, n_total=None, dump_budget=0):
+    """Returns dict(ms kernel-only, ms e2e, per-rank units of one step, launches, wall), and with ``dump_budget`` the
+    outputs of the last timed kernel-only step (``Job.outputs``)."""
     import torch
     from cobel_rl_b200 import _lib
     L = _lib.lib()
@@ -499,6 +525,8 @@ def measure(job, k, warmup, cdist, dev, flush, e2e=True, n_total=None):
         WORKLOADS['sfma'] = job.wl
     out = {'ms': sum(ms) / len(ms), 'wall': wall, 'units': units, 'launches': int(launches), 'res': res,
            'steps_units': float(res['n_steps'].sum().item()), 'replay_units': float(res['n_replay'].sum().item())}
+    if dump_budget:
+        out['outputs'] = job.outputs(res, dump_budget)        # before the end-to-end steps overwrite the tables
     if e2e:
         for _ in range(2):
             job.step_e2e()
@@ -575,7 +603,7 @@ def run_ours(args):
     names = [args.workload]
     if args.workload == 'dynaq' and not args.no_pma:
         names += ['pma'] if args.extras == 'pma' else (EXTRAS if args.extras == 'all' else [])
-    blocks, head_clocks = {}, None
+    blocks, head_clocks, dumps = {}, None, {}
     for name in names:
         wl = WORKLOADS[name]
         if wl.get('scaling') == 'strong':
@@ -603,8 +631,10 @@ def run_ours(args):
         sampler = ClockSampler(local)
         if rank == 0:
             sampler.start()
-        k = args.steps if name == names[0] else max(3, min(args.steps, 5))
-        m = measure(job, k, args.warmup, cdist, dev, flush, n_total=n_total if world > 1 else None)
+        m = measure(job, args.steps, args.warmup, cdist, dev, flush, n_total=n_total if world > 1 else None,
+                    dump_budget=DUMP_BYTES // len(names) if args.dump_outputs and rank == 0 else 0)
+        if 'outputs' in m:
+            dumps[name] = m['outputs']
         clocks = sampler.stop() if rank == 0 else None
         if name == names[0]:
             head_clocks = clocks
@@ -630,6 +660,11 @@ def run_ours(args):
         torch.cuda.empty_cache()
     if rank != 0:
         return
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arrs in dumps.items():
+            for k, a in arrs.items():
+                np.save(os.path.join(args.dump_outputs, '%s_%s.npy' % (name, k)), a)
     head = blocks[names[0]]
     out = {
         'metric': head['metric'], 'value': head['value'], 'unit': head['unit'], 'n_gpus': world,
@@ -656,7 +691,7 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=10)
+    ap.add_argument('--steps', type=int, default=10, help='timed steps of every workload')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--workload', default='dynaq', choices=sorted(WORKLOADS))
@@ -667,7 +702,12 @@ def main():
                     help='extra workloads reported under their own keys next to the Dyna-Q headline: all = PMA (the second '
                          'headline metric), Dyna-Q at 65536 agents, QAgent, dense SR, SFMA C4, compact SR C5')
     ap.add_argument('--profile-one', action='store_true', help='one step between cudaProfilerStart/Stop, for ncu')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step of each workload computed as DIR/<workload>_<name>.npy '
+                         '(float32 / float64; a fixed, seeded sample of the agents of rank 0, at most 64 MB in all)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.agents:
         for w in WORKLOADS.values():
             w['agents_per_gpu'] = args.agents

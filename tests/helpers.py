@@ -25,6 +25,115 @@ def load_golden(name):
         return {k: z[k] for k in z.files}
 
 
+# --------------------------------------------------------------------------- #
+# recorded values of the parity checks against the reference
+# --------------------------------------------------------------------------- #
+# The reference sources are not part of this repository.  Its tests/test_oracle_vs_reference.py and the reference
+# comparisons of the *_cpu tests therefore check against values stored under tests/golden/: whole records as arrays
+# (recorded_records.npz) and everything else in a canonical JSON form (recorded_values.json).
+#
+# Provenance: these values were NOT produced by the reference.  They were recorded (COBEL_RECORD_REFERENCE=ours) from
+# this repository's own oracle and product code at commit 0d657d9, whose oracle/ and product code are identical to
+# commit b46dadc, where the same comparisons ran live against the unmodified reference and passed.  They are believed
+# equal to what the reference returns but were never checked against it; until they are re-recorded from the reference
+# (COBEL_RECORD_REFERENCE=reference, with its sources importable through oracle/ref_loader.py) they guard against
+# changes of this repository's results, not against a divergence from the reference that already existed.
+# Whenever the reference sources are importable the tests also compare the live reference with the stored values.
+RECORDED_RECORDS = os.path.join(GOLDEN, 'recorded_records.npz')
+RECORDED_VALUES = os.path.join(GOLDEN, 'recorded_values.json')
+_RECORD = os.environ.get('COBEL_RECORD_REFERENCE')
+assert _RECORD in (None, 'reference', 'ours'), _RECORD
+_INLINE = 256         # canonical forms longer than this (JSON characters) are stored as their SHA-256
+
+
+def _reference_live():
+    from oracle import ref_loader
+    return ref_loader.available()
+
+
+def _canonical(x):
+    """JSON form of ``x`` under which equal forms mean ``==`` in Python: numbers as floats (0 == 0.0 == False),
+    arrays with their dtype and shape, tuples apart from lists, dict items sorted (their order does not count)."""
+    import json
+    if hasattr(x, 'detach'):            # a torch tensor
+        x = x.detach().cpu().numpy()
+    if isinstance(x, np.ndarray):
+        return {'ndarray': x.dtype.str, 'shape': list(x.shape), 'values': _canonical(x.ravel().tolist())}
+    if isinstance(x, np.generic):
+        x = x.item()
+    if isinstance(x, (bool, int, float)):
+        return float(x)
+    if isinstance(x, dict):
+        items = [(json.dumps(_canonical(k), sort_keys=True), _canonical(v)) for k, v in x.items()]
+        return {'dict': sorted(items, key=lambda kv: kv[0])}
+    if isinstance(x, tuple):
+        return {'tuple': [_canonical(v) for v in x]}
+    if isinstance(x, list):
+        return [_canonical(v) for v in x]
+    assert x is None or isinstance(x, str), type(x)
+    return x
+
+
+def _stored_form(x):
+    """The canonical form of ``x`` if short, else its SHA-256 with the array dtype / shape or container length."""
+    import hashlib
+    import json
+    c = _canonical(x)
+    text = json.dumps(c, sort_keys=True)
+    if len(text) <= _INLINE:
+        return c
+    out = {'sha256': hashlib.sha256(text.encode()).hexdigest()}
+    if isinstance(c, dict) and 'ndarray' in c:
+        out.update(ndarray=c['ndarray'], shape=c['shape'])
+    elif isinstance(c, dict):
+        out['len'] = len(next(iter(c.values())))
+    elif isinstance(c, list):
+        out['len'] = len(c)
+    return out
+
+
+def world_form(world):
+    """A WorldDict as the reference builds it: without the product's successor table ``succ``, and with
+    ``invalid_transitions`` as the sorted list of pairs (make_gridworld only tests membership)."""
+    w = {k: v for k, v in world.items() if k != 'succ'}
+    w['invalid_transitions'] = sorted((int(s), int(t)) for s, t in w['invalid_transitions'])
+    return w
+
+
+def check_stored(label, ours, live=None):
+    """``ours`` equals the value recorded for ``label`` (see the provenance above); ``live()`` is the same call of the
+    reference, compared with the recorded value when the reference sources are importable."""
+    import json
+    stored = json.load(open(RECORDED_VALUES)) if os.path.exists(RECORDED_VALUES) else {}
+    if _RECORD:
+        stored[label] = _stored_form(live() if _RECORD == 'reference' else ours)
+        with open(RECORDED_VALUES, 'w') as f:         # one label per line
+            f.write('{\n%s\n}\n' % ',\n'.join('%s: %s' % (json.dumps(k), json.dumps(v, sort_keys=True, separators=(',', ':')))
+                                              for k, v in sorted(stored.items())))
+        return
+    assert label in stored, 'no recorded value for %s' % label
+    for who, value in [('ours', ours)] + ([('live reference', live())] if live is not None and _reference_live() else []):
+        got = json.loads(json.dumps(_stored_form(value)))
+        assert got == stored[label], '%s: %s gives %.400s; recorded: %.400s' % (label, who, got, stored[label])
+
+
+def check_stored_record(case, got, keys, live=None, rtol=None):
+    """``got`` equals the arrays (e.g. trajectory, replay, tables, draws) recorded for ``case`` field by field over
+    ``keys`` (see assert_equal_records and the provenance above); ``live()`` reruns the case in the reference."""
+    stored = load_golden('recorded_records') if os.path.exists(RECORDED_RECORDS) else {}
+    if _RECORD:
+        rec = live() if _RECORD == 'reference' else got
+        stored = {k: v for k, v in stored.items() if not k.startswith(case + '__')}
+        stored.update({'%s__%s' % (case, k): np.asarray(rec[k]) for k in keys})
+        np.savez_compressed(RECORDED_RECORDS, **stored)
+        return
+    want = {k[len(case) + 2:]: v for k, v in stored.items() if k.startswith(case + '__')}
+    assert want, 'no recorded record for %s' % case
+    assert_equal_records(got, want, keys, rtol=rtol, what=case)
+    if live is not None and _reference_live():
+        assert_equal_records(live(), want, keys, rtol=rtol, what='live reference, ' + case)
+
+
 def make_world(name, tools=None):
     """WorldDict of a named case world, built with the product's builder by default."""
     if tools is None:

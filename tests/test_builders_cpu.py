@@ -1,10 +1,13 @@
-"""CPU (build container only: needs /root/reference): the product's world / graph builders produce
-exactly the reference's WorldDicts and node dictionaries (keys, dtypes, values, neighbour order)."""
+"""CPU: the product's world / graph builders produce exactly the reference's WorldDicts and node dictionaries (keys,
+dtypes, values, neighbour order).  The comparison is with values recorded from this repository's builders, which matched
+the reference when it was last run live; see the provenance note in tests/helpers.py.  With the reference sources
+present its builders are called live as well."""
 import numpy as np
 import pytest
 
 from cobel_rl_b200.misc import gridworld_tools as mg, topology_tools as mt
 from cobel_rl_b200.memory.utils import metrics as mm
+from helpers import check_stored, check_stored_record, world_form
 
 WALLS = [(1, 2), (2, 1), (6, 7), (7, 6), (11, 12), (12, 11), (13, 8), (8, 13)]
 
@@ -18,58 +21,59 @@ def same_world(a, b):
             assert x == y, (k, x, y)
 
 
-def test_gridworld_builders(reference):
-    from cobel.misc import gridworld_tools as rg
+def check_builder(module, fn, *args, **kw):
+    """``module.fn(*args, **kw)`` of the product against the same builder of the reference (``module`` names both)."""
+    def live():
+        import importlib
+        from oracle import ref_loader
+        ref_loader.load()
+        return getattr(importlib.import_module('cobel.misc.' + module), fn)(*args, **kw)
+    ours = getattr({'gridworld_tools': mg, 'topology_tools': mt}[module], fn)(*args, **kw)
+    label = '%s.%s%r%s' % (module, fn, args, ('' if not kw else ' ' + repr(sorted(kw.items()))))
+    if module == 'gridworld_tools':
+        check_stored(label, world_form(ours), lambda: world_form(live()))
+    else:
+        check_stored(label, ours, live)
+    return ours
+
+
+def test_gridworld_builders():
     kw = dict(terminals=[4], rewards=np.array([[4, 10]]), goals=[4], starting_states=[12], invalid_transitions=WALLS)
-    same_world(mg.make_gridworld(5, 5, **kw), rg.make_gridworld(5, 5, **kw))
-    same_world(mg.make_open_field(7, 4, 3, 2.5), rg.make_open_field(7, 4, 3, 2.5))
-    same_world(mg.make_empty_field(3, 6), rg.make_empty_field(3, 6))
+    check_builder('gridworld_tools', 'make_gridworld', 5, 5, **kw)
+    check_builder('gridworld_tools', 'make_open_field', 7, 4, 3, 2.5)
+    check_builder('gridworld_tools', 'make_empty_field', 3, 6)
     cols = np.array([0, 0, 0, 1, 1, 1, 2, 2, 1, 0])
-    same_world(mg.make_windy_gridworld(7, 10, cols, 37, 1., 'up'), rg.make_windy_gridworld(7, 10, cols, 37, 1., 'up'))
-    same_world(mg.make_windy_gridworld(7, 10, cols, 37, 1., 'down'), rg.make_windy_gridworld(7, 10, cols, 37, 1., 'down'))
-    same_world(mg.make_gridworld(6, 6, invalid_states=[7, 8, 20]), rg.make_gridworld(6, 6, invalid_states=[7, 8, 20]))
+    check_builder('gridworld_tools', 'make_windy_gridworld', 7, 10, cols, 37, 1., 'up')
+    check_builder('gridworld_tools', 'make_windy_gridworld', 7, 10, cols, 37, 1., 'down')
+    check_builder('gridworld_tools', 'make_gridworld', 6, 6, invalid_states=[7, 8, 20])
     big = mg.make_open_field(100, 100, 0, 1, dense_sas=False)
     assert big['sas'] is None and big['succ'].shape == (10000, 4)
 
 
-def same_maze(a, b):
-    """Like same_world, with `invalid_transitions` compared as the set it is (make_gridworld only tests membership)."""
-    for k in b:
-        x, y = a[k], b[k]
-        if k == 'invalid_transitions':
-            as_set = lambda w: {(int(s), int(t)) for s, t in w}
-            assert as_set(x) == as_set(y) and len(x) == len(y)
-        elif isinstance(y, np.ndarray):
-            assert x.dtype == y.dtype and np.array_equal(x, y), k
-        else:
-            assert x == y, (k, x, y)
-
-
-def test_maze_templates(reference):
-    from cobel.misc import gridworld_tools as rg
+def test_maze_templates():
+    # (world_form compares invalid_transitions as the sorted list of pairs: make_gridworld only tests membership)
     for stem in (1, 2, 3, 4):
         for arm in (1, 2, 3):
             for goal in ('left', 'right'):
-                same_maze(mg.make_t_maze(stem, arm, goal, 2.5), rg.make_t_maze(stem, arm, goal, 2.5))
+                check_builder('gridworld_tools', 'make_t_maze', stem, arm, goal, 2.5)
             for goal in ('left-left', 'left-right', 'right-left', 'right-right'):
-                same_maze(mg.make_double_t_maze(stem, arm, goal), rg.make_double_t_maze(stem, arm, goal))
-                same_maze(mg.make_two_sided_t_maze(stem, arm, goal), rg.make_two_sided_t_maze(stem, arm, goal))
+                check_builder('gridworld_tools', 'make_double_t_maze', stem, arm, goal)
+                check_builder('gridworld_tools', 'make_two_sided_t_maze', stem, arm, goal)
     for ch in (1, 2, 3, 4, 5):
         for lw in (1, 2, 3):
             for goal in ('left', 'right'):
-                same_maze(mg.make_8_maze(ch, lw, goal, 3.0), rg.make_8_maze(ch, lw, goal, 3.0))
+                check_builder('gridworld_tools', 'make_8_maze', ch, lw, goal, 3.0)
     for ch in (3, 4, 5, 6):
         for lw, arm in ((3, 1), (4, 1), (5, 2), (7, 2), (7, 3)):
             for chirality in ('left', 'right'):
                 for goal in ('left', 'right'):
-                    same_maze(mg.make_two_choice_t_maze(ch, lw, arm, chirality, goal, 2.0),
-                              rg.make_two_choice_t_maze(ch, lw, arm, chirality, goal, 2.0))
+                    check_builder('gridworld_tools', 'make_two_choice_t_maze', ch, lw, arm, chirality, goal, 2.0)
     for ws, hs, dw, dh in ((1, 1, 1, 1), (2, 2, 2, 1), (1, 3, 4, 2), (3, 2, 1, 3)):
-        same_maze(mg.make_detour_maze(ws, hs, ws + dw, hs + dh, 2.0), rg.make_detour_maze(ws, hs, ws + dw, hs + dh, 2.0))
+        check_builder('gridworld_tools', 'make_detour_maze', ws, hs, ws + dw, hs + dh, 2.0)
     for arm in (1, 2, 3, 4):
         for aw in (1, 2, 3):
             for goal in ('left', 'top', 'right', 'bottom'):
-                same_maze(mg.make_cross_maze(arm, aw, goal, 2.0), rg.make_cross_maze(arm, aw, goal, 2.0))
+                check_builder('gridworld_tools', 'make_cross_maze', arm, aw, goal, 2.0)
 
 
 def test_maze_templates_known_answers():
@@ -101,36 +105,40 @@ def test_maze_templates_known_answers():
     assert len(x['invalid_transitions']) == 32 and x['rewards'][12] == 1 and x['terminals'][18] == 1
 
 
-def test_topology_builders(reference):
-    from cobel.misc import topology_tools as rt
+def test_topology_builders():
     for args in [(10, 2, 1.0, 20., 'right'), (5, 1, 0.5, 1., 'left'), (4, 3)]:
-        assert mt.linear_track(*args) == rt.linear_track(*args), args
+        check_builder('topology_tools', 'linear_track', *args)
     for args in [(5,), ((3, 4),), (4, (0., 2.), 3., '5'), ((2, 5), ((0., 1.), (1., 3.)))]:
-        assert mt.grid(*args) == rt.grid(*args), args
+        check_builder('topology_tools', 'grid', *args)
     for args in [(4, 3, 1), (6, 3, 2), (2, 2, 3, 0.5, 2., 'left')]:
-        assert mt.t_maze(*args) == rt.t_maze(*args), args
+        check_builder('topology_tools', 't_maze', *args)
     for args in [(10,), (6,), (5, (0., 2.), 3., '7'), (2,), (9, (1.0, 4.0))]:
-        assert mt.hexagonal(*args) == rt.hexagonal(*args), args
+        check_builder('topology_tools', 'hexagonal', *args)
     for args in [(3, 1), (2, 2, 0.5, 30.0), (4, 3, 2.0, 90.0), (1, 1)]:
-        assert mt.cross(*args) == rt.cross(*args), args
+        check_builder('topology_tools', 'cross', *args)
 
 
-def test_metrics(reference):
-    from cobel.memory.utils import metrics as rm
-    from cobel.misc import gridworld_tools as rg
-    world = rg.make_gridworld(5, 5, terminals=[4], invalid_transitions=WALLS)
-    np.testing.assert_array_equal(mm.DR(5, 5, world['sas'], 0.9, WALLS).D, rm.DR(5, 5, world['sas'], 0.9, WALLS).D)
-    np.testing.assert_array_equal(mm.DR(5, 5, world['sas'], 0.9, []).D, rm.DR(5, 5, world['sas'], 0.9, []).D)
-    np.testing.assert_array_equal(mm.SR(world['sas'], 0.8).D, rm.SR(world['sas'], 0.8).D)
-    np.testing.assert_allclose(mm.Euclidean(4, 3).D, rm.Euclidean(4, 3).D, rtol=1e-15)
+def test_metrics():
+    world = mg.make_gridworld(5, 5, terminals=[4], invalid_transitions=WALLS)
+
+    def matrices(m):
+        return {'DR_walls': m.DR(5, 5, world['sas'], 0.9, WALLS).D, 'DR_open': m.DR(5, 5, world['sas'], 0.9, []).D,
+                'SR': m.SR(world['sas'], 0.8).D, 'Euclidean': m.Euclidean(4, 3).D}
+
+    def live():
+        from oracle import ref_loader
+        return matrices(ref_loader.load().memory.utils.metrics)
+    ours = matrices(mm)
+    check_stored_record('metrics', ours, ['DR_walls', 'DR_open', 'SR'], live)
+    check_stored_record('metrics_euclidean', ours, ['Euclidean'], live, rtol={'Euclidean': 1e-15})
 
 
-def test_pickled_world_round_trip(reference, tmp_path):
+def test_pickled_world_round_trip(tmp_path):
     """The gridworld editor's file format (misc/gridworld_gui.py:203-239: a pickled WorldDict)."""
     import pickle
-    from cobel.misc import gridworld_tools as rg
     from cobel_rl_b200.interface.gridworld import successor_table
-    ref_world = rg.make_t_maze(3, 2)                 # as the reference's editor would have saved it (no 'succ' key)
+    ref_world = check_builder('gridworld_tools', 'make_t_maze', 3, 2)
+    ref_world = {k: v for k, v in ref_world.items() if k != 'succ'}     # as the reference's editor saved it
     path = tmp_path / 'maze.pkl'
     with open(path, 'wb') as f:
         pickle.dump(ref_world, f)

@@ -1,20 +1,38 @@
-"""CPU: host logic of the batched grid-search back-end and the monitors (no GPU needed)."""
+"""CPU: host logic of the batched grid-search back-end and the monitors (no GPU needed).  The comparisons with the
+reference check against values recorded from this repository's code, which matched the reference when it was last run
+live; see the provenance note in tests/helpers.py.  With the reference sources present the reference runs live too."""
 import numpy as np
 import pytest
 import torch
 
 from cobel_rl_b200.monitor import EscapeLatencyMonitor, RewardMonitor
 from cobel_rl_b200.optimizer import EAOptimizer, GridSearchOptimizer
+from helpers import check_stored
+
+
+def _reference(module):
+    import importlib
+    from oracle import ref_loader
+    ref_loader.load()
+    return importlib.import_module('cobel.' + module)
+
+
+def _f64(xs):
+    """Arrays compared by value (np.array_equal), whatever their dtype."""
+    return [np.asarray(x, dtype=np.float64) for x in xs]
 
 PARAMS = {'x_1': [0, 1, 2, 3, 4], 'x_2': [0., 0.1, 0.2, 0.3, 0.4], 'x_3': np.array([0.9, 0.5, 0.6, 0.7, 0.8])}
 
 
 @pytest.mark.parametrize('order', ['nested', 'systematic'])
-def test_parameter_combinations_match_reference(order, reference, tmp_path):
-    from cobel.optimizer import GridSearchOptimizer as Ref
+def test_parameter_combinations_match_reference(order, tmp_path):
+    def live():
+        ref = _reference('optimizer').GridSearchOptimizer(str(tmp_path) + '/', PARAMS, 2, order,
+                                                          rng=np.random.default_rng(4))
+        return list(ref.parameter_combinations.items())
     ours = GridSearchOptimizer(str(tmp_path) + '/', PARAMS, 2, order, rng=np.random.default_rng(4))
-    ref = Ref(str(tmp_path) + '/', PARAMS, 2, order, rng=np.random.default_rng(4))
-    assert list(ours.parameter_combinations.items()) == list(ref.parameter_combinations.items())
+    check_stored('GridSearchOptimizer.parameter_combinations %s' % order, list(ours.parameter_combinations.items()),
+                    live)
 
 
 def test_shuffled_order_is_a_permutation(tmp_path):
@@ -76,35 +94,41 @@ def test_ea_optimizer_reference_constructor_cannot_run(reference, tmp_path):
         Ref(str(tmp_path) + '/', _ea_params(np.random.default_rng(0)), 1, 1, np.random.default_rng(0))
 
 
-def test_ea_optimizer_matches_reference_fit_method(reference, tmp_path):
+def test_ea_optimizer_matches_reference_fit_method(tmp_path):
     """The reference's unmodified ``fit`` (on an object whose constructor is bypassed) against the batched back-end
     in ``bookkeeping='reference'`` mode: same run_<r>.pkl files, same returned fit, same rng consumption."""
     import os
     import pickle
-    from cobel.optimizer.evolution import EAOptimizer as Ref
     d_ref, d_our = str(tmp_path) + '/ref/', str(tmp_path) + '/our/'
     os.makedirs(d_ref); os.makedirs(d_our)
-    rng_ref, rng_our = np.random.default_rng(11), np.random.default_rng(11)
-    ref = object.__new__(Ref)
-    import copy
-    ref.parameters = copy.deepcopy(_ea_params(rng_ref))      # evolution.py:65 (a bound mutator gets its own copy of the generator)
-    for p in ref.parameters.values():               # what evolution.py:68-72 would have filled in
-        p.setdefault('init_range', {'low': -1, 'high': 1})
-        p.setdefault('param_range', {'a_min': None, 'a_max': None})
-    ref.file_path, ref.nb_runs, ref.population_size, ref.rng, ref.present_files = d_ref, 2, 3, rng_ref, []
+
+    def outcome(fit, d, rng):
+        return fit, [pickle.load(open(d + 'run_%d.pkl' % r, 'rb')) for r in range(2)], rng.uniform()
+
+    def live():
+        import copy
+        rng_ref = np.random.default_rng(11)
+        ref = object.__new__(_reference('optimizer.evolution').EAOptimizer)
+        ref.parameters = copy.deepcopy(_ea_params(rng_ref))      # evolution.py:65 (a bound mutator gets its own copy of the generator)
+        for p in ref.parameters.values():               # what evolution.py:68-72 would have filled in
+            p.setdefault('init_range', {'low': -1, 'high': 1})
+            p.setdefault('param_range', {'a_min': None, 'a_max': None})
+        ref.file_path, ref.nb_runs, ref.population_size, ref.rng, ref.present_files = d_ref, 2, 3, rng_ref, []
+        f_ref = ref.fit(lambda task, ind: ind['a'] * task['x'] + ind['b'], EA_TASKS, EA_DATA, _ea_loss, generations=6,
+                        individuals=5)
+        return outcome(f_ref, d_ref, rng_ref)
     calls = []
-    f_ref = ref.fit(lambda task, ind: ind['a'] * task['x'] + ind['b'], EA_TASKS, EA_DATA, _ea_loss, generations=6, individuals=5)
 
     def sim_batch(task, params):
         calls.append(len(params['_run']))
         return params['a'] * task['x'] + params['b']
+    rng_our = np.random.default_rng(11)
     ours = EAOptimizer(d_our, _ea_params(rng_our), 2, 3, rng_our, bookkeeping='reference')
     f_our = ours.fit(sim_batch, EA_TASKS, EA_DATA, _ea_loss, generations=6, individuals=5)
-    assert f_our == f_ref and len(f_ref) >= 1
+    assert len(f_our) >= 1
     assert calls == [5 * 3] * (2 * 6 * 2)            # one batched call per task and generation: individuals x repetitions
-    for r in range(2):
-        assert pickle.load(open(d_our + 'run_%d.pkl' % r, 'rb')) == pickle.load(open(d_ref + 'run_%d.pkl' % r, 'rb'))
-    assert rng_our.uniform() == rng_ref.uniform()    # same number of draws consumed
+    # same fit, same run_<r>.pkl contents, same number of draws consumed (the next uniform)
+    check_stored('EAOptimizer.fit reference bookkeeping', outcome(f_our, d_our, rng_our), live)
 
 
 def test_ea_optimizer_intended_bookkeeping_converges_and_resumes(tmp_path):
@@ -137,20 +161,25 @@ def test_monitors_from_callbacks_and_results():
     assert single.get_trace().tolist() == [0, 7]
 
 
-def test_response_and_q_monitors_match_reference(reference):
+def test_response_and_q_monitors_match_reference():
     """monitor/behavior.py:212-301, 388-464: same traces as the reference's monitors fed the same logs."""
-    import importlib
     import numpy as np
     from cobel_rl_b200.monitor import QMonitor, ResponseMonitor
-    rb = importlib.import_module('cobel.monitor.behavior')
     rewards = [0.0, 1.0, 0.0, 2.5, 0.0, 1.0]
-    ref, mine = rb.ResponseMonitor(6), ResponseMonitor(6)
-    for t, r in enumerate(rewards):
-        logs = {'trial': t, 'trial_reward': r}
-        if t == 4:
-            logs['response'] = 3
-        ref.update(dict(logs)); mine.update(dict(logs))
-    assert np.array_equal(ref.get_trace(), mine.get_trace()) and np.array_equal(ref.CRC, mine.get_cumulative())
+
+    def feed(m):
+        for t, r in enumerate(rewards):
+            logs = {'trial': t, 'trial_reward': r}
+            if t == 4:
+                logs['response'] = 3
+            m.update(dict(logs))
+        return m
+
+    def live_response():
+        ref = feed(_reference('monitor.behavior').ResponseMonitor(6))
+        return _f64([ref.get_trace(), ref.CRC])
+    mine = feed(ResponseMonitor(6))
+    check_stored('ResponseMonitor trace, cumulative', _f64([mine.get_trace(), mine.get_cumulative()]), live_response)
 
     class _Agent:
         def __init__(self):
@@ -159,11 +188,14 @@ def test_response_and_q_monitors_match_reference(reference):
         def predict_on_batch(self, batch):
             self.k += 1
             return np.arange(len(batch) * 4, dtype=float).reshape(len(batch), 4) * self.k
-    a1, a2 = _Agent(), _Agent()
-    ref, mine = rb.QMonitor(3, [0, 2, 5]), QMonitor(3, [0, 2, 5])
-    for t in range(3):
-        ref.update({'trial': t, 'agent': a1}); mine.update({'trial': t, 'agent': a2})
-    assert all(np.array_equal(x, y) for x, y in zip(ref.get_trace(), mine.get_trace())) and len(mine.get_trace()) == 3
+    def q_trace(m):
+        a = _Agent()
+        for t in range(3):
+            m.update({'trial': t, 'agent': a})
+        return _f64(m.get_trace())
+    mine = q_trace(QMonitor(3, [0, 2, 5]))
+    assert len(mine) == 3
+    check_stored('QMonitor trace', mine, lambda: q_trace(_reference('monitor.behavior').QMonitor(3, [0, 2, 5])))
     # batched response monitor: one row per agent
     m = ResponseMonitor(3, n_agents=2)
     for t, r in enumerate(([0.0, 1.0], [2.0, 0.0], [0.0, 0.0])):
@@ -171,13 +203,11 @@ def test_response_and_q_monitors_match_reference(reference):
     assert np.array_equal(m.get_trace(), [[0, 1, 0], [1, 0, 0]]) and np.array_equal(m.get_cumulative(), [[0, 1, 1], [1, 1, 1]])
 
 
-def test_occupancy_map_and_match(reference):
+def test_occupancy_map_and_match():
     """analysis/behavior_spatial.py:9-111 against the reference over random inputs, plus known answers."""
-    import importlib
     import numpy as np
     import torch
     from cobel_rl_b200.analysis import get_occupancy_map, match
-    ra = importlib.import_module('cobel.analysis.behavior_spatial')
     rs = np.random.default_rng(0)
     for k in range(120):
         w, h = rs.uniform(1, 6, 2)
@@ -186,12 +216,12 @@ def test_occupancy_map_and_match(reference):
             b, w, h = [0.5, 1.0, 0.25][k % 3], float(int(w) + 1), float(int(h) + 1)
         margins = ['expand', 'include', 'ignore'][k % 3]
         trajs = [np.round(rs.uniform(0, max(w, h) + 0.5, (int(rs.integers(1, 30)), 2)), 1 if k % 2 else 6) for _ in range(3)]
-        want = ra.get_occupancy_map(trajs, w, h, b, margins)
-        got = get_occupancy_map(trajs, w, h, b, margins).numpy()
-        assert got.shape == want.shape and np.array_equal(got, want), (k, w, h, b, margins)
+        live = lambda: _f64([_reference('analysis.behavior_spatial').get_occupancy_map(trajs, w, h, b, margins)])
+        check_stored('get_occupancy_map %d' % k, _f64([get_occupancy_map(trajs, w, h, b, margins).numpy()]), live)
     for k in range(60):
         seq, tpl = rs.integers(0, 4, int(rs.integers(1, 20))), rs.integers(0, 4, int(rs.integers(1, 8)))
-        assert np.array_equal(ra.match(seq, tpl), match(seq, tpl))
+        check_stored('match %d' % k, _f64([match(seq, tpl)]),
+                        lambda: _f64([_reference('analysis.behavior_spatial').match(seq, tpl)]))
     # a NaN-padded [N, T, 2] tensor gives the same map as the list of its valid rows
     pos = torch.tensor([[[0.5, 0.5], [1.5, 0.5], [float('nan')] * 2], [[0.5, 1.5], [0.5, 1.5], [1.5, 1.5]]], dtype=torch.float64)
     occ = get_occupancy_map(pos, 2.0, 2.0, 1.0)

@@ -16,5 +16,6 @@ def test_oracle_matches_golden(name):
         keys += ['test_states', 'test_actions', 'test_trial_steps', 'test_trial_reward', 'draws_after_test']
     if 'modes' in want:          # SFMA dynamic mode: the per-trial replay modes and the TD accumulator
         keys += ['modes', 'td']
-    # same NumPy / LAPACK on both sides in this image: even PMA's SR is bit-equal
-    assert_equal_records(got, want, keys, what=name)
+    # PMA's SR = inv(I - gamma T) comes from LAPACK on both sides, whose kernels (and last bits) depend on the host
+    # CPU: SR within the norm-wise bound of tests/test_pma_gpu.py, everything else (trajectory, replay, Q, T) bit-equal
+    assert_equal_records(got, want, keys, rtol={'SR': 1e-12}, what=name)
