@@ -137,10 +137,10 @@ COBEL_DEV double np_sum(const double (&x)[A]) {
 }
 
 // ---------------------------------------------------------------------------
-// Host-side error plumbing shared by the entry points.
+// Host-side plumbing shared by the entry points: errors, the action-count dispatch, kernel launches.
 // ---------------------------------------------------------------------------
 void cobel_set_error(const char* fmt, ...);
-void cobel_count_launch(int n = 1);
+void cobel_count_launch();
 #define COBEL_REQUIRE(cond, code, ...)                 \
   do {                                                 \
     if (!(cond)) { cobel_set_error(__VA_ARGS__); return (code); } \
@@ -153,3 +153,34 @@ void cobel_count_launch(int n = 1);
       return COBEL_ECUDA;                                                          \
     }                                                                              \
   } while (0)
+
+// Runs CALL with `constexpr int A` = A_ for the action counts the kernels are built for.
+#define COBEL_DISPATCH_A(A_, CALL)                                                                       \
+  switch (A_) {                                                                                          \
+    case 2: { constexpr int A = 2; CALL; } break;                                                        \
+    case 3: { constexpr int A = 3; CALL; } break;                                                        \
+    case 4: { constexpr int A = 4; CALL; } break;                                                        \
+    case 6: { constexpr int A = 6; CALL; } break;                                                        \
+    case 8: { constexpr int A = 8; CALL; } break;                                                        \
+    default: cobel_set_error("unsupported number of actions %d (built for 2,3,4,6,8)", (int)(A_)); return COBEL_EUNSUPPORTED; \
+  }
+
+// Largest dynamic shared memory of one block on sm_100 (227 KB).
+constexpr int kMaxSmem = 227 * 1024;
+
+// One kernel launch: raises the kernel's dynamic shared-memory limit to `smem`, launches, counts the launch and
+// reports a launch error as COBEL_ECUDA.
+template <typename... Params, typename... Args>
+int launch_kernel(void (*kernel)(Params...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, const Args&... args) {
+  COBEL_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kernel<<<grid, block, smem, st>>>(args...);
+  cobel_count_launch();
+  COBEL_CUDA_OK(cudaGetLastError());
+  return COBEL_OK;
+}
+
+// Checks shared by the fused train()/test() entry points (util.cu).
+int cobel_validate_common(int64_t n_agents, const CobelWorld& w, const CobelStream& s, const CobelPolicy& pol,
+                          const CobelTrace& tr, int trials, int steps);
+// carry[n, 0] = state[n], carry[n, 1..stride) = 0: the per-agent state a stand-alone replay starts from (util.cu).
+int cobel_set_carry(int64_t* carry, int stride, const int32_t* state, int64_t n_agents, cudaStream_t st);

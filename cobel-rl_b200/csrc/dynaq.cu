@@ -15,7 +15,6 @@
 //     sequential 32-update chain collapses to about five rounds with bit-identical results.
 // (v1 of this kernel used one thread per agent: 180 warp-instructions per update at one
 //  instruction per 5 cycles, profiles/r1_dynaq_v1_thread_per_agent.txt.)
-#include <cstdlib>
 #include "warp_agent.cuh"
 
 namespace {
@@ -453,67 +452,34 @@ int launch(const CobelDynaQParams& p, cudaStream_t st) {
                      p.batch == 32 && !p.stream.user_stream;
   const AgentSmem ao(S, A, plain);
   const size_t sm = (size_t)wo.bytes + (size_t)kWarpsPerCta * ao.bytes;
-  if (sm > 227 * 1024) {
+  if (sm > kMaxSmem) {
     // the tables do not fit: they stay in HBM / L2, only the dependency masks of the replay are staged
     const AgentSmem go(S, A, false, false);
     int warps = kWarpsPerCta;
-    while (warps > 1 && (size_t)warps * go.bytes > 227 * 1024) warps >>= 1;
+    while (warps > 1 && (size_t)warps * go.bytes > kMaxSmem) warps >>= 1;
     const size_t smg = (size_t)warps * go.bytes;
-    COBEL_REQUIRE(smg <= 227 * 1024, COBEL_EUNSUPPORTED,
+    COBEL_REQUIRE(smg <= kMaxSmem, COBEL_EUNSUPPORTED,
                   "Dyna-Q: the replay's dependency masks of %d states do not fit in shared memory (%zu bytes)", S, smg);
-    COBEL_CUDA_OK(cudaFuncSetAttribute(dynaq_warp_kernel<A, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smg));
-    dynaq_warp_kernel<A, false, true><<<(unsigned)((p.n_agents + warps - 1) / warps), warps * 32, smg, st>>>(p);
-    cobel_count_launch();
-    COBEL_CUDA_OK(cudaGetLastError());
-    return COBEL_OK;
+    return launch_kernel(dynaq_warp_kernel<A, false, true>, (unsigned)((p.n_agents + warps - 1) / warps), warps * 32, smg, st, p);
   }
-  const unsigned grid = (unsigned)((p.n_agents + kWarpsPerCta - 1) / kWarpsPerCta);
   if constexpr (A <= 4) {
-    // the production case: two agents per warp (COBEL_DYNAQ_PAIR=0 keeps the warp-per-agent kernel, for A/B runs)
+    // The production case from two waves of the warp-per-agent kernel on: two agents per warp.  It pays once the
+    // machine is full either way: with fewer agents the halved number of warps costs more issue rate than the shared
+    // instructions save (4096 agents: 1.39e9 against 1.58e9 agent-steps/s; 16384: 2.26e9 against 2.05e9; 262144: 2.66e9
+    // against 2.27e9).
     const PairSmem po(S, A);
     const size_t smp = (size_t)wo.bytes + (size_t)kPairWarps * 2 * po.bytes;
-    // It pays once the machine is full either way: with fewer agents than two waves of the warp-per-agent kernel
-    // the halved number of warps costs more issue rate than the shared instructions save (4096 agents: 1.39e9
-    // against 1.58e9 agent-steps/s; 16384: 2.26e9 against 2.05e9; 262144: 2.66e9 against 2.27e9).
-    // COBEL_DYNAQ_PAIR=0 / 1 forces one kernel or the other (A/B runs).
-    static const int pair_env = [] { const char* e = getenv("COBEL_DYNAQ_PAIR"); return e ? (e[0] == '0' ? 0 : 1) : -1; }();
     static const int n_sm = [] { int d = 0, v = 148; if (cudaGetDevice(&d) == cudaSuccess) cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, d); return v; }();
-    const bool pair_on = pair_env >= 0 ? pair_env == 1 : p.n_agents >= (int64_t)2 * 7 * kWarpsPerCta * n_sm;
-    if (plain && pair_on && smp <= 227 * 1024 && S <= 0x7FFF) {
+    if (plain && p.n_agents >= (int64_t)2 * 7 * kWarpsPerCta * n_sm && smp <= kMaxSmem && S <= 0x7FFF) {
       const int64_t per_cta = kPairWarps * 2;
-      COBEL_CUDA_OK(cudaFuncSetAttribute(dynaq_pair_kernel<A>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smp));
-      dynaq_pair_kernel<A><<<(unsigned)((p.n_agents + per_cta - 1) / per_cta), kPairWarps * 32, smp, st>>>(p);
-      cobel_count_launch();
-      COBEL_CUDA_OK(cudaGetLastError());
-      return COBEL_OK;
+      return launch_kernel(dynaq_pair_kernel<A>, (unsigned)((p.n_agents + per_cta - 1) / per_cta), kPairWarps * 32, smp, st, p);
     }
   }
-  if (plain) {
-    COBEL_CUDA_OK(cudaFuncSetAttribute(dynaq_warp_kernel<A, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-    dynaq_warp_kernel<A, true><<<grid, kWarpsPerCta * 32, sm, st>>>(p);
-  } else {
-    COBEL_CUDA_OK(cudaFuncSetAttribute(dynaq_warp_kernel<A, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-    dynaq_warp_kernel<A, false><<<grid, kWarpsPerCta * 32, sm, st>>>(p);
-  }
-  cobel_count_launch();
-  COBEL_CUDA_OK(cudaGetLastError());
-  return COBEL_OK;
+  return launch_kernel(plain ? dynaq_warp_kernel<A, true> : dynaq_warp_kernel<A, false>,
+                       (unsigned)((p.n_agents + kWarpsPerCta - 1) / kWarpsPerCta), kWarpsPerCta * 32, sm, st, p);
 }
 
 }  // namespace
-
-int cobel_validate_common(int64_t n_agents, const CobelWorld& w, const CobelStream& s, const CobelPolicy& pol,
-                          const CobelTrace& tr, int trials, int steps) {
-  COBEL_REQUIRE(n_agents > 0, COBEL_EINVAL, "n_agents must be positive");
-  COBEL_REQUIRE(w.n_states > 0 && w.n_actions > 0 && w.n_starts > 0, COBEL_EINVAL, "empty world");
-  COBEL_REQUIRE(w.succ && w.reward && w.terminal && w.starts, COBEL_EINVAL, "world tables missing");
-  COBEL_REQUIRE(s.draw_count, COBEL_EINVAL, "stream.draw_count missing");
-  COBEL_REQUIRE(pol.param && pol.kind >= 0 && pol.kind <= 2, COBEL_EINVAL, "bad policy");
-  COBEL_REQUIRE(trials >= 0 && steps > 0, COBEL_EINVAL, "trials must be >= 0 and steps > 0");
-  COBEL_REQUIRE(tr.n_steps && tr.n_replay && (trials == 0 || (tr.trial_steps && tr.trial_reward)), COBEL_EINVAL,
-                "trace.trial_steps/trial_reward/n_steps/n_replay are mandatory");
-  return COBEL_OK;
-}
 
 extern "C" int cobel_dynaq_run(const CobelDynaQParams* pp, void* stream) {
   COBEL_REQUIRE(pp != nullptr, COBEL_EINVAL, "null params");
@@ -524,14 +490,5 @@ extern "C" int cobel_dynaq_run(const CobelDynaQParams* pp, void* stream) {
   COBEL_REQUIRE(p.batch >= 0, COBEL_EINVAL, "batch must be >= 0");
   if (p.trials == 0) return COBEL_OK;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  switch (p.world.n_actions) {
-    case 2: return launch<2>(p, st);
-    case 3: return launch<3>(p, st);
-    case 4: return launch<4>(p, st);
-    case 6: return launch<6>(p, st);
-    case 8: return launch<8>(p, st);
-    default:
-      cobel_set_error("unsupported number of actions %d (built for 2,3,4,6,8)", p.world.n_actions);
-      return COBEL_EUNSUPPORTED;
-  }
+  COBEL_DISPATCH_A(p.world.n_actions, return launch<A>(p, st));
 }

@@ -12,16 +12,6 @@ namespace {
 constexpr int kT = 128;
 inline unsigned grid_for(int64_t n) { return (unsigned)((n + kT - 1) / kT); }
 
-#define COBEL_DISPATCH_A(A_, CALL)                                                                       \
-  switch (A_) {                                                                                          \
-    case 2: { constexpr int A = 2; CALL; } break;                                                        \
-    case 3: { constexpr int A = 3; CALL; } break;                                                        \
-    case 4: { constexpr int A = 4; CALL; } break;                                                        \
-    case 6: { constexpr int A = 6; CALL; } break;                                                        \
-    case 8: { constexpr int A = 8; CALL; } break;                                                        \
-    default: cobel_set_error("unsupported number of actions %d (built for 2,3,4,6,8)", (int)(A_)); return COBEL_EUNSUPPORTED; \
-  }
-
 // ---- environment: interface/gridworld.py:92-145, interface/topology.py:126-172 --------------------------------
 __global__ void env_reset_kernel(CobelWorld w, CobelStream s, int64_t n_agents, int32_t* state) {
   const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;

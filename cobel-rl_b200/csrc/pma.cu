@@ -1535,62 +1535,73 @@ __global__ void __launch_bounds__(kMainWarps * 32, BIG ? 1 : 4) pma_main_kernel(
   }
 }
 
+// Shared memory of the main kernel (kMainWarps agents per CTA)
+template <int A>
+int main_smem(int S, size_t& bytes) {
+  bytes = (size_t)kMainWarps * MainSmem(S, A).bytes;
+  COBEL_REQUIRE(bytes <= kMaxSmem, COBEL_EUNSUPPORTED, "PMA: %d states x %d actions do not fit in shared memory", S, A);
+  return COBEL_OK;
+}
+
+// The dense update_sr kernel for S states (register tile 7 up to 112 states, else 10) and its shared memory
+auto sr_kernel_for(int S, size_t& bytes) {
+  const int tile = S <= 7 * 16 ? 7 : 10;
+  bytes = (size_t)(4 * (tile * 16 + 2) + ((S + 1) & ~1) + S * S) * 8;
+  return tile == 7 ? pma_sr_kernel<7> : pma_sr_kernel<10>;
+}
+
+// The final SR refresh of a banded call (the narrowest register window BW >= sr_band) and its shared memory
+auto sr_band_kernel_for(int S, int sr_band, size_t& bytes) {
+  static const struct { int bw; void (*kernel)(CobelPMAParams); } kLadder[] = {
+      {4, pma_sr_band_kernel<4>}, {6, pma_sr_band_kernel<6>}, {8, pma_sr_band_kernel<8>}, {10, pma_sr_band_kernel<10>},
+      {12, pma_sr_band_kernel<12>}, {16, pma_sr_band_kernel<16>}, {24, pma_sr_band_kernel<24>}, {32, pma_sr_band_kernel<32>}};
+  int i = 0;
+  while (i < 7 && kLadder[i].bw < sr_band) ++i;
+  bytes = (size_t)S * (2 * kLadder[i].bw + 2) * 8;
+  return kLadder[i].kernel;
+}
+
+// The tie-pattern policy tables of a call (A <= 4, n_tab > 0)
+template <int A>
+int policy_tables(const CobelPMAParams& p, cudaStream_t st) {
+  if constexpr (A <= 4) {
+    if (p.n_tab > 0)
+      return launch_kernel(pma_policy_table_kernel<A>, (unsigned)p.n_tab + 1, 256, 0, st, p.tab_kind, p.tab_param, p.tab_scratch);
+  }
+  return COBEL_OK;
+}
+
 template <int A>
 int run(const CobelPMAParams& p, cudaStream_t st) {
   const int S = p.world.n_states;
   COBEL_REQUIRE(S <= 512 && S * A <= 2048, COBEL_EUNSUPPORTED,
                 "PMA kernels support at most 512 states and 2048 one-step backups, got %d states x %d actions", S, A);
   const bool big = S > 160 || S * A > 1024;             // pma_main_kernel<A, false, BIG>
-  const MainSmem so(S, A);
-  const size_t sm_main = (size_t)kMainWarps * so.bytes;
-  COBEL_REQUIRE(sm_main <= 227 * 1024, COBEL_EUNSUPPORTED, "PMA: %d states x %d actions do not fit in shared memory", S, A);
-  const bool tabs = p.n_tab > 0 && A <= 4;
+  size_t sm_main, sm_sr;
+  if (int rc = main_smem<A>(S, sm_main)) return rc;
   COBEL_REQUIRE(p.n_tab == 0 || (p.tab_kind && p.tab_param && p.tab_scratch), COBEL_EINVAL,
                 "n_tab > 0 needs tab_kind, tab_param and tab_scratch[n_tab, COBEL_PMA_TAB_DOUBLES(A)]");
-  const bool plain = !big && tabs && p.policy.kind == COBEL_POLICY_EPS_GREEDY && p.mem_policy.kind == COBEL_POLICY_EPS_GREEDY && p.learn &&
-                     !p.no_replay && !p.options && !p.world.tp_off && !p.trace.step_sa && !p.trace.replay_idx &&
-                     !p.trace.replay_len && !p.stream.user_stream;
+  const bool plain = !big && p.n_tab > 0 && A <= 4 && p.policy.kind == COBEL_POLICY_EPS_GREEDY &&
+                     p.mem_policy.kind == COBEL_POLICY_EPS_GREEDY && p.learn && !p.no_replay && !p.options &&
+                     !p.world.tp_off && !p.trace.step_sa && !p.trace.replay_idx && !p.trace.replay_len && !p.stream.user_stream;
   const bool do_replay = p.learn && !p.no_replay;
   const bool band = do_replay && p.sr_band >= 0;
   COBEL_REQUIRE(!big || !do_replay || band, COBEL_EUNSUPPORTED,
                 "PMA: more than 160 states need the banded update_sr (sr_band >= 0; the dense S x S eliminations are "
                 "register-tiled for S <= 160), got %d states", S);
-  const int tile = S <= 7 * 16 ? 7 : 10;
-  const size_t sm_sr = (size_t)(4 * (tile * 16 + 2) + ((S + 1) & ~1) + S * S) * 8;
-  if (!big) {
-    if (tile == 7) COBEL_CUDA_OK(cudaFuncSetAttribute(pma_sr_kernel<7>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_sr));
-    else COBEL_CUDA_OK(cudaFuncSetAttribute(pma_sr_kernel<10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_sr));
-  }
+  const auto sr_kernel = sr_kernel_for(S, sm_sr);
+  auto main_kernel = big ? pma_main_kernel<A, false, true> : pma_main_kernel<A, false>;
   if constexpr (A <= 4) {
-    if (tabs) {                                        // the tie-pattern policy tables of this call
-      pma_policy_table_kernel<A><<<(unsigned)p.n_tab + 1, 256, 0, st>>>(p.tab_kind, p.tab_param, p.tab_scratch);
-      cobel_count_launch();
-    }
+    if (plain) main_kernel = pma_main_kernel<A, true>;
   }
   const unsigned grid_main = (unsigned)((p.n_agents + kMainWarps - 1) / kMainWarps);
-  auto main_launch = [&](MainPhase ph) -> int {
-    auto go = [&](auto kernel) -> int {
-      COBEL_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_main));
-      kernel<<<grid_main, kMainWarps * 32, sm_main, st>>>(p, ph);
-      cobel_count_launch();
-      return COBEL_OK;
-    };
-    if constexpr (A <= 4) {
-      if (plain) return go(pma_main_kernel<A, true>);
-    }
-    if (big) return go(pma_main_kernel<A, false, true>);
-    return go(pma_main_kernel<A, false>);
-  };
-  auto sr_launch = [&](int final_only) {
-    if (tile == 7) pma_sr_kernel<7><<<(unsigned)p.n_agents, kThreads, sm_sr, st>>>(p, final_only);
-    else pma_sr_kernel<10><<<(unsigned)p.n_agents, kThreads, sm_sr, st>>>(p, final_only);
-    cobel_count_launch();
-  };
-  int rc = COBEL_OK;
+  auto main_launch = [&](MainPhase ph) { return launch_kernel(main_kernel, grid_main, kMainWarps * 32, sm_main, st, p, ph); };
+  auto sr_launch = [&](int final_only) { return launch_kernel(sr_kernel, (unsigned)p.n_agents, kThreads, sm_sr, st, p, final_only); };
+  int rc = policy_tables<A>(p, st);
+  if (rc) return rc;
   // MainPhase{init_carry, end_replay, reset, n_trials, trial_first, scratch_need}
-  if (!do_replay) {
-    rc = main_launch(MainPhase{1, 0, 1, p.trials, 0, 0});      // no replay: all trials in one launch
-  } else if (band) {
+  if (!do_replay) return main_launch(MainPhase{1, 0, 1, p.trials, 0, 0});      // no replay: all trials in one launch
+  if (band) {
     // banded update_sr, its own kernels (one warp per agent, full occupancy) between the launches of the main kernel:
     //   main(reset, start replay from the caller's SR, steps of trial 0)
     //   trial t: factor(update_sr; need of the end replay) -> main(end replay t, reset t+1)
@@ -1598,71 +1609,39 @@ int run(const CobelPMAParams& p, cudaStream_t st) {
     //   (a world with ONE starting state: factor also solves SR[start], and the two main launches are one)
     // and SR = inv(I - gamma T) once, densely, from the last factors
     const unsigned grid_band = (unsigned)((p.n_agents + kBandWarps - 1) / kBandWarps);
-    const BandSmem bso(S, p.sr_band);
-    const size_t sm_bandk = (size_t)kBandWarps * bso.bytes;
-    COBEL_CUDA_OK(cudaFuncSetAttribute(pma_band_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_bandk));
-    COBEL_CUDA_OK(cudaFuncSetAttribute(pma_band_factor_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_bandk));
-    if (!p.band_trusted) {                             // the caller's band guarantee on the initial T
-      pma_band_check_kernel<<<(unsigned)p.n_agents, 256, 0, st>>>(p);
-      cobel_count_launch();
-    }
-    rc = main_launch(MainPhase{1, 0, 1, 1, 0, 0});
+    const size_t sm_bandk = (size_t)kBandWarps * BandSmem(S, p.sr_band).bytes;
+    if (!p.band_trusted)                               // the caller's band guarantee on the initial T
+      rc = launch_kernel(pma_band_check_kernel, (unsigned)p.n_agents, 256, 0, st, p);
+    if (!rc) rc = main_launch(MainPhase{1, 0, 1, 1, 0, 0});
     const bool one_start = p.world.n_starts == 1;      // the start row is known before the reset draw
     for (int t = 0; t < p.trials && !rc; ++t) {
       const int more = t + 1 < p.trials ? 1 : 0;
-      pma_band_factor_kernel<<<grid_band, kBandWarps * 32, sm_bandk, st>>>(p, one_start && more);
-      cobel_count_launch();
+      rc = launch_kernel(pma_band_factor_kernel, grid_band, kBandWarps * 32, sm_bandk, st, p, one_start && more);
+      if (rc) break;
       if (one_start) {                                 // end replay t, reset, start replay and steps of trial t + 1
         rc = main_launch(MainPhase{0, 1, more, more, t + 1, 2});
         continue;
       }
       rc = main_launch(MainPhase{0, 1, more, 0, t + 1, 1});
       if (rc || !more) break;
-      pma_band_solve_kernel<<<grid_band, kBandWarps * 32, sm_bandk, st>>>(p, 4);
-      cobel_count_launch();
-      rc = main_launch(MainPhase{0, 0, 0, 1, t + 1, 1});
+      rc = launch_kernel(pma_band_solve_kernel, grid_band, kBandWarps * 32, sm_bandk, st, p, 4);
+      if (!rc) rc = main_launch(MainPhase{0, 0, 0, 1, t + 1, 1});
     }
     if (rc) return rc;
-    const int bwp = p.sr_band <= 4 ? 4 : p.sr_band <= 6 ? 6 : p.sr_band <= 8 ? 8 : p.sr_band <= 10 ? 10 : p.sr_band <= 12 ? 12 :
-                    p.sr_band <= 16 ? 16 : p.sr_band <= 24 ? 24 : 32;
-    const size_t sm_band = (size_t)S * (2 * bwp + 2) * 8;
-    if (sm_band <= 227 * 1024) {
-      auto go = [&](auto kernel) -> int {
-        COBEL_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_band));
-        kernel<<<(unsigned)p.n_agents, (S + 31) & ~31, sm_band, st>>>(p);
-        cobel_count_launch();
-        return COBEL_OK;
-      };
-      rc = p.sr_band <= 4 ? go(pma_sr_band_kernel<4>) : p.sr_band <= 6 ? go(pma_sr_band_kernel<6>) :
-           p.sr_band <= 8 ? go(pma_sr_band_kernel<8>) : p.sr_band <= 10 ? go(pma_sr_band_kernel<10>) :
-           p.sr_band <= 12 ? go(pma_sr_band_kernel<12>) : p.sr_band <= 16 ? go(pma_sr_band_kernel<16>) :
-           p.sr_band <= 24 ? go(pma_sr_band_kernel<24>) : go(pma_sr_band_kernel<32>);
-      if (rc) return rc;
-    } else {
-      COBEL_REQUIRE(!big, COBEL_EUNSUPPORTED, "PMA: the band factors of %d states do not fit in shared memory", S);
-      sr_launch(1);
-    }
-  } else {
-    // trial t: main(reset, start replay, steps) -> sr(update_sr [+ stationary]) -> main(end replay, then trial t+1)
-    rc = main_launch(MainPhase{1, 0, 1, 1, 0, 0});
-    for (int t = 0; t < p.trials && !rc; ++t) {
-      sr_launch(0);
-      const int more = t + 1 < p.trials ? 1 : 0;
-      rc = main_launch(MainPhase{0, 1, more, more, t + 1, 0});
-    }
+    size_t sm_band;
+    const auto band_kernel = sr_band_kernel_for(S, p.sr_band, sm_band);
+    if (sm_band <= kMaxSmem) return launch_kernel(band_kernel, (unsigned)p.n_agents, (S + 31) & ~31, sm_band, st, p);
+    COBEL_REQUIRE(!big, COBEL_EUNSUPPORTED, "PMA: the band factors of %d states do not fit in shared memory", S);
+    return sr_launch(1);
   }
-  if (rc) return rc;
-  COBEL_CUDA_OK(cudaGetLastError());
-  return COBEL_OK;
-}
-
-// carry <- {state, 0, 0, 0, 0, ...}: the per-agent state a stand-alone replay starts from
-__global__ void pma_set_carry_kernel(int64_t* carry, const int32_t* state, int64_t n_agents) {
-  const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (n >= n_agents) return;
-#pragma unroll
-  for (int k = 0; k < 8; ++k) carry[n * 8 + k] = 0;
-  carry[n * 8 + 0] = state[n];
+  // trial t: main(reset, start replay, steps) -> sr(update_sr [+ stationary]) -> main(end replay, then trial t+1)
+  rc = main_launch(MainPhase{1, 0, 1, 1, 0, 0});
+  for (int t = 0; t < p.trials && !rc; ++t) {
+    rc = sr_launch(0);
+    const int more = t + 1 < p.trials ? 1 : 0;
+    if (!rc) rc = main_launch(MainPhase{0, 1, more, more, t + 1, 0});
+  }
+  return rc;
 }
 
 // PMAMemory.replay(Q, action_mask, batch, current_state) as a stand-alone call: the end-of-trial phase of the main kernel
@@ -1671,38 +1650,18 @@ int replay_only(const CobelPMAParams& p, const int32_t* state, int update_sr, cu
   const int S = p.world.n_states;
   COBEL_REQUIRE(S <= 160 && S * A <= 1024, COBEL_EUNSUPPORTED,
                 "PMA kernels support at most 160 states (register-tiled S x S eliminations), got %d", S);
-  const MainSmem so(S, A);
-  const size_t sm_main = (size_t)kMainWarps * so.bytes;
-  COBEL_REQUIRE(sm_main <= 227 * 1024, COBEL_EUNSUPPORTED, "PMA: %d states x %d actions do not fit in shared memory", S, A);
-  if constexpr (A <= 4) {
-    if (p.n_tab > 0) {
-      pma_policy_table_kernel<A><<<(unsigned)p.n_tab + 1, 256, 0, st>>>(p.tab_kind, p.tab_param, p.tab_scratch);
-      cobel_count_launch();
-    }
-  }
-  pma_set_carry_kernel<<<(unsigned)((p.n_agents + 127) / 128), 128, 0, st>>>(p.carry, state, p.n_agents);
+  size_t sm_main, sm_sr;
+  if (int rc = main_smem<A>(S, sm_main)) return rc;
+  const auto sr_kernel = sr_kernel_for(S, sm_sr);
+  if (int rc = policy_tables<A>(p, st)) return rc;
+  if (int rc = cobel_set_carry(p.carry, 8, state, p.n_agents, st)) return rc;
   // M.update_sr() and / or the stationary need of the agents whose current state is None
-  const int tile = S <= 7 * 16 ? 7 : 10;
-  const size_t sm_sr = (size_t)(4 * (tile * 16 + 2) + ((S + 1) & ~1) + S * S) * 8;
-  if (tile == 7) {
-    COBEL_CUDA_OK(cudaFuncSetAttribute(pma_sr_kernel<7>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_sr));
-    pma_sr_kernel<7><<<(unsigned)p.n_agents, kThreads, sm_sr, st>>>(p, update_sr ? 0 : 2);
-  } else {
-    COBEL_CUDA_OK(cudaFuncSetAttribute(pma_sr_kernel<10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_sr));
-    pma_sr_kernel<10><<<(unsigned)p.n_agents, kThreads, sm_sr, st>>>(p, update_sr ? 0 : 2);
-  }
-  auto kernel = pma_main_kernel<A, false>;
-  COBEL_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_main));
-  kernel<<<(unsigned)((p.n_agents + kMainWarps - 1) / kMainWarps), kMainWarps * 32, sm_main, st>>>(p, MainPhase{0, 1, 0, 0, 0, 0});
-  cobel_count_launch(3);
-  COBEL_CUDA_OK(cudaGetLastError());
-  return COBEL_OK;
+  if (int rc = launch_kernel(sr_kernel, (unsigned)p.n_agents, kThreads, sm_sr, st, p, update_sr ? 0 : 2)) return rc;
+  return launch_kernel(pma_main_kernel<A, false>, (unsigned)((p.n_agents + kMainWarps - 1) / kMainWarps), kMainWarps * 32,
+                       sm_main, st, p, MainPhase{0, 1, 0, 0, 0, 0});
 }
 
 }  // namespace
-
-int cobel_validate_common(int64_t n_agents, const CobelWorld& w, const CobelStream& s, const CobelPolicy& pol,
-                          const CobelTrace& tr, int trials, int steps);
 
 extern "C" int cobel_pma_run(const CobelPMAParams* pp, void* stream) {
   COBEL_REQUIRE(pp != nullptr, COBEL_EINVAL, "null params");
@@ -1718,16 +1677,7 @@ extern "C" int cobel_pma_run(const CobelPMAParams* pp, void* stream) {
                 "sr_band must be < 0 (dense update_sr) or 0..31 with band_scratch[N, S*(2*sr_band+1)]");
   if (p.trials == 0) return COBEL_OK;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  switch (p.world.n_actions) {
-    case 2: return run<2>(p, st);
-    case 3: return run<3>(p, st);
-    case 4: return run<4>(p, st);
-    case 6: return run<6>(p, st);
-    case 8: return run<8>(p, st);
-    default:
-      cobel_set_error("unsupported number of actions %d (built for 2,3,4,6,8)", p.world.n_actions);
-      return COBEL_EUNSUPPORTED;
-  }
+  COBEL_DISPATCH_A(p.world.n_actions, return run<A>(p, st));
 }
 
 extern "C" int cobel_pma_replay(const CobelPMAParams* pp, const int32_t* state, int update_sr, void* stream) {
@@ -1742,14 +1692,5 @@ extern "C" int cobel_pma_replay(const CobelPMAParams* pp, const int32_t* state, 
   COBEL_REQUIRE(p.learn && !p.no_replay, COBEL_EINVAL, "cobel_pma_replay needs learn = 1 and no_replay = 0");
   COBEL_REQUIRE(p.n_tab == 0 || (p.tab_kind && p.tab_param && p.tab_scratch), COBEL_EINVAL, "policy tables incomplete");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  switch (p.world.n_actions) {
-    case 2: return replay_only<2>(p, state, update_sr, st);
-    case 3: return replay_only<3>(p, state, update_sr, st);
-    case 4: return replay_only<4>(p, state, update_sr, st);
-    case 6: return replay_only<6>(p, state, update_sr, st);
-    case 8: return replay_only<8>(p, state, update_sr, st);
-    default:
-      cobel_set_error("unsupported number of actions %d (built for 2,3,4,6,8)", p.world.n_actions);
-      return COBEL_EUNSUPPORTED;
-  }
+  COBEL_DISPATCH_A(p.world.n_actions, return replay_only<A>(p, state, update_sr, st));
 }

@@ -196,39 +196,23 @@ int launch(const CobelQParams& p, cudaStream_t st) {
   const QWorldSmem wo(p.world.n_states, A, p.world.n_starts);
   const QSmem ao(p.n_keys, A);
   const size_t sm = (size_t)wo.bytes + (size_t)kWarpsPerCta * ao.bytes;
-  if (sm > 227 * 1024) {
+  if (sm > kMaxSmem) {
     // the tables do not fit: Q stays in HBM / L2, only the dependency masks of the replay are staged
     const QSmem go(p.n_keys, A, false);
     int warps = kWarpsPerCta;
-    while (warps > 1 && (size_t)warps * go.bytes > 227 * 1024) warps >>= 1;
+    while (warps > 1 && (size_t)warps * go.bytes > kMaxSmem) warps >>= 1;
     const size_t smg = (size_t)warps * go.bytes;
-    COBEL_REQUIRE(smg <= 227 * 1024, COBEL_EUNSUPPORTED,
+    COBEL_REQUIRE(smg <= kMaxSmem, COBEL_EUNSUPPORTED,
                   "QAgent: the replay's dependency masks of %d keys do not fit in shared memory (%zu bytes)", p.n_keys, smg);
-    COBEL_CUDA_OK(cudaFuncSetAttribute(q_warp_kernel<A, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smg));
-    q_warp_kernel<A, false, true><<<(unsigned)((p.n_agents + warps - 1) / warps), warps * 32, smg, st>>>(p);
-    cobel_count_launch();
-    COBEL_CUDA_OK(cudaGetLastError());
-    return COBEL_OK;
+    return launch_kernel(q_warp_kernel<A, false, true>, (unsigned)((p.n_agents + warps - 1) / warps), warps * 32, smg, st, p);
   }
-  const unsigned grid = (unsigned)((p.n_agents + kWarpsPerCta - 1) / kWarpsPerCta);
   const bool plain = !p.world.tp_off && !p.trace.step_sa && !p.trace.replay_idx && !p.trace.replay_len &&
                      p.policy.kind == COBEL_POLICY_EPS_GREEDY && p.learn && p.batch == 32 && !p.stream.user_stream;
-  if (plain) {
-    COBEL_CUDA_OK(cudaFuncSetAttribute(q_warp_kernel<A, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-    q_warp_kernel<A, true><<<grid, kWarpsPerCta * 32, sm, st>>>(p);
-  } else {
-    COBEL_CUDA_OK(cudaFuncSetAttribute(q_warp_kernel<A, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-    q_warp_kernel<A, false><<<grid, kWarpsPerCta * 32, sm, st>>>(p);
-  }
-  cobel_count_launch();
-  COBEL_CUDA_OK(cudaGetLastError());
-  return COBEL_OK;
+  return launch_kernel(plain ? q_warp_kernel<A, true> : q_warp_kernel<A, false>,
+                       (unsigned)((p.n_agents + kWarpsPerCta - 1) / kWarpsPerCta), kWarpsPerCta * 32, sm, st, p);
 }
 
 }  // namespace
-
-int cobel_validate_common(int64_t n_agents, const CobelWorld& w, const CobelStream& s, const CobelPolicy& pol,
-                          const CobelTrace& tr, int trials, int steps);
 
 extern "C" int cobel_q_run(const CobelQParams* pp, void* stream) {
   COBEL_REQUIRE(pp != nullptr, COBEL_EINVAL, "null params");
@@ -241,14 +225,5 @@ extern "C" int cobel_q_run(const CobelQParams* pp, void* stream) {
   if (p.trials == 0) return COBEL_OK;                  // a zero-trial session is a no-op (no log needed)
   COBEL_REQUIRE(!p.learn || (p.log && p.log_len && p.log_cap > 0), COBEL_EINVAL, "experience log missing");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  switch (p.world.n_actions) {
-    case 2: return launch<2>(p, st);
-    case 3: return launch<3>(p, st);
-    case 4: return launch<4>(p, st);
-    case 6: return launch<6>(p, st);
-    case 8: return launch<8>(p, st);
-    default:
-      cobel_set_error("unsupported number of actions %d (built for 2,3,4,6,8)", p.world.n_actions);
-      return COBEL_EUNSUPPORTED;
-  }
+  COBEL_DISPATCH_A(p.world.n_actions, return launch<A>(p, st));
 }

@@ -16,7 +16,6 @@
 // reference's operation order; exp() and the CDF prefix sums are not bit-identical to NumPy's
 // and only decide the sampled index, so a draw that falls within 1e-12 of a bin edge raises
 // COBEL_FLAG_CDF_NEAR_TIE instead of silently risking a different index.
-#include <cstdlib>
 #include "warp_agent.cuh"
 #include "thread_agent.cuh"
 
@@ -1175,36 +1174,48 @@ __global__ void __launch_bounds__(256) sfma_kernel(const __grid_constant__ Cobel
   }
 }
 
+// The replay kernel's CTA size for S*A experiences and the capacity of its list of experienced (s, a) at that size
+template <int A>
+int replay_plan(const CobelSFMAParams& p, int& threads, int& cap) {
+  const int S = p.world.n_states, N = S * A;
+  threads = N <= 128 ? 64 : N <= 4096 ? 128 : 256;
+  cap = ReplaySmem::fit(S, A, threads, p.batch, p.random_replay != 0, kMaxSmem - 512);
+  const ReplaySmem rso(S, A, threads, p.batch, p.random_replay != 0, cap);
+  COBEL_REQUIRE(cap >= 1 && rso.bytes <= kMaxSmem, COBEL_EUNSUPPORTED,
+                "SFMA replay of %d states x %d actions needs %d bytes of shared memory", S, A, rso.bytes);
+  return COBEL_OK;
+}
+
+// One launch of the replay kernel: `threads` per agent, a list of ph.list_cap entries
+template <int A>
+int replay_launch(const CobelSFMAParams& p, SfmaPhase ph, int threads, cudaStream_t st) {
+  const ReplaySmem so(p.world.n_states, A, threads, p.batch, p.random_replay != 0, ph.list_cap);
+  return launch_kernel(sfma_replay_kernel<A>, (unsigned)p.n_agents, threads, so.bytes, st, p, ph);
+}
+
 template <int A>
 int launch(const CobelSFMAParams& p, cudaStream_t st) {
   const int S = p.world.n_states, N = S * A;
   COBEL_REQUIRE(S <= 0x7FFF, COBEL_EUNSUPPORTED, "SFMA kernel supports at most 32767 states");
   const int T = N <= 128 ? 64 : N <= 512 ? 128 : 256;
   // Split path: per-step work that touches single table entries only (no decay of C, M.T neither read nor kept,
-  // no strength modulation over all experiences), and the caller provided the carry scratch
+  // no strength modulation over all experiences)
   const bool track_t = p.recency != 0 || (p.learn && p.no_replay);
-  const bool split = p.carry != nullptr && p.decay_strength == 1.0 && !track_t && !(p.mod_flags & COBEL_SFMA_MOD_REWARD);
+  const bool split = p.decay_strength == 1.0 && !track_t && !(p.mod_flags & COBEL_SFMA_MOD_REWARD);
   // (state spaces whose tables exceed shared memory run on the split path only: its step kernel works on the tables
   //  in HBM and its replay kernel stages just the list of experienced (s, a))
   if (split) {
-    // CTA size of the replay kernel: its passes run over the compact list of experienced (s, a) -- a few hundred
-    // entries -- and every warp repeats the block-wide combines, so a small CTA with more CTAs per SM wins (20x20,
-    // 65536 agents, lists of <= 800 entries: 0.88 / 1.19 / 1.11 / 0.73 x 10^9 agent-steps/s with 32 / 64 / 128 / 256
-    // threads); chosen per launch from the length bound of the list
-    int TR = N <= 128 ? 64 : N <= 4096 ? 128 : 256;
-    bool tr_forced = false;
-    if (const char* e = getenv("COBEL_SFMA_REPLAY_THREADS")) { const int v = atoi(e); if (v == 32 || v == 64 || v == 128 || v == 256) { TR = v; tr_forced = true; } }
-    const int cap = ReplaySmem::fit(S, A, TR, p.batch, p.random_replay != 0, 227 * 1024 - 512);
-    const ReplaySmem rso(S, A, TR, p.batch, p.random_replay != 0, cap);
-    COBEL_REQUIRE(cap >= 1 && rso.bytes <= 227 * 1024, COBEL_EUNSUPPORTED,
-                  "SFMA replay of %d states x %d actions needs %d bytes of shared memory", S, A, rso.bytes);
-    COBEL_CUDA_OK(cudaFuncSetAttribute(sfma_replay_kernel<A>, cudaFuncAttributeMaxDynamicSharedMemorySize, rso.bytes));
+    int TR, cap;
+    if (int rc = replay_plan<A>(p, TR, cap)) return rc;
     COBEL_CUDA_OK(cudaFuncSetAttribute(sfma_replay_kernel<A>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     const unsigned grid_step = (unsigned)((p.n_agents + 63) / 64);
-    auto step = [&](SfmaPhase ph) { sfma_step_kernel<A><<<grid_step, 64, 0, st>>>(p, ph); cobel_count_launch(); };
+    auto step = [&](SfmaPhase ph) { return launch_kernel(sfma_step_kernel<A>, grid_step, 64, 0, st, p, ph); };
     // The list of experienced (s, a) of a replay holds at most what the agent had when the call started plus one new
     // pair per step taken since (A with state_mod): with the caller's bound (exp_bound) a launch stages that many entries instead of
     // S*A -- at C4 22 KB instead of 40 KB per agent, 8 instead of 5 resident CTAs per SM.
+    // CTA size: the replay's passes run over that list -- a few hundred entries -- and every warp repeats the
+    // block-wide combines, so a small CTA with more CTAs per SM wins (20x20, 65536 agents, lists of <= 800 entries:
+    // 0.88 / 1.19 / 1.11 / 0.73 x 10^9 agent-steps/s with 32 / 64 / 128 / 256 threads): 64 threads up to 1024 entries.
     auto replay = [&](SfmaPhase ph) {
       int lc = cap;
       if (p.exp_bound > 0) {
@@ -1213,76 +1224,42 @@ int launch(const CobelSFMAParams& p, cudaStream_t st) {
         const long long bound = (long long)p.exp_bound - 1 + (long long)(ph.trial + (ph.start_replay ? 0 : 1)) * p.steps * per_step;
         if (bound < lc) lc = bound < 1 ? 1 : (int)bound;
       }
-      const int tr = (tr_forced || lc > cap) ? TR : (lc <= 1024 ? 64 : TR);
-      const ReplaySmem ls(S, A, tr, p.batch, p.random_replay != 0, lc);
       ph.list_cap = lc;
-      sfma_replay_kernel<A><<<(unsigned)p.n_agents, tr, ls.bytes, st>>>(p, ph);
-      cobel_count_launch();
+      return replay_launch<A>(p, ph, lc <= 1024 ? 64 : TR, st);
     };
     // SfmaPhase{init, reset, n_trials, trial, start_replay}
-    if (!p.learn) {
-      step(SfmaPhase{1, 1, p.trials, 0, 0, cap});                  // test(): all trials in one launch
-    } else {
-      for (int t = 0; t < p.trials; ++t) {
-        if (p.start_replay) {                                      // agent/sfma.py:272-275: trace only, no Q updates
-          step(SfmaPhase{t == 0, 1, 0, t, 0, cap});
-          replay(SfmaPhase{0, 0, 0, t, 1, cap});
-          step(SfmaPhase{0, 0, 1, t, 0, cap});
-        } else {
-          step(SfmaPhase{t == 0, 1, 1, t, 0, cap});
-        }
-        replay(SfmaPhase{0, 0, 0, t, 0, cap});                          // agent/sfma.py:300-324 (no_replay keeps M.T: fused path)
+    if (!p.learn) return step(SfmaPhase{1, 1, p.trials, 0, 0, cap});     // test(): all trials in one launch
+    for (int t = 0; t < p.trials; ++t) {
+      if (p.start_replay) {                                      // agent/sfma.py:272-275: trace only, no Q updates
+        if (int rc = step(SfmaPhase{t == 0, 1, 0, t, 0, cap})) return rc;
+        if (int rc = replay(SfmaPhase{0, 0, 0, t, 1, cap})) return rc;
+        if (int rc = step(SfmaPhase{0, 0, 1, t, 0, cap})) return rc;
+      } else if (int rc = step(SfmaPhase{t == 0, 1, 1, t, 0, cap})) {
+        return rc;
       }
-      // M.T.fill(0) after every trial with replay (agent/sfma.py:324); M.T is not tracked on this path
-      if (p.trials > 0) COBEL_CUDA_OK(cudaMemsetAsync(p.T, 0, (size_t)p.n_agents * N * sizeof(double), st));
+      if (int rc = replay(SfmaPhase{0, 0, 0, t, 0, cap})) return rc;   // agent/sfma.py:300-324 (no_replay keeps M.T: fused path)
     }
-    COBEL_CUDA_OK(cudaGetLastError());
+    // M.T.fill(0) after every trial with replay (agent/sfma.py:324); M.T is not tracked on this path
+    if (p.trials > 0) COBEL_CUDA_OK(cudaMemsetAsync(p.T, 0, (size_t)p.n_agents * N * sizeof(double), st));
     return COBEL_OK;
   }
   const SfmaSmem so(S, A, T, p.batch, p.recency != 0 || p.no_replay != 0, p.random_replay != 0);
-  COBEL_REQUIRE(so.bytes <= 227 * 1024, COBEL_EUNSUPPORTED,
+  COBEL_REQUIRE(so.bytes <= kMaxSmem, COBEL_EUNSUPPORTED,
                 "SFMA tables of %d states x %d actions need %d bytes of shared memory", S, A, so.bytes);
-  if (p.mod_flags) {
-    COBEL_CUDA_OK(cudaFuncSetAttribute(sfma_kernel<A, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, so.bytes));
-    sfma_kernel<A, true><<<(unsigned)p.n_agents, T, so.bytes, st>>>(p);
-  } else {
-    COBEL_CUDA_OK(cudaFuncSetAttribute(sfma_kernel<A, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, so.bytes));
-    sfma_kernel<A, false><<<(unsigned)p.n_agents, T, so.bytes, st>>>(p);
-  }
-  cobel_count_launch();
-  COBEL_CUDA_OK(cudaGetLastError());
-  return COBEL_OK;
-}
-
-__global__ void sfma_set_carry_kernel(int64_t* carry, const int32_t* state, int64_t n_agents) {
-  const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (n >= n_agents) return;
-  carry[n * 4 + 0] = state[n];
-  carry[n * 4 + 1] = 0; carry[n * 4 + 2] = 0; carry[n * 4 + 3] = 0;
+  return launch_kernel(p.mod_flags ? sfma_kernel<A, true> : sfma_kernel<A, false>, (unsigned)p.n_agents, T, so.bytes, st, p);
 }
 
 // SFMAMemory.replay(batch, state) / SFMA.replay(batch, state) as a stand-alone call: the replay kernel of the split path
 template <int A>
 int replay_only(const CobelSFMAParams& p, const int32_t* state, int apply_updates, cudaStream_t st) {
-  const int S = p.world.n_states, N = S * A;
-  COBEL_REQUIRE(S <= 0x7FFF, COBEL_EUNSUPPORTED, "SFMA kernel supports at most 32767 states");
-  const int T = N <= 128 ? 64 : N <= 4096 ? 128 : 256;
-  const int cap = ReplaySmem::fit(S, A, T, p.batch, p.random_replay != 0, 227 * 1024 - 512);
-  const ReplaySmem rso(S, A, T, p.batch, p.random_replay != 0, cap);
-  COBEL_REQUIRE(cap >= 1 && rso.bytes <= 227 * 1024, COBEL_EUNSUPPORTED,
-                "SFMA replay of %d states x %d actions needs %d bytes of shared memory", S, A, rso.bytes);
-  COBEL_CUDA_OK(cudaFuncSetAttribute(sfma_replay_kernel<A>, cudaFuncAttributeMaxDynamicSharedMemorySize, rso.bytes));
-  sfma_set_carry_kernel<<<(unsigned)((p.n_agents + 127) / 128), 128, 0, st>>>(p.carry, state, p.n_agents);
-  sfma_replay_kernel<A><<<(unsigned)p.n_agents, T, rso.bytes, st>>>(p, SfmaPhase{0, 0, 0, 0, apply_updates == 1 ? 0 : (apply_updates == 2 ? 2 : 1), cap});
-  cobel_count_launch(2);
-  COBEL_CUDA_OK(cudaGetLastError());
-  return COBEL_OK;
+  COBEL_REQUIRE(p.world.n_states <= 0x7FFF, COBEL_EUNSUPPORTED, "SFMA kernel supports at most 32767 states");
+  int T, cap;
+  if (int rc = replay_plan<A>(p, T, cap)) return rc;
+  if (int rc = cobel_set_carry(p.carry, 4, state, p.n_agents, st)) return rc;
+  return replay_launch<A>(p, SfmaPhase{0, 0, 0, 0, apply_updates == 1 ? 0 : (apply_updates == 2 ? 2 : 1), cap}, T, st);
 }
 
 }  // namespace
-
-int cobel_validate_common(int64_t n_agents, const CobelWorld& w, const CobelStream& s, const CobelPolicy& pol,
-                          const CobelTrace& tr, int trials, int steps);
 
 extern "C" int cobel_sfma_run(const CobelSFMAParams* pp, void* stream) {
   COBEL_REQUIRE(pp != nullptr, COBEL_EINVAL, "null params");
@@ -1291,20 +1268,12 @@ extern "C" int cobel_sfma_run(const CobelSFMAParams* pp, void* stream) {
   if (rc) return rc;
   COBEL_REQUIRE(p.Q && p.Mr && p.Ms && p.Mt && p.C && p.T && p.I && p.D && p.lr && p.gamma && p.mem_lr, COBEL_EINVAL,
                 "agent tables missing");
+  COBEL_REQUIRE(p.carry, COBEL_EINVAL, "carry scratch missing");
   COBEL_REQUIRE(p.batch >= 0 && p.nb_replays >= 0, COBEL_EINVAL, "batch and nb_replays must be >= 0");
   COBEL_REQUIRE(p.mode >= MODE_DEFAULT && p.mode <= MODE_SWEEPING, COBEL_EINVAL, "unknown replay mode %d", p.mode);
   if (p.trials == 0) return COBEL_OK;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  switch (p.world.n_actions) {
-    case 2: return launch<2>(p, st);
-    case 3: return launch<3>(p, st);
-    case 4: return launch<4>(p, st);
-    case 6: return launch<6>(p, st);
-    case 8: return launch<8>(p, st);
-    default:
-      cobel_set_error("unsupported number of actions %d (built for 2,3,4,6,8)", p.world.n_actions);
-      return COBEL_EUNSUPPORTED;
-  }
+  COBEL_DISPATCH_A(p.world.n_actions, return launch<A>(p, st));
 }
 
 extern "C" int cobel_sfma_replay(const CobelSFMAParams* pp, const int32_t* state, int apply_updates, void* stream) {
@@ -1317,14 +1286,5 @@ extern "C" int cobel_sfma_replay(const CobelSFMAParams* pp, const int32_t* state
   COBEL_REQUIRE(p.batch >= 0 && p.nb_replays >= 0 && !p.recency, COBEL_EINVAL, "batch and nb_replays must be >= 0; recency runs inside train() only");
   COBEL_REQUIRE(p.mode >= MODE_DEFAULT && p.mode <= MODE_SWEEPING, COBEL_EINVAL, "unknown replay mode %d", p.mode);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  switch (p.world.n_actions) {
-    case 2: return replay_only<2>(p, state, apply_updates, st);
-    case 3: return replay_only<3>(p, state, apply_updates, st);
-    case 4: return replay_only<4>(p, state, apply_updates, st);
-    case 6: return replay_only<6>(p, state, apply_updates, st);
-    case 8: return replay_only<8>(p, state, apply_updates, st);
-    default:
-      cobel_set_error("unsupported number of actions %d (built for 2,3,4,6,8)", p.world.n_actions);
-      return COBEL_EUNSUPPORTED;
-  }
+  COBEL_DISPATCH_A(p.world.n_actions, return replay_only<A>(p, state, apply_updates, st));
 }

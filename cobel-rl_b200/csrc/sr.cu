@@ -13,7 +13,6 @@
 // (S*S*8 bytes per agent: 5 KB at 5x5, 1.28 MB at 20x20) and is streamed through L1/L2 with
 // coalesced fp64 row accesses: A+2 row reads and one row write per step (8S(A+4) algorithmic
 // bytes); rewards / model / Q scratch live in shared memory.
-#include <cstdlib>
 #include "warp_agent.cuh"
 #include "tma.cuh"
 
@@ -446,30 +445,18 @@ int launch(const CobelSRParams& p, cudaStream_t st) {
   const int S = p.world.n_states;
   PairwisePlan pl;
   COBEL_REQUIRE(make_plan(pl, S), COBEL_EUNSUPPORTED, "dense SR kernel supports at most %d states", kMaxLeaves * 128);
-  // TMA path: rows are 16-byte multiples and both row sets fit in shared memory (COBEL_SR_NO_TMA=1: profiling aid)
+  // TMA path: rows are 16-byte multiples and both row sets fit in shared memory
   const SRTmaSmem to(S, A, pl.nl);
-  if (S % 2 == 0 && to.bytes <= 200 * 1024 && !getenv("COBEL_SR_NO_TMA")) {
-    COBEL_CUDA_OK(cudaFuncSetAttribute(sr_tma_kernel<A>, cudaFuncAttributeMaxDynamicSharedMemorySize, to.bytes));
-    sr_tma_kernel<A><<<(unsigned)p.n_agents, 128, to.bytes, st>>>(p, pl);
-    cobel_count_launch();
-    COBEL_CUDA_OK(cudaGetLastError());
-    return COBEL_OK;
-  }
+  if (S % 2 == 0 && to.bytes <= 200 * 1024)
+    return launch_kernel(sr_tma_kernel<A>, (unsigned)p.n_agents, 128, to.bytes, st, p, pl);
   const SRSmem so(S, A, pl.nl);
-  COBEL_REQUIRE(so.bytes <= 227 * 1024, COBEL_EUNSUPPORTED, "dense SR kernel: %d states need %d bytes of shared memory",
+  COBEL_REQUIRE(so.bytes <= kMaxSmem, COBEL_EUNSUPPORTED, "dense SR kernel: %d states need %d bytes of shared memory",
                 S, so.bytes);
-  COBEL_CUDA_OK(cudaFuncSetAttribute(sr_kernel<A>, cudaFuncAttributeMaxDynamicSharedMemorySize, so.bytes));
   const int T = S <= 32 ? 32 : S <= 64 ? 64 : S <= 256 ? 128 : 256;
-  sr_kernel<A><<<(unsigned)p.n_agents, T, so.bytes, st>>>(p, pl);
-  cobel_count_launch();
-  COBEL_CUDA_OK(cudaGetLastError());
-  return COBEL_OK;
+  return launch_kernel(sr_kernel<A>, (unsigned)p.n_agents, T, so.bytes, st, p, pl);
 }
 
 }  // namespace
-
-int cobel_validate_common(int64_t n_agents, const CobelWorld& w, const CobelStream& s, const CobelPolicy& pol,
-                          const CobelTrace& tr, int trials, int steps);
 
 extern "C" int cobel_sr_run(const CobelSRParams* pp, void* stream) {
   COBEL_REQUIRE(pp != nullptr, COBEL_EINVAL, "null params");
@@ -479,14 +466,5 @@ extern "C" int cobel_sr_run(const CobelSRParams* pp, void* stream) {
   COBEL_REQUIRE(p.SR && p.rewards && p.model && p.lr && p.gamma, COBEL_EINVAL, "agent tables missing");
   if (p.trials == 0) return COBEL_OK;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  switch (p.world.n_actions) {
-    case 2: return launch<2>(p, st);
-    case 3: return launch<3>(p, st);
-    case 4: return launch<4>(p, st);
-    case 6: return launch<6>(p, st);
-    case 8: return launch<8>(p, st);
-    default:
-      cobel_set_error("unsupported number of actions %d (built for 2,3,4,6,8)", p.world.n_actions);
-      return COBEL_EUNSUPPORTED;
-  }
+  COBEL_DISPATCH_A(p.world.n_actions, return launch<A>(p, st));
 }

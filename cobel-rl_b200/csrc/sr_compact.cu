@@ -249,25 +249,14 @@ template <int A>
 int launch(const CobelSRCompactParams& p, cudaStream_t st) {
   const CompactSmem so(p.max_visited, A);
   const size_t sm = (size_t)kWarpsPerCta * so.bytes;
-  COBEL_REQUIRE(sm <= 227 * 1024, COBEL_EUNSUPPORTED, "max_visited %d does not fit in shared memory", p.max_visited);
-  const unsigned grid = (unsigned)((p.n_agents + kWarpsPerCta - 1) / kWarpsPerCta);
-  if (!p.action_mask && !p.world.tp_off && !p.trace.step_sa && p.policy.kind == COBEL_POLICY_EPS_GREEDY &&
-      !p.stream.user_stream) {
-    COBEL_CUDA_OK(cudaFuncSetAttribute(sr_compact_kernel<A, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-    sr_compact_kernel<A, true><<<grid, kWarpsPerCta * 32, sm, st>>>(p);
-  } else {
-    COBEL_CUDA_OK(cudaFuncSetAttribute(sr_compact_kernel<A, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-    sr_compact_kernel<A, false><<<grid, kWarpsPerCta * 32, sm, st>>>(p);
-  }
-  cobel_count_launch();
-  COBEL_CUDA_OK(cudaGetLastError());
-  return COBEL_OK;
+  COBEL_REQUIRE(sm <= kMaxSmem, COBEL_EUNSUPPORTED, "max_visited %d does not fit in shared memory", p.max_visited);
+  const bool plain = !p.action_mask && !p.world.tp_off && !p.trace.step_sa && p.policy.kind == COBEL_POLICY_EPS_GREEDY &&
+                     !p.stream.user_stream;
+  return launch_kernel(plain ? sr_compact_kernel<A, true> : sr_compact_kernel<A, false>,
+                       (unsigned)((p.n_agents + kWarpsPerCta - 1) / kWarpsPerCta), kWarpsPerCta * 32, sm, st, p);
 }
 
 }  // namespace
-
-int cobel_validate_common(int64_t n_agents, const CobelWorld& w, const CobelStream& s, const CobelPolicy& pol,
-                          const CobelTrace& tr, int trials, int steps);
 
 extern "C" int cobel_sr_compact_run(const CobelSRCompactParams* pp, void* stream) {
   COBEL_REQUIRE(pp != nullptr, COBEL_EINVAL, "null params");
@@ -279,14 +268,5 @@ extern "C" int cobel_sr_compact_run(const CobelSRCompactParams* pp, void* stream
   COBEL_REQUIRE(p.max_visited >= 2 && p.max_visited <= 65535, COBEL_EINVAL, "max_visited must be in 2..65535");
   if (p.trials == 0) return COBEL_OK;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  switch (p.world.n_actions) {
-    case 2: return launch<2>(p, st);
-    case 3: return launch<3>(p, st);
-    case 4: return launch<4>(p, st);
-    case 6: return launch<6>(p, st);
-    case 8: return launch<8>(p, st);
-    default:
-      cobel_set_error("unsupported number of actions %d (built for 2,3,4,6,8)", p.world.n_actions);
-      return COBEL_EUNSUPPORTED;
-  }
+  COBEL_DISPATCH_A(p.world.n_actions, return launch<A>(p, st));
 }

@@ -1,4 +1,5 @@
-// util.cu -- error plumbing, launch counter and the stream-contract probe.
+// util.cu -- error plumbing, launch counter, the checks and the carry set-up shared by the entry points, and the
+// stream-contract probe.
 #include "common.cuh"
 #include <atomic>
 #include <cstdarg>
@@ -26,7 +27,30 @@ __global__ void stream_next_kernel(CobelStream s, int64_t n_agents, int64_t n_dr
   for (int64_t k = 0; k < n_draws; ++k) out[a * n_draws + k] = rng.next();
   s.draw_count[a] = (int64_t)rng.k;
 }
+__global__ void set_carry_kernel(int64_t* carry, int stride, const int32_t* state, int64_t n_agents) {
+  const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (n >= n_agents) return;
+  carry[n * stride] = state[n];
+  for (int k = 1; k < stride; ++k) carry[n * stride + k] = 0;
+}
 }  // namespace
+
+int cobel_validate_common(int64_t n_agents, const CobelWorld& w, const CobelStream& s, const CobelPolicy& pol,
+                          const CobelTrace& tr, int trials, int steps) {
+  COBEL_REQUIRE(n_agents > 0, COBEL_EINVAL, "n_agents must be positive");
+  COBEL_REQUIRE(w.n_states > 0 && w.n_actions > 0 && w.n_starts > 0, COBEL_EINVAL, "empty world");
+  COBEL_REQUIRE(w.succ && w.reward && w.terminal && w.starts, COBEL_EINVAL, "world tables missing");
+  COBEL_REQUIRE(s.draw_count, COBEL_EINVAL, "stream.draw_count missing");
+  COBEL_REQUIRE(pol.param && pol.kind >= 0 && pol.kind <= 2, COBEL_EINVAL, "bad policy");
+  COBEL_REQUIRE(trials >= 0 && steps > 0, COBEL_EINVAL, "trials must be >= 0 and steps > 0");
+  COBEL_REQUIRE(tr.n_steps && tr.n_replay && (trials == 0 || (tr.trial_steps && tr.trial_reward)), COBEL_EINVAL,
+                "trace.trial_steps/trial_reward/n_steps/n_replay are mandatory");
+  return COBEL_OK;
+}
+
+int cobel_set_carry(int64_t* carry, int stride, const int32_t* state, int64_t n_agents, cudaStream_t st) {
+  return launch_kernel(set_carry_kernel, (unsigned)((n_agents + 127) / 128), 128, 0, st, carry, stride, state, n_agents);
+}
 
 void cobel_set_error(const char* fmt, ...) {
   va_list ap;
@@ -35,7 +59,7 @@ void cobel_set_error(const char* fmt, ...) {
   va_end(ap);
 }
 
-void cobel_count_launch(int n) { g_launches += n; }
+void cobel_count_launch() { ++g_launches; }
 
 extern "C" int cobel_abi_version(void) { return COBEL_ABI_VERSION; }
 

@@ -48,7 +48,7 @@ class SFMAMemory(TableMemory):
         self._C = torch.zeros((n, S * A), dtype=torch.float64, device=dev)
         self._T = torch.zeros((n, S * A), dtype=torch.float64, device=dev)
         self._I = torch.zeros((n, S), dtype=torch.float64, device=dev)
-        self._carry = torch.zeros((n, 4), dtype=torch.int64, device=dev)            # kernel scratch (split path)
+        self._carry = torch.zeros((n, 4), dtype=torch.int64, device=dev)            # kernel scratch
 
     C = property(lambda self: self._view(self._C))
     T = property(lambda self: self._view(self._T))
@@ -81,7 +81,7 @@ class SFMAMemory(TableMemory):
 
     # ---- C ABI parameters ------------------------------------------------------------------------------------------
     def _params(self, st, world, pol, tr, keep, agent=None, n_tr=0, steps=1, batch=0, no_replay=False, learn=True,
-                dynamic=False, trial_mode=None, split=True, nb_replays=None, random=None):
+                dynamic=False, trial_mode=None, nb_replays=None, random=None):
         """``CobelSFMAParams`` around the memory's tables; ``agent`` (an SFMA agent) adds Q, the action mask, the agent's
         hyper-parameters and replay switches."""
         mlr = st.param(self.learning_rate, 'memory learning_rate')
@@ -110,7 +110,7 @@ class SFMAMemory(TableMemory):
             self.mode_id(), 1 if self.recency else 0, 1 if self.deterministic else 0, n_tr, steps, batch,
             nbr, 1 if start_replay else 0, 1 if rnd else 0, 1 if dynamic else 0,
             1 if no_replay else 0, 1 if learn else 0, _lib.ptr(td), _lib.ptr(trial_mode),
-            float(self.reward_modulation), self.mod_flags(), 0, self._carry.data_ptr() if split else None)
+            float(self.reward_modulation), self.mod_flags(), 0, self._carry.data_ptr())
 
     def _table_world(self):
         return _lib.World(self.nb_states, self.nb_actions, 0, 0, None, None, None, None, None, None, None)

@@ -255,9 +255,8 @@ typedef struct CobelSFMAParams {
   int32_t  exp_bound;        /* 1 + an upper bound on the number of (s, a) with C > 0 that any agent holds when the call starts; 0 =
                                 unknown.  The split path sizes the replay kernel's on-chip list by exp_bound - 1 + the steps taken
                                 so far instead of S*A: less shared memory per agent, more agents per SM */
-  int64_t* carry;            /* optional scratch [N,4]: per-agent state between the launches of the split path (one
-                                thread per agent for the online steps, one CTA per agent for the replays); NULL = the
-                                fused one-CTA-per-agent kernel */
+  int64_t* carry;            /* scratch [N,4], required: per-agent state between the launches of the split path (one
+                                thread per agent for the online steps, one CTA per agent for the replays) */
 } CobelSFMAParams;
 
 int cobel_sfma_run(const CobelSFMAParams* p, void* stream);

@@ -17,7 +17,8 @@ from cobel_rl_b200.policy import EpsilonGreedy  # noqa: E402
 
 def main():
     dev = 'cuda:0'
-    # Dyna-Q: COBEL_DYNAQ_PAIR=1 / 0 in the environment selects the two-agents-per-warp / warp-per-agent kernel
+    # Dyna-Q: 37 and 6 agents are fewer than two waves, so both runs use the warp-per-agent kernel (the
+    # two-agents-per-warp kernel is selected from 2 * 7 * 4 agents per SM on)
     for n in (37, 6):
         st = cb.BatchStream(n, seed=1, device=dev)
         env = Gridworld(make_open_field(5, 5, 0, 1), rng=st)

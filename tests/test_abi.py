@@ -63,3 +63,57 @@ def test_integration_md_stub_matches_library(built, monkeypatch):
     ns = {}
     exec(compile(defs, 'INTEGRATION.md', 'exec'), ns)
     assert ctypes.sizeof(ns['DynaQParams']) == built.cobel_sizeof(b'CobelDynaQParams')
+
+
+# ---- argument checks of the entry points: every call below is rejected before any kernel launches, so the table
+# pointers may be small host buffers (validation only checks them for non-NULL) ---------------------------------------
+EINVAL, EUNSUPPORTED = -1, -2
+
+
+def _params(cls, buf, n_actions):
+    """A parameter struct whose pointers (nested structs included) all point at `buf`, with valid sizes."""
+    def fill(s):
+        for name, typ in s._fields_:
+            if typ is ctypes.c_void_p:
+                setattr(s, name, ctypes.addressof(buf))
+            elif issubclass(typ, ctypes.Structure):
+                fill(getattr(s, name))
+    p = cls()
+    fill(p)
+    p.n_agents = 1
+    p.world.n_states, p.world.n_actions, p.world.n_starts = 4, n_actions, 1
+    for name, value in (('trials', 1), ('steps', 1), ('learn', 1), ('n_keys', 4), ('log_cap', 1), ('max_visited', 4),
+                        ('sr_band', -1)):
+        if hasattr(p, name):
+            setattr(p, name, value)
+    return p
+
+
+def _last_error(L):
+    buf = ctypes.create_string_buffer(512)
+    L.cobel_last_error(buf, 512)
+    return buf.value.decode()
+
+
+@pytest.mark.parametrize('entry, struct, replay', [
+    ('cobel_dynaq_run', 'DynaQParams', False), ('cobel_q_run', 'QParams', False), ('cobel_sr_run', 'SRParams', False),
+    ('cobel_sr_compact_run', 'SRCompactParams', False), ('cobel_sfma_run', 'SFMAParams', False),
+    ('cobel_pma_run', 'PMAParams', False), ('cobel_sfma_replay', 'SFMAParams', True),
+    ('cobel_pma_replay', 'PMAParams', True)])
+def test_unsupported_action_count(built, entry, struct, replay):
+    from cobel_rl_b200 import _lib
+    L = _lib.lib()
+    buf = ctypes.create_string_buffer(256)
+    p = _params(getattr(_lib, struct), buf, 5)
+    args = (ctypes.addressof(buf), 1) if replay else ()
+    assert getattr(L, entry)(ctypes.byref(p), *args, None) == EUNSUPPORTED
+    assert _last_error(L) == 'unsupported number of actions 5 (built for 2,3,4,6,8)'
+
+
+def test_sfma_run_requires_carry(built):
+    from cobel_rl_b200 import _lib
+    L = _lib.lib()
+    buf = ctypes.create_string_buffer(256)
+    p = _params(_lib.SFMAParams, buf, 4)
+    p.trials, p.carry = 0, None
+    assert L.cobel_sfma_run(ctypes.byref(p), None) == EINVAL
