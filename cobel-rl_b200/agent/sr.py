@@ -9,6 +9,7 @@ transition model ``transitions[S,A,S]`` is held as its arg-max ``model[S,A]``.
 state spaces (100x100 and beyond, csrc/sr_compact.cu): per agent only the V x V block of the
 SR over the states it has touched is stored, everything else is implied (identity rows,
 self-loop model, zero reward); results are bit-identical to the dense agent.
+Memory (``N·V²·8`` bytes of ``SRc``) is the only limit on ``max_visited``.
 """
 import numpy as np
 import torch

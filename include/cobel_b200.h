@@ -193,7 +193,9 @@ typedef struct CobelSRCompactParams {
   const uint8_t* action_mask;/* [S,A] shared by all agents; NULL = mask_actions False */
   const double* lr;          /* [N] */
   const double* gamma;       /* [N] */
-  int32_t max_visited;       /* Vmax */
+  int32_t max_visited;       /* Vmax, 2..65535.  Up to the on-chip limit (1309 / 1066 / 900 / 685 / 553 at 2 / 3 / 4 / 6 / 8
+                                actions) visited / rewards / model are staged in shared memory; above it they stay in
+                                HBM (one CTA per agent), limited only by the n_states slot map fitting in shared memory */
   int32_t trials, steps;
   int32_t learn;
 } CobelSRCompactParams;
