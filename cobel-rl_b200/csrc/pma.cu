@@ -300,8 +300,12 @@ __global__ void __launch_bounds__(kThreads, TILE <= 7 ? 2 : 1) pma_sr_kernel(con
     gth_stationary<TILE>(Tg, Mat, xv, S, elim, tid, flags);
     for (int e = tid; e < S; e += kThreads) p.need_scratch[(size_t)n * S + e] = xv[e];
   }
-  flags = __syncthreads_or(flags);
-  if (tid == 0 && flags && p.trace.flags) p.trace.flags[n] |= flags;
+  __shared__ int block_flags;                        // the OR of the threads' COBEL_FLAG_* bits (__syncthreads_or gives 0 / 1)
+  if (tid == 0) block_flags = 0;
+  __syncthreads();
+  if (flags) atomicOr(&block_flags, flags);
+  __syncthreads();
+  if (tid == 0 && block_flags && p.trace.flags) p.trace.flags[n] |= block_flags;
 }
 
 // ---------------------------------------------------------------------------
@@ -550,7 +554,8 @@ __device__ __noinline__ int band_gth(const double* __restrict__ Tg, double* fac,
 //           row carry[.,0] for the end replay of a trial that reached a terminal state, row carry[.,4] (the next
 //           trial's start state) for the start replay
 // ---------------------------------------------------------------------------
-constexpr int kBandWarps = 8;
+constexpr int kBandWarps = 8;                         // agents per CTA (kBandWarpsWide when their rings do not fit)
+constexpr int kBandWarpsWide = 6;
 struct BandSmem {                                     // per warp (agent)
   int ring, x, w, bytes;
   __host__ __device__ BandSmem(int S, int bw) {
@@ -563,14 +568,20 @@ struct BandSmem {                                     // per warp (agent)
   }
 };
 
+// Agents (warps) per CTA of the band kernels: kBandWarps, or kBandWarpsWide when eight rings do not fit in shared
+// memory -- from half band 27 on the ring has 64 rows, and eight agents would need up to 288 KB; six fit for every
+// sr_band <= 31 and S <= 512 (at most 216 KB).
+inline int band_warps(int S, int bw) { return kBandWarps * BandSmem(S, bw).bytes <= kMaxSmem ? kBandWarps : kBandWarpsWide; }
+
 // (A one-thread-per-agent factor kernel -- window of bw + 2 rows lane-interleaved in shared memory, 5.5
 //  instructions per element update, 3x fewer instructions per agent -- measured 1.28 ms against 1.0 ms for this one
 //  at 16384 agents: 32 KB of window per 16 agents leave 1.75 warps per scheduler on strictly dependent steps.)
-__global__ void __launch_bounds__(kBandWarps * 32) pma_band_factor_kernel(const __grid_constant__ CobelPMAParams p,
+template <int WARPS>
+__global__ void __launch_bounds__(WARPS * 32) pma_band_factor_kernel(const __grid_constant__ CobelPMAParams p,
                                                                          const int solve_start) {
   extern __shared__ __align__(16) unsigned char smem[];
   const int S = p.world.n_states, bw = p.sr_band, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int64_t n = (int64_t)blockIdx.x * kBandWarps + warp;
+  const int64_t n = (int64_t)blockIdx.x * WARPS + warp;
   if (n >= p.n_agents) return;
   const BandSmem so(S, bw);
   unsigned char* blk = smem + (size_t)warp * so.bytes;
@@ -609,10 +620,11 @@ __global__ void __launch_bounds__(kBandWarps * 32) pma_band_factor_kernel(const 
   if (lane == 0 && flags && p.trace.flags) p.trace.flags[n] |= flags;
 }
 
-__global__ void __launch_bounds__(kBandWarps * 32) pma_band_solve_kernel(const __grid_constant__ CobelPMAParams p, const int which) {
+template <int WARPS>
+__global__ void __launch_bounds__(WARPS * 32) pma_band_solve_kernel(const __grid_constant__ CobelPMAParams p, const int which) {
   extern __shared__ __align__(16) unsigned char smem[];
   const int S = p.world.n_states, bw = p.sr_band, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int64_t n = (int64_t)blockIdx.x * kBandWarps + warp;
+  const int64_t n = (int64_t)blockIdx.x * WARPS + warp;
   if (n >= p.n_agents) return;
   const int64_t c = p.carry[n * 8 + which];          // which = 0: the last state of the trial, 4: the next start state
   if (c < 0) return;                                  // timed-out trial: need_scratch holds the stationary need
@@ -1590,6 +1602,12 @@ int run(const CobelPMAParams& p, cudaStream_t st) {
                 "PMA: more than 160 states need the banded update_sr (sr_band >= 0; the dense S x S eliminations are "
                 "register-tiled for S <= 160), got %d states", S);
   const auto sr_kernel = sr_kernel_for(S, sm_sr);
+  // every size is checked before the first launch: a call that cannot finish leaves Q, T and the stream untouched
+  size_t sm_band = 0;
+  const auto band_kernel = band ? sr_band_kernel_for(S, p.sr_band, sm_band) : nullptr;
+  COBEL_REQUIRE(!band || !big || sm_band <= kMaxSmem, COBEL_EUNSUPPORTED,
+                "PMA: the final SR refresh of %d states at half band %d needs %zu bytes of shared memory (at most %d); "
+                "beyond 160 states there is no dense update_sr to fall back on", S, p.sr_band, sm_band, kMaxSmem);
   auto main_kernel = big ? pma_main_kernel<A, false, true> : pma_main_kernel<A, false>;
   if constexpr (A <= 4) {
     if (plain) main_kernel = pma_main_kernel<A, true>;
@@ -1608,15 +1626,18 @@ int run(const CobelPMAParams& p, cudaStream_t st) {
     //            -> solve(need = SR[start]) -> main(start replay, steps of trial t+1)
     //   (a world with ONE starting state: factor also solves SR[start], and the two main launches are one)
     // and SR = inv(I - gamma T) once, densely, from the last factors
-    const unsigned grid_band = (unsigned)((p.n_agents + kBandWarps - 1) / kBandWarps);
-    const size_t sm_bandk = (size_t)kBandWarps * BandSmem(S, p.sr_band).bytes;
+    const int warps = band_warps(S, p.sr_band);
+    const unsigned grid_band = (unsigned)((p.n_agents + warps - 1) / warps);
+    const size_t sm_bandk = (size_t)warps * BandSmem(S, p.sr_band).bytes;
+    const auto factor_kernel = warps == kBandWarps ? pma_band_factor_kernel<kBandWarps> : pma_band_factor_kernel<kBandWarpsWide>;
+    const auto solve_kernel = warps == kBandWarps ? pma_band_solve_kernel<kBandWarps> : pma_band_solve_kernel<kBandWarpsWide>;
     if (!p.band_trusted)                               // the caller's band guarantee on the initial T
       rc = launch_kernel(pma_band_check_kernel, (unsigned)p.n_agents, 256, 0, st, p);
     if (!rc) rc = main_launch(MainPhase{1, 0, 1, 1, 0, 0});
     const bool one_start = p.world.n_starts == 1;      // the start row is known before the reset draw
     for (int t = 0; t < p.trials && !rc; ++t) {
       const int more = t + 1 < p.trials ? 1 : 0;
-      rc = launch_kernel(pma_band_factor_kernel, grid_band, kBandWarps * 32, sm_bandk, st, p, one_start && more);
+      rc = launch_kernel(factor_kernel, grid_band, warps * 32, sm_bandk, st, p, one_start && more);
       if (rc) break;
       if (one_start) {                                 // end replay t, reset, start replay and steps of trial t + 1
         rc = main_launch(MainPhase{0, 1, more, more, t + 1, 2});
@@ -1624,15 +1645,12 @@ int run(const CobelPMAParams& p, cudaStream_t st) {
       }
       rc = main_launch(MainPhase{0, 1, more, 0, t + 1, 1});
       if (rc || !more) break;
-      rc = launch_kernel(pma_band_solve_kernel, grid_band, kBandWarps * 32, sm_bandk, st, p, 4);
+      rc = launch_kernel(solve_kernel, grid_band, warps * 32, sm_bandk, st, p, 4);
       if (!rc) rc = main_launch(MainPhase{0, 0, 0, 1, t + 1, 1});
     }
     if (rc) return rc;
-    size_t sm_band;
-    const auto band_kernel = sr_band_kernel_for(S, p.sr_band, sm_band);
     if (sm_band <= kMaxSmem) return launch_kernel(band_kernel, (unsigned)p.n_agents, (S + 31) & ~31, sm_band, st, p);
-    COBEL_REQUIRE(!big, COBEL_EUNSUPPORTED, "PMA: the band factors of %d states do not fit in shared memory", S);
-    return sr_launch(1);
+    return sr_launch(1);                               // (S <= 160: checked above)
   }
   // trial t: main(reset, start replay, steps) -> sr(update_sr [+ stationary]) -> main(end replay, then trial t+1)
   rc = main_launch(MainPhase{1, 0, 1, 1, 0, 0});

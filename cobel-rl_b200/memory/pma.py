@@ -13,6 +13,12 @@ from ..stream import cuda_stream
 from .dyna_q import TableMemory
 
 
+def _check_singular(flags):
+    """COBEL_FLAG_SINGULAR of a stand-alone call: raise instead of returning a vector that means nothing."""
+    if bool((flags & 8).any()):
+        raise _lib.CobelError('PMA: singular elimination (T has a closed class without a unique stationary distribution)')
+
+
 class PMAMemory(TableMemory):
     def __init__(self, sas, policy, learning_rate=0.9, learning_rate_q=0.9, gamma=0.9, gamma_q=0.9, rng=None):
         sas = np.asarray(sas)
@@ -58,7 +64,7 @@ class PMAMemory(TableMemory):
         self._need_scratch = torch.zeros((2, n, S), dtype=torch.float64, device=dev)   # kernel scratch
         self._band_T = self._matrix_band(self._T0)     # half bandwidth of T; None = must be re-measured
         self._band_scratch = None
-        self.sr_band_max = 24                          # wider T: dense update_sr every trial (csrc/pma.cu)
+        self.sr_band_max = 24                          # wider T: dense update_sr every trial (csrc/pma.cu); at most 31
         self.compute_update_mask()
 
     @staticmethod
@@ -116,15 +122,18 @@ class PMAMemory(TableMemory):
         p = self._mem_params(keep)
         n, dev = st.n_agents, st.device
         tmp = {'Q': torch.zeros((n, S, A), dtype=torch.float64, device=dev), 'one': torch.ones(n, dtype=torch.float64, device=dev),
-               'cnt': torch.zeros((2, n), dtype=torch.int64, device=dev), 'state': torch.zeros(n, dtype=torch.int32, device=dev)}
+               'cnt': torch.zeros((2, n), dtype=torch.int64, device=dev), 'state': torch.zeros(n, dtype=torch.int32, device=dev),
+               'flags': torch.zeros(n, dtype=torch.int32, device=dev)}
         keep.append(tmp)
         p.Q, p.lr, p.gamma = tmp['Q'].data_ptr(), tmp['one'].data_ptr(), tmp['one'].data_ptr()
         p.policy = self.policy.c_struct(st, keep)
         p.trace.n_steps, p.trace.n_replay = tmp['cnt'][0].data_ptr(), tmp['cnt'][1].data_ptr()
+        p.trace.flags = tmp['flags'].data_ptr()
         p.batch = 0
         dc = st.draw_count.clone()
         _lib.call('cobel_pma_replay', dev, p, tmp['state'].data_ptr(), 1, cuda_stream(dev))
         st.draw_count.copy_(dc)                      # a replay of length 0 draws nothing; keep the stream untouched either way
+        _check_singular(tmp['flags'])
 
     def check_supported(self):
         pass        # every replay switch of the reference's PMAMemory is implemented
@@ -246,8 +255,7 @@ class PMAMemory(TableMemory):
             _lib.call('cobel_pma_replay', dev, p, state.data_ptr(), 1 if update_sr else 0, cuda_stream(dev))
         finally:
             agent._action_mask, agent.mask_actions = saved_mask, saved_flag
-        if bool((flags & 8).any()):
-            raise _lib.CobelError('PMA: singular elimination (T has a closed class without a unique stationary distribution)')
+        _check_singular(flags)
         return self._view(idx), agent.Q
 
     def compute_gain_batch(self, q_function, action_mask=None):
@@ -282,13 +290,15 @@ class PMAMemory(TableMemory):
             n, dev = st.n_agents, st.device
             tmp = {'Q': torch.zeros((n, self.nb_states, self.nb_actions), dtype=torch.float64, device=dev),
                    'one': torch.ones(n, dtype=torch.float64, device=dev), 'cnt': torch.zeros((2, n), dtype=torch.int64, device=dev),
-                   'dc': st.draw_count.clone()}
+                   'dc': st.draw_count.clone(), 'flags': torch.zeros(n, dtype=torch.int32, device=dev)}
             keep.append(tmp)
             p.Q, p.lr, p.gamma = tmp['Q'].data_ptr(), tmp['one'].data_ptr(), tmp['one'].data_ptr()
             p.policy = self.policy.c_struct(st, keep)
             p.trace.n_steps, p.trace.n_replay = tmp['cnt'][0].data_ptr(), tmp['cnt'][1].data_ptr()
+            p.trace.flags = tmp['flags'].data_ptr()
             p.batch = 0
             _lib.call('cobel_pma_replay', dev, p, state.data_ptr(), 0, cuda_stream(dev))
+            _check_singular(tmp['flags'])
         out = torch.empty((st.n_agents, self.nb_states * self.nb_actions), dtype=torch.float64, device=st.device)
         _lib.call('cobel_pma_op', st.device, p, _lib.OP_NEED, None, state.data_ptr(), out.data_ptr(), cuda_stream(st.device))
         return self._view(out)

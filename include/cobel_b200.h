@@ -306,7 +306,7 @@ typedef struct CobelPMAParams {
   int32_t trials, steps, batch;
   int32_t no_replay;
   int32_t learn;             /* 1 = train(), 0 = test() */
-  /* Banded update_sr (memory/pma.py:413-415 needs only the SR rows that replay reads, :401-411).  sr_band >= 0 is
+  /* Banded update_sr (memory/pma.py:413-415 needs only the SR rows that replay reads, :401-411).  sr_band in 0..31 is
    * the caller's guarantee that T[i][j] == 0 for |i - j| > sr_band and that every world transition satisfies
    * |s' - s| <= sr_band (a W-wide gridworld: sr_band = W): each agent then factorises its banded I - gamma T after
    * every trial (its own kernels between the phases of the main kernel) and solves for the one SR row a replay call needs, and SR is refreshed

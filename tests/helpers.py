@@ -442,3 +442,142 @@ def oracle_sample(kind, seed, agent_ids, **cfg):
     with mp.get_context('spawn').Pool(procs) as pool:
         out = pool.map(_oracle_sample_worker, jobs, chunksize=1)
     return dict(zip([int(g) for g in agent_ids], out))
+
+
+# ---- extended-precision reference for PMA's update_sr (SR = inv(I - gamma T) and the stationary need) -------------
+# np.longdouble is the 80-bit format on x86-64 (eps 1.08e-19) and binary128 on aarch64 Linux (eps 1.9e-34); both are
+# far enough below fp64 (eps 2.2e-16) that the reference's own error vanishes next to the kernels' gates.
+LD = np.longdouble
+EPS64 = float(np.finfo(np.float64).eps)
+
+
+def _ld_check():
+    assert np.finfo(LD).eps <= 1.1e-19, 'np.longdouble is not an extended format here: use mpmath for the reference'
+
+
+def _lu_ld(A):
+    """LU with partial pivoting in longdouble: (packed factors, row permutation)."""
+    A = np.array(A, dtype=LD)
+    S = A.shape[0]
+    piv = np.arange(S)
+    for k in range(S - 1):
+        p = k + int(np.argmax(np.abs(A[k:, k])))
+        if p != k:
+            A[[k, p]] = A[[p, k]]
+            piv[[k, p]] = piv[[p, k]]
+        A[k + 1:, k] /= A[k, k]
+        A[k + 1:, k + 1:] -= np.multiply.outer(A[k + 1:, k], A[k, k + 1:])
+    return A, piv
+
+
+def _lu_solve_ld(LU, piv, B):
+    X = np.array(B, dtype=LD)[piv]
+    S = LU.shape[0]
+    for k in range(S):                         # L y = P b (unit diagonal)
+        X[k + 1:] -= np.multiply.outer(LU[k + 1:, k], X[k])
+    for k in range(S - 1, -1, -1):             # U x = y
+        X[k] /= LU[k, k]
+        X[:k] -= np.multiply.outer(LU[:k, k], X[k])
+    return X
+
+
+def ref_inverse(M):
+    """inv(M) in longdouble: LU with partial pivoting, then two steps of iterative refinement whose residual
+    I - M X is formed in longdouble."""
+    _ld_check()
+    M = np.array(M, dtype=LD)
+    S = M.shape[0]
+    I = np.eye(S, dtype=LD)
+    LU, piv = _lu_ld(M)
+    X = _lu_solve_ld(LU, piv, I)
+    for _ in range(2):
+        X += _lu_solve_ld(LU, piv, I - M @ X)
+    return X
+
+
+def ref_stationary(T):
+    """Stationary distribution of the row-stochastic T by GTH elimination in longdouble, as |x| / ||x||_2 (what the
+    kernels return).  GTH forms every quantity from the non-negative entries of T without a subtraction, so each
+    entry -- the tiny ones of a nearly decoupled chain included -- has a small relative error."""
+    _ld_check()
+    P = np.array(T, dtype=LD)
+    S = P.shape[0]
+    for k in range(S - 1, 0, -1):
+        s = P[k, :k].sum()
+        P[:k, k] /= s
+        P[:k, :k] += np.multiply.outer(P[:k, k], P[k, :k])
+    x = np.zeros(S, dtype=LD)
+    x[0] = 1
+    for k in range(1, S):
+        x[k] = x[:k] @ P[:k, k]
+    x = np.abs(x)
+    return x / np.sqrt((x * x).sum())
+
+
+def nopivot_inverse(M):
+    """inv(M) in fp64 by the kernels' own algorithm -- LU without pivoting, then L y = e_c and U x = y per column --
+    in NumPy: the fp64 baseline of that elimination order, whose rounding errors differ from LAPACK's pivoted
+    getrf / getri."""
+    A = np.array(M, dtype=np.float64)
+    S = A.shape[0]
+    for k in range(S - 1):
+        A[k + 1:, k] /= A[k, k]
+        A[k + 1:, k + 1:] -= np.multiply.outer(A[k + 1:, k], A[k, k + 1:])
+    X = np.eye(S)
+    for k in range(S):
+        X[k + 1:] -= np.multiply.outer(A[k + 1:, k], X[k])
+    for k in range(S - 1, -1, -1):
+        X[k] /= A[k, k]
+        X[:k] -= np.multiply.outer(A[:k, k], X[k])
+    return X
+
+
+def kappa_inf(M, R):
+    """kappa_inf(M) = ||M||_inf ||inv(M)||_inf with inv(M) = R."""
+    return float(np.abs(np.asarray(M, dtype=LD)).sum(axis=1).max() * np.abs(R).sum(axis=1).max())
+
+
+# Matrix generators (fixed seeds).  Every T is row-stochastic.
+def _normalise(T):
+    return T / T.sum(axis=1, keepdims=True)
+
+
+def band_T(S, bw, seed):
+    """Random T of half bandwidth bw with EVERY offset in [-bw, bw] non-zero (where it lies inside the matrix), its
+    entries spread log-uniformly over 1e-8..1 before the rows are normalised."""
+    rng = np.random.default_rng(seed)
+    i, j = np.indices((S, S))
+    T = np.where(np.abs(i - j) <= bw, 10.0 ** rng.uniform(-8, 0, (S, S)), 0.0)
+    return _normalise(T)
+
+
+def dense_T(S, seed):
+    """Random dense T, entries log-uniform over 1e-8..1 before normalisation."""
+    rng = np.random.default_rng(seed)
+    return _normalise(10.0 ** rng.uniform(-8, 0, (S, S)))
+
+
+def decoupled_T(S, seed, eps=1e-9):
+    """Nearly decoupled chain: a block of states 0..m-1 leaks into the block m..S-1 only with probability `eps` (from
+    state m-1), and every state of the second block returns to state 0 with probability 1/2.  The second block's
+    stationary mass is about `eps` times the first's: the entries span more than 8 orders of magnitude.  S >= 2."""
+    rng = np.random.default_rng(seed)
+    m = max(1, S // 2)
+    T = np.zeros((S, S))
+    T[:m, :m] = _normalise(rng.uniform(0.1, 1.0, (m, m)))
+    T[m - 1, :m] *= 1.0 - eps
+    T[m - 1, m] = eps
+    T[m:, m:] = 0.5 * _normalise(rng.uniform(0.1, 1.0, (S - m, S - m)))
+    T[m:, 0] += 0.5
+    return T
+
+
+def reducible_T(S, seed, bw=None):
+    """Two closed classes (states below S // 2 and the rest), no transition between them: no unique stationary
+    distribution.  `bw`: each block is banded with that half width."""
+    m = S // 2
+    T = np.zeros((S, S))
+    for lo, hi, k in ((0, m, 0), (m, S, 1)):
+        n = hi - lo
+        T[lo:hi, lo:hi] = dense_T(n, seed + k) if bw is None else band_T(n, bw, seed + k)
+    return T

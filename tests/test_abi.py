@@ -117,3 +117,19 @@ def test_sfma_run_requires_carry(built):
     p = _params(_lib.SFMAParams, buf, 4)
     p.trials, p.carry = 0, None
     assert L.cobel_sfma_run(ctypes.byref(p), None) == EINVAL
+
+
+def test_pma_band_refresh_too_large_is_rejected_before_any_launch(built):
+    """Half bands 25..31 beyond 440 states: the final SR refresh (pma_sr_band_kernel<32>, S * 66 doubles of shared
+    memory) does not fit, and more than 160 states have no dense update_sr.  cobel_pma_run must say so before its
+    first launch, so that a failed call leaves Q, T and the random stream as they were."""
+    from cobel_rl_b200 import _lib
+    L = _lib.lib()
+    buf = ctypes.create_string_buffer(256)
+    p = _params(_lib.PMAParams, buf, 4)
+    p.world.n_states, p.sr_band = 450, 25
+    before = L.cobel_launch_count()
+    assert L.cobel_pma_run(ctypes.byref(p), None) == EUNSUPPORTED
+    assert _last_error(L) == ('PMA: the final SR refresh of 450 states at half band 25 needs 237600 bytes of shared '
+                              'memory (at most 232448); beyond 160 states there is no dense update_sr to fall back on')
+    assert L.cobel_launch_count() == before
