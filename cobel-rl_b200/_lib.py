@@ -131,6 +131,8 @@ _SIGNATURES = {
     'cobel_dynaq_op': (C.c_int, [C.POINTER(DynaQParams), C.c_int, C.POINTER(Experiences), c_ptr]),
     'cobel_q_op': (C.c_int, [C.POINTER(QParams), C.c_int, C.POINTER(Experiences), c_ptr]),
     'cobel_sr_op': (C.c_int, [C.POINTER(SRParams), C.c_int, C.POINTER(Experiences), c_ptr, c_ptr, c_ptr]),
+    'cobel_sr_compact_op': (C.c_int, [C.POINTER(SRCompactParams), C.c_int, C.POINTER(Experiences), c_ptr, C.c_int32,
+                                      c_ptr, c_ptr]),
     'cobel_sfma_op': (C.c_int, [C.POINTER(SFMAParams), C.c_int, C.POINTER(Experiences), c_ptr]),
     'cobel_sfma_replay': (C.c_int, [C.POINTER(SFMAParams), c_ptr, C.c_int, c_ptr]),
     'cobel_pma_op': (C.c_int, [C.POINTER(PMAParams), C.c_int, C.POINTER(Experiences), c_ptr, c_ptr, c_ptr]),

@@ -9,7 +9,11 @@ transition model ``transitions[S,A,S]`` is held as its arg-max ``model[S,A]``.
 state spaces (100x100 and beyond, csrc/sr_compact.cu): per agent only the V x V block of the
 SR over the states it has touched is stored, everything else is implied (identity rows,
 self-loop model, zero reward); results are bit-identical to the dense agent.
-Memory (``N·V²·8`` bytes of ``SRc``) is the only limit on ``max_visited``.
+Memory (``N·V²·8`` bytes of ``SRc``) is the only limit on ``max_visited``.  The stand-alone methods
+``update``, ``retrieve_q`` and ``predict_on_batch`` act on the compact tables too (``cobel_sr_compact_op``, one
+launch per call): ``update`` inserts ``state``, then ``next_state``, into the visited set exactly as a learning
+step of ``train()`` does, so hand-written loops and fused training interleave freely; ``retrieve_q`` /
+``predict_on_batch`` insert nothing and return the dense agent's values (an unvisited state's row is ``e_s``).
 """
 import numpy as np
 import torch
@@ -18,6 +22,9 @@ from .. import _lib
 from ..experience import Experience, ExperienceBatch  # noqa: F401  (Experience: agent/sr.py:16-22)
 from ..spaces import Discrete
 from .agent import Agent, launch_stream
+
+_VISITED_OVERFLOW = ('an agent visited more than max_visited=%d distinct states; raise max_visited or shorten the '
+                     'horizon')
 
 
 class SR(Agent):
@@ -116,8 +123,7 @@ class SR(Agent):
                                          gm.data_ptr(), self.max_visited, n_tr, steps, 1 if learn else 0)
                 _lib.call('cobel_sr_compact_run', st.device, p, launch_stream(st))
                 if bool((res['flags'] & 16).any()):
-                    raise _lib.CobelError('an agent visited more than max_visited=%d distinct states; raise max_visited '
-                                          'or shorten the horizon' % self.max_visited)
+                    raise _lib.CobelError(_VISITED_OVERFLOW % self.max_visited)
             else:
                 p = _lib.SRParams(st.n_agents, interface.c_world(), st.c_struct(), pol.c_struct(st, keep), tr,
                                   self._SR.data_ptr(), self._rewards.data_ptr(), self._model.data_ptr(), mptr, mstride,
@@ -143,7 +149,6 @@ class SR(Agent):
     # ---- stand-alone methods -----------------------------------------------------------------------------------
     def _op_params(self):
         st = self._stream
-        assert not self.compact, 'the stand-alone SR methods act on the dense tables'
         S, A = self._SR.shape[1], self._model.shape[2]
         lr, gm = st.param(self.learning_rate, 'learning_rate'), st.param(self.gamma, 'gamma')
         world = _lib.World(S, A, 0, 0, None, None, None, None, None, None, None)
@@ -151,21 +156,56 @@ class SR(Agent):
                           self._rewards.data_ptr(), self._model.data_ptr(), None, 0, lr.data_ptr(), gm.data_ptr(), 0, 0, 1, 0)
         return p, (lr, gm)
 
+    def _compact_op(self, op, e=None, states=None, q=None, flags=None):
+        """One launch of ``cobel_sr_compact_op`` (csrc/sr_compact.cu) on the compact tables."""
+        st = self._stream
+        S, A = int(self.observation_space.n), self._model.shape[2]
+        lr, gm = st.param(self.learning_rate, 'learning_rate'), st.param(self.gamma, 'gamma')
+        world = _lib.World(S, A, 0, 0, None, None, None, None, None, None, None)
+        tr = _lib.Trace()
+        tr.flags = _lib.ptr(flags)
+        p = _lib.SRCompactParams(st.n_agents, world, st.c_struct(), _lib.Policy(0, 0, None), tr, self._SRc.data_ptr(),
+                                 self._rewards.data_ptr(), self._model.data_ptr(), self._visited.data_ptr(),
+                                 self._n_visited.data_ptr(), None, lr.data_ptr(), gm.data_ptr(), self.max_visited, 0, 0, 1)
+        n_query = 0 if states is None else states.shape[1]
+        _lib.call('cobel_sr_compact_op', st.device, p, op, e, _lib.ptr(states), n_query, _lib.ptr(q), launch_stream(st))
+
+    def _compact_retrieve_q(self, states):
+        """Q of the compact tables for ``states[N, B]`` -> ``[N, B, A]``, one launch."""
+        st = self._stream
+        S = int(self.observation_space.n)
+        if bool(((states < 0) | (states >= S)).any()):
+            raise IndexError('state outside the tables')
+        states = states.to(torch.int32).contiguous()
+        q = torch.empty((st.n_agents, states.shape[1], self._model.shape[2]), dtype=torch.float64, device=st.device)
+        self._compact_op(_lib.OP_RETRIEVE_Q, states=states, q=q)
+        return q
+
     def update(self, experience):
         """agent/sr.py:255-286 for all agents: learned reward, transition model and the SR row of ``state``."""
         st = self._stream
         batch = ExperienceBatch.from_dicts(st, experience)
-        S = self._SR.shape[1]
+        S = int(self.observation_space.n)
         if bool(((batch.state < 0) | (batch.state >= S) | (batch.next_state < 0) | (batch.next_state >= S)).any()):
             raise IndexError('experience with a state outside the tables')
+        if self.compact:
+            flags = torch.zeros(st.n_agents, dtype=torch.int32, device=st.device)
+            self._compact_op(_lib.OP_STORE, e=batch.c_struct(), flags=flags)
+            if bool((flags & 16).any()):           # COBEL_FLAG_VISITED_OVERFLOW
+                raise _lib.CobelError(_VISITED_OVERFLOW % self.max_visited)
+            return experience
         p, keep = self._op_params()
         e = batch.c_struct()
         _lib.call('cobel_sr_op', st.device, p, _lib.OP_STORE, e, None, None, launch_stream(st))
         return experience
 
     def retrieve_q(self, state):
-        """agent/sr.py:288-308: ``Q[a] = np.sum(SR[m(s, a)] * rewards)`` in NumPy's pairwise order (csrc/ops.cu)."""
+        """agent/sr.py:288-308: ``Q[a] = np.sum(SR[m(s, a)] * rewards)`` in NumPy's pairwise order (csrc/ops.cu;
+        compact agents: csrc/sr_compact.cu).  ``state`` is a scalar or ``[N]``; returns ``[N, A]`` (``[A]`` single)."""
         st = self._stream
+        if self.compact:
+            s = torch.as_tensor(state, device=st.device).reshape(-1, 1)
+            return self._view(self._compact_retrieve_q(s.expand(st.n_agents, 1))[:, 0])
         s = torch.as_tensor(state, device=st.device).reshape(-1).to(torch.int32)
         s = (s.expand(st.n_agents) if s.numel() == 1 else s).contiguous()
         q = torch.empty((st.n_agents, self._model.shape[2]), dtype=torch.float64, device=st.device)
@@ -174,6 +214,13 @@ class SR(Agent):
         return self._view(q)
 
     def predict_on_batch(self, batch):
+        """Q of every state of ``batch`` for all agents: ``[N, B, A]``, or a NumPy ``[B, A]`` for a single-agent stream.
+        Compact agents evaluate the whole batch in one launch."""
         idx = np.array(batch).astype(int).reshape(-1)
+        if self.compact:
+            st = self._stream
+            s = torch.as_tensor(idx, device=st.device).reshape(1, -1)
+            out = self._compact_retrieve_q(s.expand(st.n_agents, -1))
+            return out[0].cpu().numpy() if st.single else out
         out = torch.stack([self.retrieve_q(int(s)) for s in idx], dim=-2)
         return out.cpu().numpy() if self._stream.single else out

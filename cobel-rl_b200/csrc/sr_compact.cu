@@ -30,7 +30,9 @@ constexpr int kWarpsPerCta = 4;
 // positions pos[t], t < k.  Follows DOUBLE_add's tree: n < 8 sequential; n <= 128: 8 strided
 // accumulators over the first n - n%8 elements, combined ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)),
 // then the tail sequentially; n > 128: sum(first n2) + sum(rest), n2 = n/2 - (n/2)%8.
-__device__ __noinline__ double pairwise_sparse(const int* pos, const double* val, int k, int n_total) {
+// pos[t] and val[t] are read through operator[] (arrays, or the accessors of sr_compact_op_kernel); each val[t] once.
+template <class Pos, class Val>
+__device__ __noinline__ double pairwise_sparse(Pos pos, Val val, int k, int n_total) {
   if (k == 0) return 0.0;
   if (k == 1) return xadd(0.0, val[0]);
   struct Frame { int lo, n, phase; double left; };
@@ -305,6 +307,50 @@ __device__ __noinline__ double pairwise_combine(const double* part, int n_total)
   return ret;
 }
 
+// One agent's compact tables in HBM and its global -> local slot map in shared memory, as used by a CTA of
+// kLargeThreads threads (sr_compact_large_kernel, sr_compact_op_kernel).
+template <int A>
+struct HbmAgent {
+  double* SRc;
+  double* rew;
+  int32_t* vis;
+  int32_t* model;
+  uint16_t* slot;                                    // [S] local index of a global state, 0xFFFF = not visited
+  int Vmax;
+
+  __device__ HbmAgent(const CobelSRCompactParams& p, int64_t n, uint16_t* slot_)
+      : SRc(p.SRc + (size_t)n * p.max_visited * p.max_visited), rew(p.rewards + (size_t)n * p.max_visited),
+        vis(p.visited + (size_t)n * p.max_visited), model(p.model + (size_t)n * p.max_visited * A), slot(slot_),
+        Vmax(p.max_visited) {}
+
+  // rebuilds slot[] from the first V entries of visited[] (whole CTA)
+  __device__ void build_slot(int S, int V) const {
+    for (int g = threadIdx.x; g < S; g += kLargeThreads) slot[g] = 0xFFFF;
+    __syncthreads();
+    for (int e = threadIdx.x; e < V; e += kLargeThreads) slot[vis[e]] = (uint16_t)e;
+    __syncthreads();
+  }
+
+  // as locate in sr_compact_kernel (whole CTA); the new index, its identity row, zero column, self-loop model and
+  // zero reward are written straight to HBM
+  __device__ int locate(int g, int& V, int& flags) const {
+    const int tid = threadIdx.x;
+    const int e = slot[g];
+    if (e != 0xFFFF) return e;
+    if (V >= Vmax) { flags |= COBEL_FLAG_VISITED_OVERFLOW; return Vmax - 1; }
+    const int v = V;
+    for (int j = tid; j <= v; j += kLargeThreads) SRc[(size_t)v * Vmax + j] = j == v ? 1.0 : 0.0;
+    for (int i = tid; i < v; i += kLargeThreads) SRc[(size_t)i * Vmax + v] = 0.0;
+    if (tid == 0) { vis[v] = g; rew[v] = 0.0; }
+    if (tid < A) model[(size_t)v * A + tid] = v;
+    ++V;
+    __syncthreads();                                 // every thread has read slot[g] before it changes
+    if (tid == 0) slot[g] = (uint16_t)v;
+    __syncthreads();
+    return v;
+  }
+};
+
 struct LargeSmem {
   int slot, leaf_lo, part, q, bytes;
   LargeSmem(int S, int L, int A) {
@@ -328,16 +374,13 @@ __global__ void __launch_bounds__(kLargeThreads) sr_compact_large_kernel(const _
   int32_t* leaf_lo = reinterpret_cast<int32_t*>(smem + so.leaf_lo);
   uint16_t* slot = reinterpret_cast<uint16_t*>(smem + so.slot);
 
-  double* SRc = p.SRc + (size_t)n * Vmax * Vmax;
-  double* rew = p.rewards + (size_t)n * Vmax;
-  int32_t* vis = p.visited + (size_t)n * Vmax;
-  int32_t* model = p.model + (size_t)n * Vmax * A;
+  const HbmAgent<A> ag(p, n, slot);
+  double* SRc = ag.SRc;
+  double* rew = ag.rew;
+  int32_t* model = ag.model;
   int V = p.n_visited[n];
-  for (int g = tid; g < S; g += kLargeThreads) slot[g] = 0xFFFF;
   if (tid == 0) pairwise_leaves(S, leaf_lo);
-  __syncthreads();
-  for (int e = tid; e < V; e += kLargeThreads) slot[vis[e]] = (uint16_t)e;
-  __syncthreads();
+  ag.build_slot(S, V);
 
   DrawWindowT<true> win; win.init(p.stream, n, (uint64_t)p.stream.draw_count[n]);
   const double lr = p.lr[n], gamma = p.gamma[n];
@@ -346,24 +389,7 @@ __global__ void __launch_bounds__(kLargeThreads) sr_compact_large_kernel(const _
   const CobelTrace& tr = p.trace;
   int64_t nsteps = 0;
   int flags = 0;
-
-  // as in sr_compact_kernel; the new index, its identity row, zero column, self-loop model and zero
-  // reward are written straight to HBM
-  auto locate = [&](int g) -> int {
-    const int e = slot[g];
-    if (e != 0xFFFF) return e;
-    if (V >= Vmax) { flags |= COBEL_FLAG_VISITED_OVERFLOW; return Vmax - 1; }
-    const int v = V;
-    for (int j = tid; j <= v; j += kLargeThreads) SRc[(size_t)v * Vmax + j] = j == v ? 1.0 : 0.0;
-    for (int i = tid; i < v; i += kLargeThreads) SRc[(size_t)i * Vmax + v] = 0.0;
-    if (tid == 0) { vis[v] = g; rew[v] = 0.0; }
-    if (tid < A) model[(size_t)v * A + tid] = v;
-    ++V;
-    __syncthreads();                                 // every thread has read slot[g] before it changes
-    if (tid == 0) slot[g] = (uint16_t)v;
-    __syncthreads();
-    return v;
-  };
+  auto locate = [&](int g) -> int { return ag.locate(g, V, flags); };
 
   for (int trial = 0; trial < p.trials; ++trial) {
     win.ensure(2, lane);
@@ -472,6 +498,135 @@ __global__ void __launch_bounds__(kLargeThreads) sr_compact_large_kernel(const _
   }
 }
 
+// ---------------------------------------------------------------------------
+// Stand-alone SR.update / SR.retrieve_q on the compact tables (cobel_sr_compact_op).  The tables live in HBM for
+// both fused kernels, so one kernel serves agents trained by either, at any max_visited.  One CTA of kLargeThreads
+// per agent; shared memory holds the slot map (rebuilt from visited on every call) and, for RETRIEVE_Q, the local
+// indices of the reward-carrying visited columns in global order:
+//     wcount[kLargeThreads / 32] | slot[S] uint16 | cols[min(Vmax, S)] uint16
+// ---------------------------------------------------------------------------
+struct OpSmem {
+  int slot, cols, bytes;
+  OpSmem(int S, int n_cols) {
+    slot = (kLargeThreads / 32) * 4;
+    cols = slot + S * 2;
+    bytes = cols + n_cols * 2;
+  }
+};
+
+// pairwise_sparse's operands over cols[]: the global state of column t, and SR[m][j] * rew[j] formed when it is read
+struct ColPos {
+  const uint16_t* cols;
+  const int32_t* vis;
+  __device__ int operator[](int t) const { return __ldg(vis + cols[t]); }
+};
+struct ColProd {
+  const uint16_t* cols;
+  const double* row;
+  const double* rew;
+  __device__ double operator[](int t) const { const int e = cols[t]; return xmul(row[e], __ldg(rew + e)); }
+};
+
+template <int A>
+__global__ void __launch_bounds__(kLargeThreads) sr_compact_op_kernel(const __grid_constant__ CobelSRCompactParams p,
+                                                                      OpSmem so, int op, CobelExperiences e,
+                                                                      const int32_t* states, int n_query, double* q_out) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  const int S = p.world.n_states, Vmax = p.max_visited;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int64_t n = blockIdx.x;
+  int32_t* wcount = reinterpret_cast<int32_t*>(smem);
+  uint16_t* slot = reinterpret_cast<uint16_t*>(smem + so.slot);
+  uint16_t* cols = reinterpret_cast<uint16_t*>(smem + so.cols);
+  const HbmAgent<A> ag(p, n, slot);
+  int V = p.n_visited[n];
+  ag.build_slot(S, V);
+
+  if (op == COBEL_OP_STORE) {
+    // ---- SR.update (agent/sr.py:255-286) as one learning step of the fused kernels: s, then s', are located or
+    // inserted; row ls from rows ls and ls'; then rew[ls'] and model[ls][a] ----------------------------------------
+    const int64_t i = n * e.batch;
+    const int s = e.state[i], a = e.action[i], s2 = e.next_state[i];
+    const bool nonterminal = e.terminal[i] != 0;
+    const double r = e.reward[i], lr = p.lr[n], gamma = p.gamma[n];
+    int flags = 0;
+    const int ls = ag.locate(s, V, flags);
+    const int ls2 = ag.locate(s2, V, flags);
+    const double* rs = ag.SRc + (size_t)ls * Vmax;
+    const double* rs2 = ag.SRc + (size_t)ls2 * Vmax;
+    double* wr = ag.SRc + (size_t)ls * Vmax;
+    for (int j = tid; j < V; j += kLargeThreads) {
+      const double old = rs[j];
+      const double x = nonterminal ? rs2[j] : (j == ls2 ? 1.0 : 0.0);
+      double td = xadd(j == ls ? 1.0 : 0.0, xmul(gamma, x));
+      td = xsub(td, old);
+      wr[j] = xadd(old, xmul(lr, td));
+    }
+    if (tid == 0) {
+      const double r0 = ag.rew[ls2];
+      ag.rew[ls2] = xadd(r0, xmul(xsub(r, r0), lr));
+      ag.model[(size_t)ls * A + a] = ls2;
+      p.n_visited[n] = V;
+      if (p.trace.flags && flags) p.trace.flags[n] |= flags;
+    }
+    return;
+  }
+
+  // ---- SR.retrieve_q (agent/sr.py:288-308) for n_query states: one ordered pass over slot[] lists the visited
+  // columns with rew != 0 in global order (block-wide stream compaction, one tile of kLargeThreads states at a time) --
+  int k = 0;
+  for (int g0 = 0; g0 < S; g0 += kLargeThreads) {
+    const int g = g0 + tid;
+    const int ev = g < S ? slot[g] : 0xFFFF;
+    const bool nz = ev != 0xFFFF && ag.rew[ev] != 0.0;
+    const unsigned b = __ballot_sync(kFull, nz);
+    if (lane == 0) wcount[warp] = __popc(b);
+    __syncthreads();
+    int off = k;
+#pragma unroll
+    for (int w = 0; w < kLargeThreads / 32; ++w) {
+      const int c = wcount[w];
+      off += w < warp ? c : 0;
+      k += c;
+    }
+    if (nz) cols[off + __popc(b & ((1u << lane) - 1u))] = (uint16_t)ev;
+    __syncthreads();                                 // wcount is rewritten by the next tile
+  }
+  // Q[b][a] = pairwise_sparse over those columns of row m(s_b, a).  An unvisited s_b has the row e_{s_b} and zero
+  // reward: every product is a signed zero and the sum is +0.0, exactly what pairwise_sparse returns for them.
+  const ColPos pos{cols, ag.vis};
+  const int64_t items = (int64_t)n_query * A;
+  for (int64_t it = tid; it < items; it += kLargeThreads) {
+    const int64_t b = it / A;
+    const int a = (int)(it - b * A);
+    const int ls = slot[states[n * n_query + b]];
+    double q = 0.0;
+    if (ls != 0xFFFF) {
+      const ColProd val{cols, ag.SRc + (size_t)ag.model[(size_t)ls * A + a] * Vmax, ag.rew};
+      q = pairwise_sparse(pos, val, k, S);
+    }
+    q_out[n * items + it] = q;
+  }
+}
+
+template <int A>
+int launch_op(const CobelSRCompactParams& p, int op, const CobelExperiences& e, const int32_t* states, int n_query,
+              double* q_out, cudaStream_t st) {
+  const int S = p.world.n_states;
+  const int n_cols = op == COBEL_OP_RETRIEVE_Q ? (p.max_visited < S ? p.max_visited : S) : 0;
+  const OpSmem so(S, n_cols);
+  if (op == COBEL_OP_STORE)
+    COBEL_REQUIRE(so.bytes <= kMaxSmem, COBEL_EUNSUPPORTED,
+                  "cobel_sr_compact_op(STORE): the slot map of %d states needs %d bytes of shared memory (at most %d)",
+                  S, so.bytes, kMaxSmem);
+  else
+    COBEL_REQUIRE(so.bytes <= kMaxSmem, COBEL_EUNSUPPORTED,
+                  "cobel_sr_compact_op(RETRIEVE_Q): the slot map of %d states and the list of up to %d reward-carrying "
+                  "states need %d bytes of shared memory (at most %d)", S, n_cols, so.bytes, kMaxSmem);
+  return launch_kernel(sr_compact_op_kernel<A>, (unsigned)p.n_agents, kLargeThreads, (size_t)so.bytes, st, p, so, op,
+                       e, states, n_query, q_out);
+}
+
 template <int A>
 int launch(const CobelSRCompactParams& p, cudaStream_t st) {
   const CompactSmem so(p.max_visited, A);
@@ -503,4 +658,22 @@ extern "C" int cobel_sr_compact_run(const CobelSRCompactParams* pp, void* stream
   if (p.trials == 0) return COBEL_OK;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   COBEL_DISPATCH_A(p.world.n_actions, return launch<A>(p, st));
+}
+
+extern "C" int cobel_sr_compact_op(const CobelSRCompactParams* pp, int op, const CobelExperiences* e,
+                                   const int32_t* states, int32_t n_query, double* q_out, void* stream) {
+  COBEL_REQUIRE(pp != nullptr, COBEL_EINVAL, "null params");
+  const CobelSRCompactParams& p = *pp;
+  COBEL_REQUIRE(p.n_agents > 0 && p.world.n_states > 0, COBEL_EINVAL, "null / empty params");
+  COBEL_REQUIRE(p.SRc && p.rewards && p.model && p.visited && p.n_visited && p.lr && p.gamma, COBEL_EINVAL,
+                "agent tables missing");
+  COBEL_REQUIRE(p.max_visited >= 2 && p.max_visited <= 65535, COBEL_EINVAL, "max_visited must be in 2..65535");
+  const bool store_ok = op == COBEL_OP_STORE && e && e->batch > 0 && e->state && e->action && e->reward &&
+                        e->next_state && e->terminal;
+  COBEL_REQUIRE(store_ok || (op == COBEL_OP_RETRIEVE_Q && states && q_out && n_query > 0), COBEL_EINVAL,
+                "cobel_sr_compact_op: op must be COBEL_OP_STORE (SR.update, with an experience) or COBEL_OP_RETRIEVE_Q "
+                "(with states, n_query > 0 and q_out)");
+  const CobelExperiences none{};
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  COBEL_DISPATCH_A(p.world.n_actions, return launch_op<A>(p, op, e ? *e : none, states, n_query, q_out, st));
 }

@@ -382,6 +382,16 @@ int cobel_dynaq_op(const CobelDynaQParams* p, int op, const CobelExperiences* e,
 int cobel_q_op(const CobelQParams* p, int op, const CobelExperiences* e, void* stream);
 /* SR.update (STORE) / SR.retrieve_q: agent/sr.py:255-308 */
 int cobel_sr_op(const CobelSRParams* p, int op, const CobelExperiences* e, const int32_t* state, double* q_out, void* stream);
+/* SR.update (STORE: e[.,0] per agent) / SR.retrieve_q for B states per agent (RETRIEVE_Q: states[N,B] -> q_out[N,B,A])
+ * on the compact tables of cobel_sr_compact_run.  Consumes no draws.  One launch per call, one CTA per agent
+ * (csrc/sr_compact.cu); reads SRc / rewards / model / visited / n_visited / lr / gamma / max_visited /
+ * world.n_states / world.n_actions / n_agents and, of the trace, only flags.  STORE locates or inserts s, then s',
+ * exactly like a learning step of train() (an insertion beyond max_visited raises COBEL_FLAG_VISITED_OVERFLOW in
+ * trace.flags); RETRIEVE_Q inserts nothing and is bit-identical to cobel_sr_op on the dense tables.  Every state
+ * must lie in 0..S-1.  COBEL_EUNSUPPORTED when the slot map of S states (and, for RETRIEVE_Q, a list of up to
+ * min(max_visited, S) columns) does not fit in shared memory. */
+int cobel_sr_compact_op(const CobelSRCompactParams* p, int op, const CobelExperiences* e, const int32_t* states,
+                        int32_t n_query, double* q_out, void* stream);
 /* SFMAMemory.store, SFMA.update_q (learn = 0: no_update), GATHER: memory/sfma.py:195-236, agent/sfma.py:423-458 */
 int cobel_sfma_op(const CobelSFMAParams* p, int op, const CobelExperiences* e, void* stream);
 /* SFMAMemory.replay(batch, state) [apply_updates = 0] / SFMA.replay(batch, state) [apply_updates = 1] /
