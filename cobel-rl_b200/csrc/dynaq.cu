@@ -10,9 +10,11 @@
 //     the PLAIN kernel keeps 256 draws in shared memory, i.e. seven steps per refill),
 //   * selects the action and steps the environment warp-uniformly (PLAIN: tie-pattern CDF table),
 //   * draws the 32 replay indices one per lane, gathers the 32 experiences in parallel and
-//     applies the 32 TD updates in dependency levels (td_batch_level_parallel): updates that
-//     do not touch each other's rows run in the same round, so the reference's strictly
-//     sequential 32-update chain collapses to about five rounds with bit-identical results.
+//     applies the 32 TD updates in dependency levels (td_batch_level_parallel): one speculative
+//     pass against the pre-batch table drops the updates that provably leave Q bit-identical
+//     (80 % of the C2 batches are no-ops as a whole), the rest run in rounds of updates that do
+//     not touch each other's rows, so the reference's strictly sequential 32-update chain
+//     collapses to 0.66 rounds on average (5.3 without the pass) with bit-identical results.
 // (v1 of this kernel used one thread per agent: 180 warp-instructions per update at one
 //  instruction per 5 cycles, profiles/r1_dynaq_v1_thread_per_agent.txt.)
 #include "warp_agent.cuh"
@@ -465,8 +467,8 @@ int launch(const CobelDynaQParams& p, cudaStream_t st) {
   if constexpr (A <= 4) {
     // The production case from two waves of the warp-per-agent kernel on: two agents per warp.  It pays once the
     // machine is full either way: with fewer agents the halved number of warps costs more issue rate than the shared
-    // instructions save (4096 agents: 1.39e9 against 1.58e9 agent-steps/s; 16384: 2.26e9 against 2.05e9; 262144: 2.66e9
-    // against 2.27e9).
+    // instructions save.  B200 at 1000 W, both kernels with the speculative replay pass: 4096 agents 2.30e9 against
+    // 2.73e9 agent-steps/s, 16384 agents 3.58e9 against 3.40e9 (before that pass: 1.39e9 / 1.58e9 and 2.26e9 / 2.05e9).
     const PairSmem po(S, A);
     const size_t smp = (size_t)wo.bytes + (size_t)kPairWarps * 2 * po.bytes;
     static const int n_sm = [] { int d = 0, v = 148; if (cudaGetDevice(&d) == cudaSuccess) cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, d); return v; }();

@@ -299,6 +299,19 @@ COBEL_DEV int select_action_eps_tab(const double (&v)[A], const double* tab, dou
 //              faster (one ballot per round).
 // Rounds execute all currently ready lanes at once; each update sees exactly the values it
 // would see in sequential order, so the result is bit-identical to the sequential loop.
+//
+// Most replayed updates leave Q bit-identical (early on most of the table is still 0; with a large
+// learning rate in a deterministic world the entries soon reach exact fixed points), so every lane
+// first evaluates its update against the pre-batch table without writing ("speculative pass"), and
+// the updates that provably change nothing are dropped before the rounds:
+//   null j  = the speculative Q[s_j,a_j] + lr*td has the same bits as Q[s_j,a_j];
+//   valid j = every earlier update that writes what j reads (row s2_j, entry (s_j,a_j)) is valid and null.
+// A valid j reads the pre-batch values in sequential order too, so its speculative value is its true
+// value; if it is also null it writes what is already there, and removing it from the sequence changes
+// no read or write before or after it.  If every lane is null, every lane is valid (induction from
+// lane 0) and the batch is a no-op: no dependency analysis at all.  Otherwise the rounds run on the
+// kept updates only, and the first round -- kept lanes whose dependences were all dropped, so their
+// inputs are pre-batch values -- commits the speculative values without reloading.
 // `wm`/`rm` are per-agent scratch arrays of S words in shared memory, zero between calls.
 // ---------------------------------------------------------------------------
 // `mbits` (optional) holds one byte per state with bit a set = action a may enter the max over
@@ -308,7 +321,37 @@ template <int A>
 COBEL_DEV void td_batch_level_parallel(double* Q, uint32_t* wm, uint32_t* rm, int S, int lane, bool active,
                                        int s, int a, double r, int s2, int nt, double lr, double gamma,
                                        const uint8_t* mbits = nullptr, double* td_out = nullptr) {
-  const unsigned act = __ballot_sync(kFull, active);
+  const double g = nt ? gamma : 0.0;
+  // this lane's update on the current table: returns Q[s,a] + lr*td, sets q = Q[s,a]
+  auto evaluate = [&](double& q) -> double {
+    double row[A];
+    load_row<A>(Q + s2 * A, row);
+    q = Q[s * A + a];
+    double mx;
+    if (mbits) {
+      const uint32_t mb = mbits[s2];
+      mx = -__longlong_as_double(0x7FF0000000000000ll);
+#pragma unroll
+      for (int x = 0; x < A; ++x) mx = (mb >> x & 1u) ? xmax(mx, row[x]) : mx;
+    } else {
+      mx = row_max<A>(row);
+    }
+    double td = xadd(r, xmul(g, mx));
+    td = xsub(td, q);
+    if (td_out) *td_out = td;
+    return xadd(q, xmul(lr, td));
+  };
+  // speculative pass against the pre-batch table; bit equality, so that -0.0 and +0.0 differ
+  double qn = 0.0;
+  bool null = true;                                                 // inactive lanes count as null
+  if (active) {
+    double q;
+    qn = evaluate(q);
+    null = __double_as_longlong(qn) == __double_as_longlong(q);
+  }
+  unsigned bad = __ballot_sync(kFull, !null);
+  if (bad == 0) return;                                             // every update is a no-op
+
   const unsigned below = (1u << lane) - 1u;
   // writers / readers per state (wm / rm are all-zero on entry and are re-zeroed on exit)
   if (active) {
@@ -325,37 +368,30 @@ COBEL_DEV void td_batch_level_parallel(double* Q, uint32_t* wm, uint32_t* rm, in
     same_a = a == x ? bx : same_a;
   }
   __syncwarp();
-  unsigned dep = 0;                                                 // earlier lanes this update has to wait for
+  unsigned raw = 0, dep = 0;                                        // earlier lanes this update has to wait for
   if (active) {
-    const unsigned same_sa = wm[s] & same_a;                        // i writes the entry j reads+writes
-    dep = (wm[s2] | same_sa | rm[s]) & below;                       // i writes into the row j reads / j writes into the row i reads
+    raw = (wm[s2] | (wm[s] & same_a)) & below;                      // i writes into the row / the entry j reads
+    dep = raw | (rm[s] & below);                                    // j writes into the row i reads
   }
   __syncwarp();
   if (active) { wm[s] = 0; rm[s2] = 0; }
-  const double g = nt ? gamma : 0.0;
-  unsigned done = ~act;
-  while (done != kFull) {
-    const bool ready = active && !(done >> lane & 1u) && (dep & ~done) == 0;
+  // valid lanes: a fixpoint from "all valid"; the set only shrinks, so `bad` (= not valid-and-null) only grows
+  for (;;) {
+    const bool valid = (raw & bad) == 0;
+    const unsigned b = __ballot_sync(kFull, !(valid && null));
+    if (b == bad) break;
+    bad = b;
+  }
+  dep &= bad;                                                       // the kept updates; dropped ones order nothing
+  unsigned done = ~bad;
+  for (bool first = true; done != kFull; first = false) {
+    const bool ready = !(done >> lane & 1u) && (dep & ~done) == 0;
     const unsigned R = __ballot_sync(kFull, ready);
     // the lanes of a round touch disjoint data (every read-write and write-write overlap is a dependence above),
     // so a lane writes straight after its reads; one barrier per round orders the rounds
     if (ready) {
-      double row[A];
-      load_row<A>(Q + s2 * A, row);
-      const double q = Q[s * A + a];
-      double mx;
-      if (mbits) {
-        const uint32_t mb = mbits[s2];
-        mx = -__longlong_as_double(0x7FF0000000000000ll);
-#pragma unroll
-        for (int x = 0; x < A; ++x) mx = (mb >> x & 1u) ? xmax(mx, row[x]) : mx;
-      } else {
-        mx = row_max<A>(row);
-      }
-      double td = xadd(r, xmul(g, mx));
-      td = xsub(td, q);
-      Q[s * A + a] = xadd(q, xmul(lr, td));
-      if (td_out) *td_out = td;
+      double q;
+      Q[s * A + a] = first ? qn : evaluate(q);
     }
     __syncwarp();
     done |= R;
