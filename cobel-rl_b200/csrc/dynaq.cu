@@ -15,6 +15,7 @@
 //     (80 % of the C2 batches are no-ops as a whole), the rest run in rounds of updates that do
 //     not touch each other's rows, so the reference's strictly sequential 32-update chain
 //     collapses to 0.66 rounds on average (5.3 without the pass) with bit-identical results.
+// The PLAIN kernel reads the replay gather before the action selection (see its step loop).
 // (v1 of this kernel used one thread per agent: 180 warp-instructions per update at one
 //  instruction per 5 cycles, profiles/r1_dynaq_v1_thread_per_agent.txt.)
 #include "warp_agent.cuh"
@@ -166,24 +167,68 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, HBM ? 1 : 7) dynaq_warp_ker
     int s = w_start(draw_integer(win.next(), K));
     double treward = 0.0;
     int step = 0;
-    for (;; ++step) {
+    if constexpr (PLAIN) {
+      // The replay gather (index, Mr, Mx) depends on the window and M only, not on the step's action: it is read
+      // before the action selection and the store, so its shared-memory latency overlaps theirs, and the lane whose
+      // index is the stored (s,a) takes the stored values -- what the sequential order reads.
+      for (;; ++step) {
+        win.ensure(34, lane);
+        const int i = draw_integer(win.peek(1 + lane), SA);
+        double rr = Mr[i];
+        int rs2, rnt;
+        m_next(i, rs2, rnt);
+        double row[A];
+        load_row<A>(Q + s * A, row);
+        int a;
+        if constexpr (kEpsTab) a = select_action_eps_tab<A>(row, ptab, win.next(), lane);
+        else a = select_action_warp<A, COBEL_POLICY_EPS_GREEDY>(row, (1u << A) - 1u, pt, win.next(), lane);
+        const int sa = s * A + a;
+        const int s2 = w_succ(sa);
+        const double r = w_rew(s2);
+        const int end = w_term(s2);
+        const int nt = 1 - end;
+        // memory/dyna_q.py:92-96 (store first), then agent/dyna_q.py:275-301 (online update)
+        const double m0 = Mr[sa];
+        const double m1 = xadd(m0, xmul(mlr, xsub(r, m0)));
+        double row2[A];
+        load_row<A>(Q + s2 * A, row2);
+        const double q = Q[sa];
+        const double g = nt ? gamma : 0.0;
+        double td = xadd(r, xmul(g, row_max<A>(row2)));
+        td = xsub(td, q);
+        const double qn = xadd(q, xmul(lr, td));
+        if (i == sa) { rr = m1; rs2 = s2; rnt = nt; }
+        const int rs = i / A, ra = i - rs * A;
+        __syncwarp();
+        if (lane == 0) {
+          Mr[sa] = m1;
+          m_set(sa, s2, nt);
+          Q[sa] = qn;
+        }
+        __syncwarp();
+        td_batch_level_parallel<A>(Q, wm, rm, S, lane, true, rs, ra, rr, rs2, rnt, lr, gamma);
+        win.advance(32);
+        ++nsteps;
+        treward = xadd(treward, r);
+        if (end || step + 1 == p.steps) break;
+        s = s2;
+      }
+    } else for (;; ++step) {
       win.ensure(2 + (step_replay && B <= 32 ? B : 0), lane);
       double row[A];
       load_row<A>(Q + s * A, row);
       uint32_t mask = (1u << A) - 1u;
-      if (!PLAIN && amask) {
+      if (amask) {
         mask = 0;
 #pragma unroll
         for (int a = 0; a < A; ++a) mask |= (amask[s * A + a] ? 1u : 0u) << a;
       }
-      int a;
-      if constexpr (kEpsTab) a = select_action_eps_tab<A>(row, ptab, win.next(), lane);
-      else a = select_action_warp<A, PLAIN ? COBEL_POLICY_EPS_GREEDY : -1>(row, mask, pt, win.next(), lane);
-      const int s2 = (!PLAIN && p.world.tp_off) ? stochastic_successor(p.world, s * A + a, win.next()) : w_succ(s * A + a);
+      const int a = select_action_warp<A>(row, mask, pt, win.next(), lane);
+      const int s2 = p.world.tp_off ? stochastic_successor(p.world, s * A + a, win.next()) : w_succ(s * A + a);
       const double r = w_rew(s2);
       const int end = w_term(s2);
       const int nt = 1 - end;
-      if (!PLAIN && tr.step_sa && lane == 0) {
+      if (tr.step_sa && lane == 0) {
         if (nsteps < tr.step_cap) { tr.step_sa[n * tr.step_cap + nsteps] = s * A + a; if (tr.step_next) tr.step_next[n * tr.step_cap + nsteps] = s2; }
         else flags |= COBEL_FLAG_TRACE_OVERFLOW;
       }
@@ -233,7 +278,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, HBM ? 1 : 7) dynaq_warp_ker
   if (lane == 0) {
     p.stream.draw_count[n] = (int64_t)win.position();
     tr.n_steps[n] += nsteps;
-    tr.n_replay[n] += nrep;
+    tr.n_replay[n] += PLAIN ? nsteps * 32 : nrep;
     if (tr.flags && flags) tr.flags[n] |= flags;
   }
 }
