@@ -127,7 +127,8 @@ class PMA(Agent):
     def replay(self, replay_length, current_state=None, update_sr=False):
         """The replay call of the reference's train loop (agent/pma.py:206-213, 248-256):
         ``updates, self.Q = M.replay(self.Q, mask, replay_length, current_state)``; returns the performed updates as a
-        padded ``[N, L]`` tensor of flat indices ``a*S + s`` (-1 = none)."""
+        padded ``[N, L]`` tensor of flat indices ``a*S + s`` (-1 = none).  Same sizes and rules as ``PMAMemory.replay``
+        (banded eliminations beyond 160 states or 1024 one-step backups)."""
         mask = self._action_mask if self.mask_actions else None
         updates, _ = self.M.replay(self, mask, replay_length, current_state, update_sr=update_sr)
         return updates

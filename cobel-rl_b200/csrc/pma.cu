@@ -28,6 +28,9 @@
 //                    dgeev `need`) by the subtraction-free GTH elimination.
 //   With replays on, the main kernel is launched per phase (MainPhase): update_sr sits between a trial's steps
 //   and its end replay, and the per-agent state travels in `carry`.
+//   cobel_pma_replay (the stand-alone PMAMemory.replay, replay_only<A>) runs the end-replay phase alone: after the
+//   dense update_sr kernel up to 160 states and 1024 backups, after the banded kernels beyond
+//   (pma_band_stationary_kernel when only the stationary need is wanted).
 //
 // (v1 ran everything in one CTA per agent and was barrier-bound: 7 of 8 warps waited for warp 0
 //  through ~12 block barriers per replay iteration, profiles/r1_pma_v1_cta_per_agent.txt.)
@@ -636,6 +639,27 @@ __global__ void __launch_bounds__(WARPS * 32) pma_band_solve_kernel(const __grid
   double* need = p.need_scratch + (size_t)n * S;
 #pragma unroll 1
   for (int e = lane; e < S; e += 32) need[e] = x[e];
+}
+
+// The factor pass of a stand-alone replay without update_sr: only the agents whose current state is None
+// (carry[.,0] < 0) need anything, the stationary vector of the banded GTH -> need_scratch; the others read the stored
+// SR row.  (A kernel of its own rather than a mode of pma_band_factor_kernel keeps train()'s instantiations as they are.)
+template <int WARPS>
+__global__ void __launch_bounds__(WARPS * 32) pma_band_stationary_kernel(const __grid_constant__ CobelPMAParams p) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  const int S = p.world.n_states, bw = p.sr_band, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int64_t n = (int64_t)blockIdx.x * WARPS + warp;
+  if (n >= p.n_agents || p.carry[n * 8 + 0] >= 0) return;
+  const BandSmem so(S, bw);
+  unsigned char* blk = smem + (size_t)warp * so.bytes;
+  double* x = reinterpret_cast<double*>(blk + so.x);
+  int flags = band_gth(p.T + (size_t)n * S * S, p.band_scratch + (size_t)n * S * (2 * bw + 1),
+                       reinterpret_cast<double*>(blk + so.ring), S, bw, x, lane);
+  double* need = p.need_scratch + (size_t)n * S;
+#pragma unroll 1
+  for (int e = lane; e < S; e += 32) need[e] = x[e];
+  flags = __reduce_or_sync(kFull, flags);
+  if (lane == 0 && flags && p.trace.flags) p.trace.flags[n] |= flags;
 }
 
 // ---------------------------------------------------------------------------
@@ -1583,11 +1607,17 @@ int policy_tables(const CobelPMAParams& p, cudaStream_t st) {
   return COBEL_OK;
 }
 
+// The size errors shared by train() / test() and the stand-alone replay
+constexpr const char* kSizeLimit = "PMA kernels support at most 512 states and 2048 one-step backups, got %d states x %d actions";
+constexpr const char* kBandRequired = "PMA: more than 160 states need the banded update_sr (sr_band >= 0; the dense S x S "
+                                      "eliminations are register-tiled for S <= 160), got %d states";
+constexpr const char* kRefreshTooLarge = "PMA: the final SR refresh of %d states at half band %d needs %zu bytes of shared "
+                                         "memory (at most %d); beyond 160 states there is no dense update_sr to fall back on";
+
 template <int A>
 int run(const CobelPMAParams& p, cudaStream_t st) {
   const int S = p.world.n_states;
-  COBEL_REQUIRE(S <= 512 && S * A <= 2048, COBEL_EUNSUPPORTED,
-                "PMA kernels support at most 512 states and 2048 one-step backups, got %d states x %d actions", S, A);
+  COBEL_REQUIRE(S <= 512 && S * A <= 2048, COBEL_EUNSUPPORTED, kSizeLimit, S, A);
   const bool big = S > 160 || S * A > 1024;             // pma_main_kernel<A, false, BIG>
   size_t sm_main, sm_sr;
   if (int rc = main_smem<A>(S, sm_main)) return rc;
@@ -1598,16 +1628,12 @@ int run(const CobelPMAParams& p, cudaStream_t st) {
                      !p.world.tp_off && !p.trace.step_sa && !p.trace.replay_idx && !p.trace.replay_len && !p.stream.user_stream;
   const bool do_replay = p.learn && !p.no_replay;
   const bool band = do_replay && p.sr_band >= 0;
-  COBEL_REQUIRE(!big || !do_replay || band, COBEL_EUNSUPPORTED,
-                "PMA: more than 160 states need the banded update_sr (sr_band >= 0; the dense S x S eliminations are "
-                "register-tiled for S <= 160), got %d states", S);
+  COBEL_REQUIRE(!big || !do_replay || band, COBEL_EUNSUPPORTED, kBandRequired, S);
   const auto sr_kernel = sr_kernel_for(S, sm_sr);
   // every size is checked before the first launch: a call that cannot finish leaves Q, T and the stream untouched
   size_t sm_band = 0;
   const auto band_kernel = band ? sr_band_kernel_for(S, p.sr_band, sm_band) : nullptr;
-  COBEL_REQUIRE(!band || !big || sm_band <= kMaxSmem, COBEL_EUNSUPPORTED,
-                "PMA: the final SR refresh of %d states at half band %d needs %zu bytes of shared memory (at most %d); "
-                "beyond 160 states there is no dense update_sr to fall back on", S, p.sr_band, sm_band, kMaxSmem);
+  COBEL_REQUIRE(!band || !big || sm_band <= kMaxSmem, COBEL_EUNSUPPORTED, kRefreshTooLarge, S, p.sr_band, sm_band, kMaxSmem);
   auto main_kernel = big ? pma_main_kernel<A, false, true> : pma_main_kernel<A, false>;
   if constexpr (A <= 4) {
     if (plain) main_kernel = pma_main_kernel<A, true>;
@@ -1663,20 +1689,54 @@ int run(const CobelPMAParams& p, cudaStream_t st) {
 }
 
 // PMAMemory.replay(Q, action_mask, batch, current_state) as a stand-alone call: the end-of-trial phase of the main kernel
+// (need = SR[c] from HBM, or need_scratch for c < 0).  Up to 160 states and 1024 one-step backups the dense update_sr
+// kernel supplies the refreshed SR and the stationary need; beyond that (the BIG main kernel) the banded kernels of
+// train() do, so the band is required there:
+//   [band check] -> update_sr: band LU [+ GTH for c < 0], then pma_sr_band_kernel refreshes SR
+//                   otherwise: GTH of the agents with c < 0 only (the others read SR as stored)
+//   -> main(end replay)
 template <int A>
 int replay_only(const CobelPMAParams& p, const int32_t* state, int update_sr, cudaStream_t st) {
   const int S = p.world.n_states;
-  COBEL_REQUIRE(S <= 160 && S * A <= 1024, COBEL_EUNSUPPORTED,
-                "PMA kernels support at most 160 states (register-tiled S x S eliminations), got %d", S);
-  size_t sm_main, sm_sr;
+  COBEL_REQUIRE(S <= 512 && S * A <= 2048, COBEL_EUNSUPPORTED, kSizeLimit, S, A);
+  const bool big = S > 160 || S * A > 1024;
+  size_t sm_main;
   if (int rc = main_smem<A>(S, sm_main)) return rc;
-  const auto sr_kernel = sr_kernel_for(S, sm_sr);
-  if (int rc = policy_tables<A>(p, st)) return rc;
-  if (int rc = cobel_set_carry(p.carry, 8, state, p.n_agents, st)) return rc;
-  // M.update_sr() and / or the stationary need of the agents whose current state is None
-  if (int rc = launch_kernel(sr_kernel, (unsigned)p.n_agents, kThreads, sm_sr, st, p, update_sr ? 0 : 2)) return rc;
-  return launch_kernel(pma_main_kernel<A, false>, (unsigned)((p.n_agents + kMainWarps - 1) / kMainWarps), kMainWarps * 32,
-                       sm_main, st, p, MainPhase{0, 1, 0, 0, 0, 0});
+  const unsigned grid_main = (unsigned)((p.n_agents + kMainWarps - 1) / kMainWarps);
+  const MainPhase end_replay{0, 1, 0, 0, 0, 0};
+  if (!big) {
+    size_t sm_sr;
+    const auto sr_kernel = sr_kernel_for(S, sm_sr);
+    if (int rc = policy_tables<A>(p, st)) return rc;
+    if (int rc = cobel_set_carry(p.carry, 8, state, p.n_agents, st)) return rc;
+    // M.update_sr() and / or the stationary need of the agents whose current state is None
+    if (int rc = launch_kernel(sr_kernel, (unsigned)p.n_agents, kThreads, sm_sr, st, p, update_sr ? 0 : 2)) return rc;
+    return launch_kernel(pma_main_kernel<A, false>, grid_main, kMainWarps * 32, sm_main, st, p, end_replay);
+  }
+  // every size is checked before the first launch, as in run<A>
+  COBEL_REQUIRE(p.sr_band >= 0, COBEL_EUNSUPPORTED, kBandRequired, S);
+  COBEL_REQUIRE(p.sr_band <= 31 && p.band_scratch, COBEL_EINVAL,
+                "sr_band must be < 0 (dense update_sr) or 0..31 with band_scratch[N, S*(2*sr_band+1)]");
+  size_t sm_band;
+  const auto band_kernel = sr_band_kernel_for(S, p.sr_band, sm_band);
+  COBEL_REQUIRE(!update_sr || sm_band <= kMaxSmem, COBEL_EUNSUPPORTED, kRefreshTooLarge, S, p.sr_band, sm_band, kMaxSmem);
+  const int warps = band_warps(S, p.sr_band);
+  const unsigned grid_band = (unsigned)((p.n_agents + warps - 1) / warps);
+  const size_t sm_bandk = (size_t)warps * BandSmem(S, p.sr_band).bytes;
+  int rc = policy_tables<A>(p, st);
+  if (!rc) rc = cobel_set_carry(p.carry, 8, state, p.n_agents, st);
+  if (!rc && !p.band_trusted) rc = launch_kernel(pma_band_check_kernel, (unsigned)p.n_agents, 256, 0, st, p);
+  if (rc) return rc;
+  if (update_sr) {
+    const auto factor_kernel = warps == kBandWarps ? pma_band_factor_kernel<kBandWarps> : pma_band_factor_kernel<kBandWarpsWide>;
+    rc = launch_kernel(factor_kernel, grid_band, warps * 32, sm_bandk, st, p, 0);
+    if (!rc) rc = launch_kernel(band_kernel, (unsigned)p.n_agents, (S + 31) & ~31, sm_band, st, p);
+  } else {
+    const auto gth_kernel = warps == kBandWarps ? pma_band_stationary_kernel<kBandWarps> : pma_band_stationary_kernel<kBandWarpsWide>;
+    rc = launch_kernel(gth_kernel, grid_band, warps * 32, sm_bandk, st, p);
+  }
+  if (!rc) rc = launch_kernel(pma_main_kernel<A, false, true>, grid_main, kMainWarps * 32, sm_main, st, p, end_replay);
+  return rc;
 }
 
 }  // namespace

@@ -3,6 +3,10 @@
 Holds, per agent, the experience tables, the learned state-state transition matrix ``T``, the
 successor representation ``SR = inv(I - gamma T)`` and ``update_mask``; the replay
 (gain x need arg-max with n-step sequences) runs inside ``PMA.train()`` (csrc/pma.cu).
+
+The stand-alone ``replay()`` and ``compute_need(None)`` run on worlds of up to 512 states and 2048 one-step backups.
+Beyond 160 states or 1024 backups they take the banded eliminations of ``train()``, so T must keep the band of the
+world (``sr_band()`` >= 0); otherwise they raise ``NotImplementedError`` before anything runs.
 """
 import numpy as np
 import torch
@@ -13,8 +17,11 @@ from ..stream import cuda_stream
 from .dyna_q import TableMemory
 
 
-def _check_singular(flags):
-    """COBEL_FLAG_SINGULAR of a stand-alone call: raise instead of returning a vector that means nothing."""
+def _check_flags(flags):
+    """COBEL_FLAG_BAND_VIOLATION and COBEL_FLAG_SINGULAR of a stand-alone call: raise instead of returning a vector
+    that means nothing."""
+    if bool((flags & 32).any()):
+        raise _lib.CobelError('PMA: T lies outside the band assumed by the banded update_sr')
     if bool((flags & 8).any()):
         raise _lib.CobelError('PMA: singular elimination (T has a closed class without a unique stationary distribution)')
 
@@ -62,7 +69,8 @@ class PMAMemory(TableMemory):
         self._min_gap = torch.full((n,), float('inf'), dtype=torch.float64, device=dev)
         self._carry = torch.zeros((n, 8), dtype=torch.int64, device=dev)            # kernel scratch
         self._need_scratch = torch.zeros((2, n, S), dtype=torch.float64, device=dev)   # kernel scratch
-        self._band_T = self._matrix_band(self._T0)     # half bandwidth of T; None = must be re-measured
+        self._world_band = self._matrix_band(self._T0)  # half bandwidth of the initial T
+        self._band_T = self._world_band                # half bandwidth of T; None = must be re-measured
         self._band_scratch = None
         self.sr_band_max = 24                          # wider T: dense update_sr every trial (csrc/pma.cu); at most 31
         self.compute_update_mask()
@@ -110,7 +118,8 @@ class PMAMemory(TableMemory):
     def update_sr(self):
         """memory/pma.py:413-415 as a stand-alone call: ``SR = inv(I - gamma T)`` for all agents by the register-tiled
         Gauss-Jordan kernel of csrc/pma.cu (a replay call of length 0 with ``update_sr`` set); more than 160 states:
-        ``torch.linalg.inv`` (``train()`` itself refreshes SR on the device from its band factors)."""
+        ``torch.linalg.inv`` (``train()`` and ``replay(..., update_sr=True)`` refresh SR on the device from the band
+        factors instead)."""
         st = self._alloc_for
         S, A = self.nb_states, self.nb_actions
         if S > 160 or S * A > 1024:
@@ -133,7 +142,7 @@ class PMAMemory(TableMemory):
         dc = st.draw_count.clone()
         _lib.call('cobel_pma_replay', dev, p, tmp['state'].data_ptr(), 1, cuda_stream(dev))
         st.draw_count.copy_(dc)                      # a replay of length 0 draws nothing; keep the stream untouched either way
-        _check_singular(tmp['flags'])
+        _check_flags(tmp['flags'])
 
     def check_supported(self):
         pass        # every replay switch of the reference's PMAMemory is implemented
@@ -224,18 +233,38 @@ class PMAMemory(TableMemory):
         if current_state is None:
             return torch.full((st.n_agents,), -1, dtype=torch.int32, device=st.device)
         s = torch.as_tensor(current_state, device=st.device).reshape(-1).to(torch.int32)
+        if bool(((s < 0) | (s >= self.nb_states)).any()):
+            raise IndexError('PMA: current_state must lie in 0..%d (None for the stationary need)' % (self.nb_states - 1))
         return (s.expand(st.n_agents) if s.numel() == 1 else s).contiguous()
+
+    def _set_band(self, p):
+        """The banded update_sr arguments of a stand-alone replay beyond 160 states or 1024 one-step backups, where the
+        library has no dense eliminations: the band ``train()`` would use, or -1, which the library rejects
+        (``NotImplementedError``) before it launches anything."""
+        S, A = self.nb_states, self.nb_actions
+        if S <= 160 and S * A <= 1024:
+            return
+        band, scratch, trusted = self.sr_band(self._world_band)
+        p.sr_band, p.band_scratch, p.band_trusted = band, _lib.ptr(scratch), 1 if trusted else 0
 
     def replay(self, q_function, action_mask, replay_length, current_state, force_first=None, update_sr=False):
         """memory/pma.py:168-267 for all agents.  ``q_function`` is the PMA agent whose Q table the replay reads and
         updates IN PLACE (the reference copies Q and the agent rebinds ``self.Q``, agent/pma.py:207); ``current_state``
-        a state per agent, or None (need = stationary distribution of T).  Returns ``(performed, Q)``: the performed
-        updates as a padded ``[N, L]`` tensor of flat indices ``a*S + s`` (-1 = none) and the agent's Q table."""
+        a state per agent in 0..S-1 (else ``IndexError``), or None (need = stationary distribution of T).
+        ``update_sr``: ``update_sr()`` first, then the need from the refreshed SR, as the reference's train loop does at
+        the end of a trial.  Returns ``(performed, Q)``: the performed updates as a padded ``[N, L]`` tensor of flat
+        indices ``a*S + s`` (-1 = none) and the agent's Q table.
+
+        Beyond 160 states or 1024 one-step backups (at most 512 and 2048) the replay takes the banded eliminations of
+        ``train()``: SR is refreshed from the band LU of ``I - gamma T`` and the stationary need comes from the banded
+        GTH elimination.  T must then lie inside the band of the memory's initial T (``sr_band()`` >= 0), else
+        ``NotImplementedError``; a T the library finds outside the band it was promised raises ``CobelError``."""
         assert force_first is None, 'force_first is not implemented by the B200 path'
         agent = q_function
         assert hasattr(agent, '_Q') and agent.M is self, 'pass the PMA agent that owns this memory as q_function'
         st = self._alloc_for
         n, dev = st.n_agents, st.device
+        state = self._states_arg(current_state)
         saved_mask, saved_flag = agent._action_mask, agent.mask_actions
         if action_mask is not None:
             agent._action_mask, agent.mask_actions = torch.as_tensor(action_mask, device=dev).bool().contiguous(), True
@@ -251,11 +280,11 @@ class PMAMemory(TableMemory):
             tr = _lib.Trace(None, None, zeros[0].data_ptr(), zeros[1].data_ptr(), None, 0, idx.data_ptr(), L,
                             ln.data_ptr(), 1, flags.data_ptr(), None)
             p = self._mem_params(keep, agent, int(replay_length), tr)
-            state = self._states_arg(current_state)
+            self._set_band(p)
             _lib.call('cobel_pma_replay', dev, p, state.data_ptr(), 1 if update_sr else 0, cuda_stream(dev))
         finally:
             agent._action_mask, agent.mask_actions = saved_mask, saved_flag
-        _check_singular(flags)
+        _check_flags(flags)
         return self._view(idx), agent.Q
 
     def compute_gain_batch(self, q_function, action_mask=None):
@@ -279,7 +308,9 @@ class PMAMemory(TableMemory):
 
     def compute_need(self, current_state=None):
         """memory/pma.py:388-411: ``tile(SR[current_state], A)``, or the stationary distribution of T (|left Perron
-        vector|, unit 2-norm) tiled when ``current_state`` is None."""
+        vector|, unit 2-norm) tiled when ``current_state`` is None.  The latter comes from the dense GTH elimination up
+        to 160 states and 1024 one-step backups and from the banded one beyond (T inside the band of the memory's
+        initial T, else ``NotImplementedError``, as for ``replay``)."""
         st = self._alloc_for
         keep = []
         p = self._mem_params(keep)
@@ -297,8 +328,9 @@ class PMAMemory(TableMemory):
             p.trace.n_steps, p.trace.n_replay = tmp['cnt'][0].data_ptr(), tmp['cnt'][1].data_ptr()
             p.trace.flags = tmp['flags'].data_ptr()
             p.batch = 0
+            self._set_band(p)
             _lib.call('cobel_pma_replay', dev, p, state.data_ptr(), 0, cuda_stream(dev))
-            _check_singular(tmp['flags'])
+            _check_flags(tmp['flags'])
         out = torch.empty((st.n_agents, self.nb_states * self.nb_actions), dtype=torch.float64, device=st.device)
         _lib.call('cobel_pma_op', st.device, p, _lib.OP_NEED, None, state.data_ptr(), out.data_ptr(), cuda_stream(st.device))
         return self._view(out)

@@ -404,7 +404,12 @@ int cobel_sfma_replay(const CobelSFMAParams* p, const int32_t* state, int apply_
 int cobel_pma_op(const CobelPMAParams* p, int op, const CobelExperiences* e, const int32_t* state, double* out, void* stream);
 /* PMAMemory.replay(Q, action_mask, batch, state) (memory/pma.py:168-267): state[N] = current state, -1 = None (the
  * need is then the stationary distribution of T).  Q is updated in place, the performed updates go to
- * trace.replay_idx / replay_len.  update_sr != 0: M.update_sr() first (dense inverse, memory/pma.py:413-415). */
+ * trace.replay_idx / replay_len.  update_sr != 0: M.update_sr() first (memory/pma.py:413-415), then the need from the
+ * refreshed SR.  At most 512 states and 2048 one-step backups.  Up to 160 states and 1024 backups SR and the
+ * stationary need come from the dense eliminations (sr_band is ignored).  Beyond either bound the banded ones are
+ * used, so sr_band must be 0..31 with band_scratch (else COBEL_EUNSUPPORTED): the band LU of I - gamma T and the full
+ * SR refresh for update_sr, the banded GTH for the agents whose state is -1.  band_trusted = 0 checks T against the
+ * band first (COBEL_FLAG_BAND_VIOLATION).  Every size is checked before the first launch. */
 int cobel_pma_replay(const CobelPMAParams* p, const int32_t* state, int update_sr, void* stream);
 
 /* ---- utilities -------------------------------------------------------------- */
