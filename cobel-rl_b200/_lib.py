@@ -8,7 +8,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'libcobel_b200.so')
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 c_f64p = C.c_void_p   # device pointers travel as raw addresses
 c_ptr = C.c_void_p
@@ -75,7 +75,8 @@ class SFMAParams(C.Structure):
                 ('trials', C.c_int32), ('steps', C.c_int32), ('batch', C.c_int32), ('nb_replays', C.c_int32),
                 ('start_replay', C.c_int32), ('random_replay', C.c_int32), ('dynamic', C.c_int32),
                 ('no_replay', C.c_int32), ('learn', C.c_int32), ('td_acc', c_ptr), ('trial_mode', c_ptr),
-                ('reward_modulation', C.c_double), ('mod_flags', C.c_int32), ('exp_bound', C.c_int32), ('carry', c_ptr)]
+                ('reward_modulation', C.c_double), ('mod_flags', C.c_int32), ('exp_bound', C.c_int32), ('carry', c_ptr),
+                ('workspace', c_ptr)]
 
 
 PMA_MAX_SEQ = 64
@@ -123,6 +124,7 @@ _SIGNATURES = {
     'cobel_sr_run': (C.c_int, [C.POINTER(SRParams), c_ptr]),
     'cobel_sr_compact_run': (C.c_int, [C.POINTER(SRCompactParams), c_ptr]),
     'cobel_sfma_run': (C.c_int, [C.POINTER(SFMAParams), c_ptr]),
+    'cobel_sfma_workspace_bytes': (C.c_int64, [C.POINTER(SFMAParams)]),
     'cobel_pma_run': (C.c_int, [C.POINTER(PMAParams), c_ptr]),
     'cobel_env_reset': (C.c_int, [C.POINTER(World), C.POINTER(Stream), C.c_int64, c_ptr, c_ptr]),
     'cobel_env_step': (C.c_int, [C.POINTER(World), C.POINTER(Stream), C.c_int64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),

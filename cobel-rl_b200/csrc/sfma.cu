@@ -6,7 +6,11 @@
 //
 // Mapping: one CTA per agent; all per-agent tables (Q, M.rewards, M.states|terminals, C, I and
 // the priority scratch R) live in shared memory, the shared similarity matrix D[S,S] is read
-// from HBM/L2 one row at a time (coalesced).  The online steps of a trial are executed by
+// from HBM/L2 one row at a time (coalesced).  When those tables exceed shared memory (above 1191
+// states with M.T tracked, 1428 without, at 4 actions) the same kernel runs with them in a
+// caller-provided workspace in HBM (sfma_kernel<A, MODS, true>, compiled in sfma_hbm.cu).
+// Which of the three kernels a call takes -- the split path below, the fused kernel on chip or
+// from the workspace -- is decided by SfmaPlan.  The online steps of a trial are executed by
 // warp 0 (warp-uniform, as in the Dyna-Q kernel); each replay reactivation is a CTA-wide pass
 // over the S*A experiences: priority R = C*D*(1-I) -> threshold -> max -> exp -> inverse-CDF
 // draw by a block scan -> inhibition update.  The replayed TD updates are applied afterwards,
@@ -317,7 +321,9 @@ struct ReplaySmem {
 #ifndef SFMA_REPLAY_MINB
 #define SFMA_REPLAY_MINB 4
 #endif
-template <int A>
+// REC = M.recency: the priority is weighted by M.T (read from HBM through the listed index).  train() runs REC = false
+// only (recency keeps M.T, so it takes the fused kernel); the stand-alone replay runs either.
+template <int A, bool REC>
 __global__ void __launch_bounds__(256, SFMA_REPLAY_MINB) sfma_replay_kernel(const __grid_constant__ CobelSFMAParams p, const __grid_constant__ SfmaPhase ph) {
   extern __shared__ __align__(16) unsigned char smem[];
   __shared__ BlockShared sh;
@@ -343,6 +349,7 @@ __global__ void __launch_bounds__(256, SFMA_REPLAY_MINB) sfma_replay_kernel(cons
   const int32_t* Ms = p.Ms + g0;
   const int32_t* Mt = p.Mt + g0;
   const double* Cg = p.C + g0;
+  const double* Tg = p.T + g0;
   const uint8_t* amask = p.action_mask ? p.action_mask + n * p.mask_agent_stride : nullptr;
   int64_t* carry = p.carry + n * 4;
   const CobelTrace& tr = p.trace;
@@ -580,6 +587,7 @@ __global__ void __launch_bounds__(256, SFMA_REPLAY_MINB) sfma_replay_kernel(cons
         const int sp = l & 0xFFFF;
         const double cn = (mf & COBEL_SFMA_C_NORMALIZE) ? xdiv(Cc[j], cmax) : Cc[j];
         double r = xmul(xmul(cn, dvec(sp, Msc[j], cur, nxt)), xsub(1.0, I[sp]));    // C * D * (1 - I)
+        if (REC) r = xmul(r, Tg[(l >> 16) * S + sp]);
         if (r < thr) r = 0.0;
         R[j] = r;
         lmax = r > lmax ? r : lmax;
@@ -696,9 +704,12 @@ __global__ void __launch_bounds__(256, SFMA_REPLAY_MINB) sfma_replay_kernel(cons
 
 // MODS = the memory's strength-modulation / normalisation switches (mod_flags) may be set; the common case
 // (none) gets an instantiation without that code.
-template <int A, bool MODS>
+// HBM = the per-agent block laid out by SfmaSmem exceeds shared memory: it lives at p.workspace + n * bytes instead,
+// with the same layout and the same code (the barriers order global accesses within the CTA as well, and the
+// dependency masks of the TD batch take their atomicOr on global memory).
+template <int A, bool MODS, bool HBM>
 __global__ void __launch_bounds__(256) sfma_kernel(const __grid_constant__ CobelSFMAParams p) {
-  extern __shared__ __align__(16) unsigned char smem[];
+  extern __shared__ __align__(16) unsigned char smem_[];
   __shared__ BlockShared sh;
   const int S = p.world.n_states, K = p.world.n_starts, N = S * A, B = p.batch;
   const int tid = threadIdx.x, T = blockDim.x, lane = tid & 31, warp = tid >> 5;
@@ -708,6 +719,8 @@ __global__ void __launch_bounds__(256) sfma_kernel(const __grid_constant__ Cobel
   // replay (agent/sfma.py:324); it has to be tracked only if it is read or survives the trial
   const bool track_t = recency || p.no_replay != 0;
   const SfmaSmem so(S, A, T, B, track_t, p.random_replay != 0);
+  unsigned char* smem = smem_;
+  if constexpr (HBM) smem = p.workspace + (size_t)n * so.bytes;
   double* Q = reinterpret_cast<double*>(smem + so.q);        // [s][a]
   double* Mr = reinterpret_cast<double*>(smem + so.mr);      // [s][a]
   double* C = reinterpret_cast<double*>(smem + so.c);        // [a*S + s]
@@ -1174,6 +1187,21 @@ __global__ void __launch_bounds__(256) sfma_kernel(const __grid_constant__ Cobel
   }
 }
 
+}  // namespace
+
+#ifdef SFMA_HBM_TU
+// sfma_hbm.cu: the fused kernel with its per-agent block in p.workspace.  It is instantiated in a translation unit of
+// its own so that the on-chip instantiations above compile exactly as without it (sharing a translation unit changes
+// how the common device helpers are inlined into them).
+int sfma_fused_hbm_launch(const CobelSFMAParams& p, int threads, cudaStream_t st) {
+  COBEL_DISPATCH_A(p.world.n_actions, return launch_kernel(p.mod_flags ? sfma_kernel<A, true, true> : sfma_kernel<A, false, true>,
+                                                           (unsigned)p.n_agents, threads, 0, st, p));
+}
+#else
+int sfma_fused_hbm_launch(const CobelSFMAParams& p, int threads, cudaStream_t st);
+
+namespace {
+
 // The replay kernel's CTA size for S*A experiences and the capacity of its list of experienced (s, a) at that size
 template <int A>
 int replay_plan(const CobelSFMAParams& p, int& threads, int& cap) {
@@ -1190,24 +1218,38 @@ int replay_plan(const CobelSFMAParams& p, int& threads, int& cap) {
 template <int A>
 int replay_launch(const CobelSFMAParams& p, SfmaPhase ph, int threads, cudaStream_t st) {
   const ReplaySmem so(p.world.n_states, A, threads, p.batch, p.random_replay != 0, ph.list_cap);
-  return launch_kernel(sfma_replay_kernel<A>, (unsigned)p.n_agents, threads, so.bytes, st, p, ph);
+  return launch_kernel(p.recency ? sfma_replay_kernel<A, true> : sfma_replay_kernel<A, false>, (unsigned)p.n_agents,
+                       threads, so.bytes, st, p, ph);
 }
+
+// Which kernel a cobel_sfma_run call takes.  Split path: per-step work that touches single table entries only (no
+// decay of C, M.T neither read nor kept, no strength modulation over all experiences).  Otherwise the fused kernel,
+// with its per-agent block (SfmaSmem, `fused_bytes`) in shared memory when it fits and in p.workspace when it does not.
+struct SfmaPlan {
+  bool split;
+  int fused_threads, fused_bytes;
+  SfmaPlan(const CobelSFMAParams& p, int A) {
+    const int S = p.world.n_states, N = S * A;
+    const bool track_t = p.recency != 0 || (p.learn && p.no_replay);
+    split = p.decay_strength == 1.0 && !track_t && !(p.mod_flags & COBEL_SFMA_MOD_REWARD);
+    fused_threads = N <= 128 ? 64 : N <= 512 ? 128 : 256;
+    fused_bytes = SfmaSmem(S, A, fused_threads, p.batch, p.recency != 0 || p.no_replay != 0, p.random_replay != 0).bytes;
+  }
+  // bytes of p.workspace per agent: 0 on the split path and when the fused kernel's block fits in shared memory
+  int64_t workspace_bytes() const { return split || fused_bytes <= kMaxSmem ? 0 : fused_bytes; }
+};
 
 template <int A>
 int launch(const CobelSFMAParams& p, cudaStream_t st) {
   const int S = p.world.n_states, N = S * A;
   COBEL_REQUIRE(S <= 0x7FFF, COBEL_EUNSUPPORTED, "SFMA kernel supports at most 32767 states");
-  const int T = N <= 128 ? 64 : N <= 512 ? 128 : 256;
-  // Split path: per-step work that touches single table entries only (no decay of C, M.T neither read nor kept,
-  // no strength modulation over all experiences)
-  const bool track_t = p.recency != 0 || (p.learn && p.no_replay);
-  const bool split = p.decay_strength == 1.0 && !track_t && !(p.mod_flags & COBEL_SFMA_MOD_REWARD);
-  // (state spaces whose tables exceed shared memory run on the split path only: its step kernel works on the tables
-  //  in HBM and its replay kernel stages just the list of experienced (s, a))
-  if (split) {
+  const SfmaPlan plan(p, A);
+  // (state spaces whose tables exceed shared memory run on the split path when its conditions hold: its step kernel
+  //  works on the tables in HBM and its replay kernel stages just the list of experienced (s, a))
+  if (plan.split) {
     int TR, cap;
     if (int rc = replay_plan<A>(p, TR, cap)) return rc;
-    COBEL_CUDA_OK(cudaFuncSetAttribute(sfma_replay_kernel<A>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    COBEL_CUDA_OK(cudaFuncSetAttribute(sfma_replay_kernel<A, false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     const unsigned grid_step = (unsigned)((p.n_agents + 63) / 64);
     auto step = [&](SfmaPhase ph) { return launch_kernel(sfma_step_kernel<A>, grid_step, 64, 0, st, p, ph); };
     // The list of experienced (s, a) of a replay holds at most what the agent had when the call started plus one new
@@ -1243,10 +1285,13 @@ int launch(const CobelSFMAParams& p, cudaStream_t st) {
     if (p.trials > 0) COBEL_CUDA_OK(cudaMemsetAsync(p.T, 0, (size_t)p.n_agents * N * sizeof(double), st));
     return COBEL_OK;
   }
-  const SfmaSmem so(S, A, T, p.batch, p.recency != 0 || p.no_replay != 0, p.random_replay != 0);
-  COBEL_REQUIRE(so.bytes <= kMaxSmem, COBEL_EUNSUPPORTED,
-                "SFMA tables of %d states x %d actions need %d bytes of shared memory", S, A, so.bytes);
-  return launch_kernel(p.mod_flags ? sfma_kernel<A, true> : sfma_kernel<A, false>, (unsigned)p.n_agents, T, so.bytes, st, p);
+  if (plan.workspace_bytes() == 0)
+    return launch_kernel(p.mod_flags ? sfma_kernel<A, true, false> : sfma_kernel<A, false, false>, (unsigned)p.n_agents,
+                         plan.fused_threads, plan.fused_bytes, st, p);
+  COBEL_REQUIRE(p.workspace, COBEL_EINVAL,
+                "SFMA tables of %d states x %d actions need %d bytes of shared memory per agent: pass a workspace of "
+                "n_agents x %d bytes (cobel_sfma_workspace_bytes)", S, A, plan.fused_bytes, plan.fused_bytes);
+  return sfma_fused_hbm_launch(p, plan.fused_threads, st);
 }
 
 // SFMAMemory.replay(batch, state) / SFMA.replay(batch, state) as a stand-alone call: the replay kernel of the split path
@@ -1283,8 +1328,18 @@ extern "C" int cobel_sfma_replay(const CobelSFMAParams* pp, const int32_t* state
                 COBEL_EINVAL, "cobel_sfma_replay needs the stream, trace.replay_idx / replay_len / n_replay and the carry scratch");
   COBEL_REQUIRE(p.Mr && p.Ms && p.Mt && p.C && p.I && p.D, COBEL_EINVAL, "memory tables missing");
   COBEL_REQUIRE(apply_updates != 1 || (p.Q && p.lr && p.gamma), COBEL_EINVAL, "Q / lr / gamma missing");
-  COBEL_REQUIRE(p.batch >= 0 && p.nb_replays >= 0 && !p.recency, COBEL_EINVAL, "batch and nb_replays must be >= 0; recency runs inside train() only");
+  COBEL_REQUIRE(!p.recency || p.T, COBEL_EINVAL, "the recency option reads M.T: T missing");
+  COBEL_REQUIRE(p.batch >= 0 && p.nb_replays >= 0, COBEL_EINVAL, "batch and nb_replays must be >= 0");
   COBEL_REQUIRE(p.mode >= MODE_DEFAULT && p.mode <= MODE_SWEEPING, COBEL_EINVAL, "unknown replay mode %d", p.mode);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   COBEL_DISPATCH_A(p.world.n_actions, return replay_only<A>(p, state, apply_updates, st));
 }
+
+extern "C" int64_t cobel_sfma_workspace_bytes(const CobelSFMAParams* pp) {
+  COBEL_REQUIRE(pp != nullptr, COBEL_EINVAL, "null params");
+  const CobelSFMAParams& p = *pp;
+  COBEL_REQUIRE(p.world.n_states > 0 && p.world.n_actions > 0 && p.batch >= 0, COBEL_EINVAL, "empty world or negative batch");
+  COBEL_REQUIRE(p.world.n_states <= 0x7FFF, COBEL_EUNSUPPORTED, "SFMA kernel supports at most 32767 states");
+  return SfmaPlan(p, p.world.n_actions).workspace_bytes();
+}
+#endif  // SFMA_HBM_TU

@@ -2,9 +2,14 @@
 
 Per-agent experience tables plus the replay-relevant structures: strengths ``C`` and recency
 ``T`` (flat index ``a*S + s``) and inhibition ``I``.  The replay itself
-(priority = C * D * (1 - I), softmax sampling, inhibition) runs inside ``SFMA.train()``
-(csrc/sfma.cu); this object owns the tensors and the tunables, with the reference's names.
+(priority = C * D * (1 - I), times ``T`` with ``recency``; softmax sampling, inhibition) runs inside ``SFMA.train()``
+(csrc/sfma.cu) or as the stand-alone ``replay()``; this object owns the tensors and the tunables, with the reference's
+names.  Every option runs up to 32767 states: configurations that need the fused kernel (``recency``,
+``decay_strength != 1``, ``reward_mod``, ``train(no_replay=True)``, ``test()`` of such a memory) keep its per-agent tables
+in a device workspace, allocated on first use, once they exceed shared memory.
 """
+import ctypes
+
 import torch
 
 from .. import _lib
@@ -41,6 +46,7 @@ class SFMAMemory(TableMemory):
         self.policy_mod = self.state_mod = False
         self.reward_modulation = 1.0
         self._D_dev = None
+        self._workspace = None
         super().__init__(nb_states, nb_actions, learning_rate, rng, init_self_loops=True)
 
     def _allocate_extra(self, stream):
@@ -110,7 +116,21 @@ class SFMAMemory(TableMemory):
             self.mode_id(), 1 if self.recency else 0, 1 if self.deterministic else 0, n_tr, steps, batch,
             nbr, 1 if start_replay else 0, 1 if rnd else 0, 1 if dynamic else 0,
             1 if no_replay else 0, 1 if learn else 0, _lib.ptr(td), _lib.ptr(trial_mode),
-            float(self.reward_modulation), self.mod_flags(), 0, self._carry.data_ptr())
+            float(self.reward_modulation), self.mod_flags(), 0, self._carry.data_ptr(), None)
+
+    def _attach_workspace(self, p, st):
+        """Point ``p.workspace`` at scratch of the size ``cobel_sfma_run`` needs for this configuration (none when its
+        tables fit in shared memory or the split path runs); the buffer is kept and grown across calls."""
+        per_agent = _lib.lib().cobel_sfma_workspace_bytes(ctypes.byref(p))
+        if per_agent < 0:
+            _lib.check(per_agent)
+        if per_agent == 0:
+            return
+        n = per_agent * st.n_agents
+        if self._workspace is None or self._workspace.numel() < n:
+            self._workspace = None                  # release the smaller buffer before allocating the larger one
+            self._workspace = torch.empty(n, dtype=torch.uint8, device=st.device)
+        p.workspace = self._workspace.data_ptr()
 
     def _table_world(self):
         return _lib.World(self.nb_states, self.nb_actions, 0, 0, None, None, None, None, None, None, None)
@@ -138,7 +158,6 @@ class SFMAMemory(TableMemory):
         return batch.to_dicts()
 
     def _replay(self, replay_length, current_state, agent=None, random=False, mask=None):
-        assert not self.recency, 'the recency option runs inside SFMA.train() only'
         st = self._alloc_for
         n, dev = st.n_agents, st.device
         L = max(int(replay_length), 1)
@@ -170,7 +189,7 @@ class SFMAMemory(TableMemory):
     def replay(self, replay_length, current_state=None, current_action=None):
         """memory/sfma.py:238-347 for all agents: the reactivated experiences as a list of Experience dicts (fields
         ``[N]`` tensors, -1 where an agent's replay ended early).  ``current_state``: one state per agent or None
-        (start drawn from the strengths)."""
+        (start drawn from the strengths).  With ``recency`` the priority is weighted by ``T``, as in ``train()``."""
         assert current_action is None, 'current_action is drawn (memory/sfma.py:264); fixing it is not implemented'
         return self._replay(replay_length, current_state)
 

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define COBEL_ABI_VERSION 4
+#define COBEL_ABI_VERSION 5
 
 enum {
   COBEL_OK = 0,
@@ -259,9 +259,17 @@ typedef struct CobelSFMAParams {
                                 so far instead of S*A: less shared memory per agent, more agents per SM */
   int64_t* carry;            /* scratch [N,4], required: per-agent state between the launches of the split path (one
                                 thread per agent for the online steps, one CTA per agent for the replays) */
+  uint8_t* workspace;        /* scratch [N, cobel_sfma_workspace_bytes(p)]: the fused kernel's per-agent tables when they
+                                exceed shared memory; may be NULL when the query returns 0 */
 } CobelSFMAParams;
 
 int cobel_sfma_run(const CobelSFMAParams* p, void* stream);
+/* Bytes of CobelSFMAParams.workspace per agent that cobel_sfma_run needs for this configuration: 0 when it takes the
+ * split path (decay_strength == 1, M.T neither read (recency) nor kept (train(no_replay=True)), no reward_mod) or when
+ * the fused kernel's per-agent tables fit in shared memory; else the size of those tables, which then live in the
+ * workspace.  Reads n_states, n_actions, batch, recency, no_replay, learn, decay_strength, mod_flags, random_replay.
+ * Negative COBEL_E* code on bad arguments (more than 32767 states: COBEL_EUNSUPPORTED). */
+int64_t cobel_sfma_workspace_bytes(const CobelSFMAParams* p);
 
 /* ---- PMA: agent/pma.py:137-369 + memory/pma.py:20-496 (Mattar & Daw gain x need replay) ---- */
 #define COBEL_PMA_MAX_SEQ 64      /* longest n-step sequence = largest replay batch */
@@ -397,7 +405,8 @@ int cobel_sfma_op(const CobelSFMAParams* p, int op, const CobelExperiences* e, v
 /* SFMAMemory.replay(batch, state) [apply_updates = 0] / SFMA.replay(batch, state) [apply_updates = 1] /
  * SFMAMemory.retrieve_random_batch(batch, mask) [apply_updates = 2, random_replay = 1]
  * (memory/sfma.py:238-347, 375-416, agent/sfma.py:392-421): state[N] = current state, -1 = None.  The reactivated
- * flat indices go to trace.replay_idx / replay_len (mandatory here); needs p.carry. */
+ * flat indices go to trace.replay_idx / replay_len (mandatory here); needs p.carry.  recency = 1 weights the priority by
+ * M.T (p.T), as train() does. */
 int cobel_sfma_replay(const CobelSFMAParams* p, const int32_t* state, int apply_updates, void* stream);
 /* PMAMemory.store, PMA.update_q (pow_gamma_q must hold agent.gamma ** k), compute_gain_batch, compute_need:
  * memory/pma.py:148-166, 333-411, agent/pma.py:319-353 */
