@@ -8,7 +8,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'libcobel_b200.so')
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 c_f64p = C.c_void_p   # device pointers travel as raw addresses
 c_ptr = C.c_void_p
@@ -32,7 +32,8 @@ class Policy(C.Structure):
 class Trace(C.Structure):
     _fields_ = [('trial_steps', c_ptr), ('trial_reward', c_ptr), ('n_steps', c_ptr), ('n_replay', c_ptr),
                 ('step_sa', c_ptr), ('step_cap', C.c_int64), ('replay_idx', c_ptr), ('replay_cap', C.c_int64),
-                ('replay_len', c_ptr), ('replay_calls_cap', C.c_int64), ('flags', c_ptr), ('step_next', c_ptr)]
+                ('replay_len', c_ptr), ('replay_calls_cap', C.c_int64), ('flags', c_ptr), ('step_next', c_ptr),
+                ('step_td', c_ptr), ('reserved', c_ptr)]
 
 
 class DynaQParams(C.Structure):

@@ -10,7 +10,8 @@ agents, so per-step Python callbacks cannot run inside the loop.  What is kept:
 * ``agent.stop`` is honoured between launches when ``trials_per_launch`` splits a
   session into several launches;
 * per-step information is available from the recorded trajectory buffers
-  (``agent.record = True`` -> ``agent.last_run``).
+  (``agent.record = True`` -> ``agent.last_run``): ``step_sa``, ``step_next`` and, for the
+  Q-learning agents when the call learns, ``step_td`` (the TD error of each step's online update).
 This is the one intentional API deviation (SURVEY.md section 7.2).
 """
 import abc
@@ -48,7 +49,15 @@ class Callbacks:
 
 
 class RunResult(dict):
-    """Per-agent outputs of one ``train()`` / ``test()`` call (CobelTrace)."""
+    """Per-agent outputs of one ``train()`` / ``test()`` call (CobelTrace).
+
+    Always: ``trial_steps``, ``trial_reward`` ``[N, trials]``; ``n_steps``, ``n_replay``, ``flags`` ``[N]``.
+    With ``agent.record``: ``step_sa`` (``s*A + a``) and ``step_next`` (arrival state) ``[N, trials*steps]`` int32,
+    -1 behind ``n_steps``; ``replay_idx`` and ``replay_len``.  With ``agent.record`` in a call that learns (Dyna-Q,
+    QAgent, SFMA, PMA ``train()``, also with ``no_replay=True``): ``step_td`` ``[N, trials*steps]`` fp64, the TD error
+    that each step's online update added to ``Q[s,a]`` (scaled by the learning rate), NaN behind ``n_steps``.
+    Entry k of every per-step buffer belongs to the agent's k-th step.  Every buffer keeps its leading agent axis,
+    also for a single-agent stream."""
     __getattr__ = dict.__getitem__
 
 
@@ -60,7 +69,7 @@ class Agent(abc.ABC):
         self.current_trial = 0
         self.stop = False
         # batched-path extras
-        self.record = False            # record per-step (s,a) and replay indices of each call
+        self.record = False            # record per-step (s,a), next state, TD error and replay indices of each call
         self.trials_per_launch = None  # split a session into launches of this many trials
         self.last_run = None
         self._stream = None
@@ -93,7 +102,9 @@ class Agent(abc.ABC):
         dst.copy_(v.reshape(dst.shape) if v.numel() == dst.numel() else v.expand_as(dst))
 
     # ---- trace plumbing --------------------------------------------------------
-    def _make_trace(self, trials, steps, replay_per_step, replay_calls_per_trial, replay_len_max, keep):
+    def _make_trace(self, trials, steps, replay_per_step, replay_calls_per_trial, replay_len_max, keep, td=False):
+        """CobelTrace of one launch and the RunResult that owns its buffers; ``td`` = the launch performs online
+        Q updates whose TD errors are recorded (``step_td``) when ``agent.record`` is set."""
         st = self._stream
         n, dev = st.n_agents, st.device
         res = RunResult()
@@ -109,13 +120,15 @@ class Agent(abc.ABC):
             replay_cap = calls_cap * replay_len_max
             res['step_sa'] = torch.full((n, max(step_cap, 1)), -1, dtype=torch.int32, device=dev)
             res['step_next'] = torch.full((n, max(step_cap, 1)), -1, dtype=torch.int32, device=dev)
+            if td:
+                res['step_td'] = torch.full((n, max(step_cap, 1)), float('nan'), dtype=torch.float64, device=dev)
             res['replay_idx'] = torch.full((n, max(replay_cap, 1)), -1, dtype=torch.int32, device=dev)
             res['replay_len'] = torch.full((n, max(calls_cap, 1)), -1, dtype=torch.int32, device=dev)
         keep.append(res)
         tr = _lib.Trace(res['trial_steps'].data_ptr(), res['trial_reward'].data_ptr(), res['n_steps'].data_ptr(),
                         res['n_replay'].data_ptr(), _lib.ptr(res.get('step_sa')), step_cap,
                         _lib.ptr(res.get('replay_idx')), replay_cap, _lib.ptr(res.get('replay_len')), calls_cap,
-                        res['flags'].data_ptr(), _lib.ptr(res.get('step_next')))
+                        res['flags'].data_ptr(), _lib.ptr(res.get('step_next')), _lib.ptr(res.get('step_td')))
         return tr, res
 
     def _mask_args(self, keep):
@@ -187,16 +200,16 @@ class Agent(abc.ABC):
     @staticmethod
     def _merge(results):
         """One RunResult for a session that ran as several launches (``trials_per_launch``).  Per-trial arrays are
-        concatenated; the recorded per-step / per-replay buffers of a launch are padded with -1 behind the data of
-        each agent, so they are compacted per agent (the merged buffer is addressed by cumulative counts, exactly
-        like the buffer of a single launch)."""
+        concatenated; the recorded per-step / per-replay buffers of a launch are padded (-1, NaN for ``step_td``)
+        behind the data of each agent, so they are compacted per agent (the merged buffer is addressed by cumulative
+        counts, exactly like the buffer of a single launch)."""
         if len(results) == 1:
             return results[0]
 
-        def compact_cat(bufs, counts):
+        def compact_cat(bufs, counts, pad=-1):
             n = bufs[0].shape[0]
             total = sum(c.long() for c in counts)
-            out = torch.full((n, max(int(total.max()), 1)), -1, dtype=bufs[0].dtype, device=bufs[0].device)
+            out = torch.full((n, max(int(total.max()), 1)), pad, dtype=bufs[0].dtype, device=bufs[0].device)
             rows = torch.arange(n, device=out.device).unsqueeze(1)
             offset = torch.zeros(n, dtype=torch.long, device=out.device)
             for b, c in zip(bufs, counts):
@@ -217,6 +230,8 @@ class Agent(abc.ABC):
                     out[k] = out[k] | r[k]
             elif k in ('step_sa', 'step_next'):
                 out[k] = compact_cat([r[k] for r in results], [r['n_steps'] for r in results])
+            elif k == 'step_td':
+                out[k] = compact_cat([r[k] for r in results], [r['n_steps'] for r in results], float('nan'))
             elif k == 'replay_idx':
                 out[k] = compact_cat([r[k] for r in results], [r['n_replay'] for r in results])
             elif k == 'replay_len':

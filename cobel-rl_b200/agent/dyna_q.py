@@ -71,7 +71,7 @@ class DynaQ(Agent):
             keep = []
             tr, res = self._make_trace(n_tr, steps, 0 if (no_replay or self.episodic_replay or not learn) else 1,
                                        1 if (learn and not no_replay and self.episodic_replay) else 0,
-                                       batch_size, keep)
+                                       batch_size, keep, td=learn)
             lr, gm, mlr = (st.param(self.learning_rate, 'learning_rate'), st.param(self.gamma, 'gamma'),
                            st.param(self.M.learning_rate, 'memory learning_rate'))
             mptr, mstride = self._mask_args(keep)

@@ -87,7 +87,7 @@ class PMA(Agent):
         results = []
         for t0, n_tr in self._chunks(trials):
             keep = []
-            tr, res = self._make_trace(n_tr, steps, 0, 2 if (learn and not no_replay) else 0, batch_size, keep)
+            tr, res = self._make_trace(n_tr, steps, 0, 2 if (learn and not no_replay) else 0, batch_size, keep, td=learn)
             band, bscratch, trusted = M.sr_band(interface.transition_band) if (learn and not no_replay) else (-1, None, False)
             p = self._params(interface.c_world(), pol, tr, n_tr, steps, batch_size, no_replay, learn, band, bscratch, keep)
             p.band_trusted = 1 if trusted else 0

@@ -89,7 +89,7 @@ class QAgent(Agent):
             keep = []
             if learn:
                 self._ensure_log(n_tr * steps)
-            tr, res = self._make_trace(n_tr, steps, 1 if learn else 0, 0, batch_size, keep)
+            tr, res = self._make_trace(n_tr, steps, 1 if learn else 0, 0, batch_size, keep, td=learn)
             lr, gm = st.param(self.learning_rate, 'learning_rate'), st.param(self.gamma, 'gamma')
             key_t = None
             if obs_key is not None:

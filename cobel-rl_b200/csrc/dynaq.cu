@@ -245,6 +245,10 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, HBM ? 1 : 7) dynaq_warp_ker
         double td = xadd(r, xmul(g, row_max<A>(row2)));
         td = xsub(td, q);
         const double qn = xadd(q, xmul(lr, td));
+        if (tr.step_td && lane == 0) {               // the step's slot of step_sa (nsteps already counts it)
+          if (nsteps <= tr.step_cap) tr.step_td[n * tr.step_cap + nsteps - 1] = td;
+          else flags |= COBEL_FLAG_TRACE_OVERFLOW;
+        }
         __syncwarp();
         if (lane == 0) {
           Mr[s * A + a] = m1;
@@ -494,7 +498,8 @@ template <int A>
 int launch(const CobelDynaQParams& p, cudaStream_t st) {
   const int S = p.world.n_states, K = p.world.n_starts;
   const WorldSmem wo(S, A, K);
-  const bool plain = !p.action_mask && !p.world.tp_off && !p.trace.step_sa && !p.trace.replay_idx && !p.trace.replay_len &&
+  const bool plain = !p.action_mask && !p.world.tp_off && !p.trace.step_sa && !p.trace.step_td && !p.trace.replay_idx &&
+                     !p.trace.replay_len &&
                      p.policy.kind == COBEL_POLICY_EPS_GREEDY && p.learn && !p.no_replay && !p.episodic_replay &&
                      p.batch == 32 && !p.stream.user_stream;
   const AgentSmem ao(S, A, plain);

@@ -1505,6 +1505,10 @@ __global__ void __launch_bounds__(kMainWarps * 32, BIG ? 1 : 4) pma_main_kernel(
         const double q = Q[s * A + a];
         td = xsub(td, q);
         const double qn = xadd(q, xmul(lr, td));
+        if (!PLAIN && tr.step_td && lane == 0) {       // the step's slot of step_sa
+          if (nsteps <= tr.step_cap) tr.step_td[n * tr.step_cap + nsteps - 1] = td;
+          else flags |= COBEL_FLAG_TRACE_OVERFLOW;
+        }
         const double m0 = Mr[s * A + a];
         const double m1 = xadd(m0, xmul(mlr, xsub(r, m0)));
 #pragma unroll
@@ -1625,7 +1629,8 @@ int run(const CobelPMAParams& p, cudaStream_t st) {
                 "n_tab > 0 needs tab_kind, tab_param and tab_scratch[n_tab, COBEL_PMA_TAB_DOUBLES(A)]");
   const bool plain = !big && p.n_tab > 0 && A <= 4 && p.policy.kind == COBEL_POLICY_EPS_GREEDY &&
                      p.mem_policy.kind == COBEL_POLICY_EPS_GREEDY && p.learn && !p.no_replay && !p.options &&
-                     !p.world.tp_off && !p.trace.step_sa && !p.trace.replay_idx && !p.trace.replay_len && !p.stream.user_stream;
+                     !p.world.tp_off && !p.trace.step_sa && !p.trace.step_td && !p.trace.replay_idx && !p.trace.replay_len &&
+                     !p.stream.user_stream;
   const bool do_replay = p.learn && !p.no_replay;
   const bool band = do_replay && p.sr_band >= 0;
   COBEL_REQUIRE(!big || !do_replay || band, COBEL_EUNSUPPORTED, kBandRequired, S);

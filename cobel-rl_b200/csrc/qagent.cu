@@ -130,6 +130,10 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, HBM ? 1 : 7) q_warp_kernel(
         double td = xadd(r, xmul(g, row_max<A>(row2)));
         td = xsub(td, q);
         const double qn = xadd(q, xmul(lr, td));
+        if (!PLAIN && tr.step_td && lane == 0) {     // the step's slot of step_sa (nsteps already counts it)
+          if (nsteps <= tr.step_cap) tr.step_td[n * tr.step_cap + nsteps - 1] = td;
+          else flags |= COBEL_FLAG_TRACE_OVERFLOW;
+        }
         const bool room = len < p.log_cap;
         __syncwarp();
         if (lane == 0) {
@@ -206,7 +210,7 @@ int launch(const CobelQParams& p, cudaStream_t st) {
                   "QAgent: the replay's dependency masks of %d keys do not fit in shared memory (%zu bytes)", p.n_keys, smg);
     return launch_kernel(q_warp_kernel<A, false, true>, (unsigned)((p.n_agents + warps - 1) / warps), warps * 32, smg, st, p);
   }
-  const bool plain = !p.world.tp_off && !p.trace.step_sa && !p.trace.replay_idx && !p.trace.replay_len &&
+  const bool plain = !p.world.tp_off && !p.trace.step_sa && !p.trace.step_td && !p.trace.replay_idx && !p.trace.replay_len &&
                      p.policy.kind == COBEL_POLICY_EPS_GREEDY && p.learn && p.batch == 32 && !p.stream.user_stream;
   return launch_kernel(plain ? q_warp_kernel<A, true> : q_warp_kernel<A, false>,
                        (unsigned)((p.n_agents + kWarpsPerCta - 1) / kWarpsPerCta), kWarpsPerCta * 32, sm, st, p);

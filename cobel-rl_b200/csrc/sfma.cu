@@ -258,6 +258,10 @@ __global__ void __launch_bounds__(64) sfma_step_kernel(const __grid_constant__ C
         double td = xadd(r, xmul(nt ? gamma : 0.0, mx));
         td = xsub(td, q);
         const double qn = xadd(q, xmul(lr, td));
+        if (tr.step_td) {                                          // the step's slot of step_sa
+          if (nsteps <= tr.step_cap) tr.step_td[n * tr.step_cap + nsteps - 1] = td;
+          else flags |= COBEL_FLAG_TRACE_OVERFLOW;
+        }
         Q[(size_t)s * A + a] = qn;
         if (s2 == s) {                                             // the carried row must see the update
 #pragma unroll
@@ -1097,6 +1101,10 @@ __global__ void __launch_bounds__(256) sfma_kernel(const __grid_constant__ Cobel
           td = xsub(td, q);
           const double qn = xadd(q, xmul(lr, td));
           tdacc = xadd(tdacc, fabs(td));
+          if (tr.step_td && lane == 0) {             // the step's slot of step_sa
+            if (nsteps <= tr.step_cap) tr.step_td[n * tr.step_cap + nsteps - 1] = td;
+            else flags |= COBEL_FLAG_TRACE_OVERFLOW;
+          }
           __syncwarp();
           if (lane == 0) {
             Mr[s * A + a] = m1;

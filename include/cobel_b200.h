@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define COBEL_ABI_VERSION 5
+#define COBEL_ABI_VERSION 6
 
 enum {
   COBEL_OK = 0,
@@ -97,10 +97,16 @@ typedef struct CobelTrace {
   int32_t* flags;            /* optional [N] in/out: COBEL_FLAG_* bits raised by the agent */
   int32_t* step_next;        /* optional [N, step_cap]: arrival state of every step (needed to reconstruct
                                 trajectories in non-deterministic worlds) */
+  double*  step_td;          /* optional [N, step_cap]: TD error of the online update of every step, the value
+                                that feeds Q[s,a] += lr * td (Dyna-Q, QAgent, SFMA, PMA; ignored by the SR agents
+                                and by runs that do not learn) */
+  void*    reserved;         /* NULL.  Pads the struct to a multiple of 16 bytes: the members that follow an embedded
+                                CobelTrace keep their 16-byte alignment in the kernel parameter block, so kernels
+                                that do not read step_td compile to the same instructions as before it existed */
 } CobelTrace;
 
 enum {
-  COBEL_FLAG_TRACE_OVERFLOW = 1,  /* a step_sa / replay_idx / replay_len buffer was too small */
+  COBEL_FLAG_TRACE_OVERFLOW = 1,  /* a step_sa / step_td / replay_idx / replay_len buffer was too small */
   COBEL_FLAG_CDF_NEAR_TIE   = 2,  /* an inverse-CDF draw fell within rounding distance of a bin edge */
   COBEL_FLAG_LOG_OVERFLOW   = 4,  /* QAgent experience log full */
   COBEL_FLAG_SINGULAR       = 8,  /* PMA: (I - gamma T) pivot underflow */
