@@ -25,9 +25,10 @@ namespace {
 constexpr int kWarpsPerCta = 4;
 
 struct AgentSmem {      // byte offsets inside one agent's shared-memory block
-  int q, mr, mx, wm, rm, ptab, draws, bytes;
+  int q, mr, mx, wm, rm, ptab, draws, vmax, pat, bytes;
   // tables = false: Q / M stay in HBM (state spaces whose tables do not fit), only the dependency masks are on chip
-  __host__ __device__ AgentSmem(int S, int A, bool plain, bool tables = true) {
+  // sums = true: the row summaries V (S doubles) and P (S bytes) of the PLAIN kernel with A <= 4
+  __host__ __device__ AgentSmem(int S, int A, bool plain, bool tables = true, bool sums = false) {
     const bool eps_tab = plain && A <= 4;
     const int SA = tables ? S * A : 0;
     q = 0;
@@ -37,7 +38,9 @@ struct AgentSmem {      // byte offsets inside one agent's shared-memory block
     mx = rm + S * 4;
     ptab = (mx + SA * 2 + 15) & ~15;
     draws = ptab + (eps_tab ? kEpsTabDoubles * 8 : 0);
-    bytes = draws + (plain ? kSmemDraws * 8 : 0);
+    vmax = draws + (plain ? kSmemDraws * 8 : 0);
+    pat = vmax + (sums ? S * 8 : 0);
+    bytes = sums ? (pat + S + 15) & ~15 : vmax;
   }
 };
 
@@ -59,15 +62,19 @@ struct WorldSmem {      // byte offsets of the CTA-shared environment tables
 // M.terminals are read and written in place in HBM / L2 (a replay is 32 independent gathers per lane-parallel
 // round, so the DRAM latency of a step is paid about six times, not 33), the world tables go through the read-only
 // path, only the two dependency masks of the level-parallel replay (8 bytes per state) stay on chip.
-template <int A, bool PLAIN, bool HBM = false>
+// SUM (PLAIN, A <= 4): the agent keeps the row summaries V[s] = row_max(Q[s,:]) and P[s] = its tie pattern on chip
+// (refresh_row_summary), so the action selection, the online update's target and the replay's speculative pass read
+// one entry instead of a row and its maximum; a step that writes a row refreshes its summaries.
+template <int A, bool PLAIN, bool HBM = false, bool SUM = false>
 __global__ void __launch_bounds__(kWarpsPerCta * 32, HBM ? 1 : 7) dynaq_warp_kernel(const __grid_constant__ CobelDynaQParams p) {
   static_assert(!(PLAIN && HBM), "the HBM path is the generic kernel");
+  static_assert(!SUM || (PLAIN && A <= 4), "row summaries go with the tie-pattern table");
   extern __shared__ __align__(16) unsigned char smem[];
   const int S = p.world.n_states, K = p.world.n_starts, SA = S * A;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const WorldSmem wo(HBM ? 0 : S, A, HBM ? 0 : K);
   constexpr bool kEpsTab = PLAIN && A <= 4;      // tie-pattern CDF table instead of per-step probabilities
-  const AgentSmem ao(S, A, PLAIN, !HBM);
+  const AgentSmem ao(S, A, PLAIN, !HBM, SUM);
 
   double* rew_s = reinterpret_cast<double*>(smem + wo.rew);
   int32_t* succ_s = reinterpret_cast<int32_t*>(smem + wo.succ);
@@ -115,6 +122,10 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, HBM ? 1 : 7) dynaq_warp_ker
   __syncwarp();
 
   for (int e = lane; e < S; e += 32) { wm[e] = 0; rm[e] = 0; }
+  double* V = reinterpret_cast<double*>(blk + ao.vmax);
+  uint8_t* P = blk + ao.pat;
+  if constexpr (SUM)      // from the staged Q, which may hold any values (ties, -0.0); eps_cdf_table_init syncs
+    for (int e = lane; e < S; e += 32) refresh_row_summary<A>(Q, V, P, e);
   typename WindowFor<PLAIN>::type win; win.init(p.stream, n, (uint64_t)p.stream.draw_count[n]);
   win.attach(reinterpret_cast<double*>(blk + ao.draws));
   const double lr = p.lr[n], gamma = p.gamma[n], mlr = p.mem_lr[n];
@@ -177,11 +188,15 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, HBM ? 1 : 7) dynaq_warp_ker
         double rr = Mr[i];
         int rs2, rnt;
         m_next(i, rs2, rnt);
-        double row[A];
-        load_row<A>(Q + s * A, row);
         int a;
-        if constexpr (kEpsTab) a = select_action_eps_tab<A>(row, ptab, win.next(), lane);
-        else a = select_action_warp<A, COBEL_POLICY_EPS_GREEDY>(row, (1u << A) - 1u, pt, win.next(), lane);
+        if constexpr (SUM) {
+          a = select_action_eps_pattern<A>(P[s], ptab, win.next(), lane);
+        } else {
+          double row[A];
+          load_row<A>(Q + s * A, row);
+          if constexpr (kEpsTab) a = select_action_eps_tab<A>(row, ptab, win.next(), lane);
+          else a = select_action_warp<A, COBEL_POLICY_EPS_GREEDY>(row, (1u << A) - 1u, pt, win.next(), lane);
+        }
         const int sa = s * A + a;
         const int s2 = w_succ(sa);
         const double r = w_rew(s2);
@@ -191,10 +206,11 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, HBM ? 1 : 7) dynaq_warp_ker
         const double m0 = Mr[sa];
         const double m1 = xadd(m0, xmul(mlr, xsub(r, m0)));
         double row2[A];
-        load_row<A>(Q + s2 * A, row2);
+        if constexpr (!SUM) load_row<A>(Q + s2 * A, row2);
         const double q = Q[sa];
         const double g = nt ? gamma : 0.0;
-        double td = xadd(r, xmul(g, row_max<A>(row2)));
+        // SUM: s2 == s reads V[s] before the write below, as the sequential update reads the row before its write
+        double td = xadd(r, xmul(g, SUM ? V[s2] : row_max<A>(row2)));
         td = xsub(td, q);
         const double qn = xadd(q, xmul(lr, td));
         if (i == sa) { rr = m1; rs2 = s2; rnt = nt; }
@@ -204,9 +220,11 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, HBM ? 1 : 7) dynaq_warp_ker
           Mr[sa] = m1;
           m_set(sa, s2, nt);
           Q[sa] = qn;
+          // warp-uniform: 7 % of C2's online updates change Q[s,a]
+          if (SUM && __double_as_longlong(qn) != __double_as_longlong(q)) refresh_row_summary<A>(Q, V, P, s);
         }
         __syncwarp();
-        td_batch_level_parallel<A>(Q, wm, rm, S, lane, true, rs, ra, rr, rs2, rnt, lr, gamma);
+        td_batch_level_parallel<A, SUM>(Q, wm, rm, S, lane, true, rs, ra, rr, rs2, rnt, lr, gamma, nullptr, nullptr, V, P);
         win.advance(32);
         ++nsteps;
         treward = xadd(treward, r);
@@ -504,6 +522,7 @@ int launch(const CobelDynaQParams& p, cudaStream_t st) {
                      p.batch == 32 && !p.stream.user_stream;
   const AgentSmem ao(S, A, plain);
   const size_t sm = (size_t)wo.bytes + (size_t)kWarpsPerCta * ao.bytes;
+  const unsigned grid = (unsigned)((p.n_agents + kWarpsPerCta - 1) / kWarpsPerCta);
   if (sm > kMaxSmem) {
     // the tables do not fit: they stay in HBM / L2, only the dependency masks of the replay are staged
     const AgentSmem go(S, A, false, false);
@@ -526,9 +545,14 @@ int launch(const CobelDynaQParams& p, cudaStream_t st) {
       const int64_t per_cta = kPairWarps * 2;
       return launch_kernel(dynaq_pair_kernel<A>, (unsigned)((p.n_agents + per_cta - 1) / per_cta), kPairWarps * 32, smp, st, p);
     }
+    // the row summaries (9 bytes per state and agent) where they fit; otherwise the PLAIN kernel without them, so
+    // that the largest world on chip stays the same
+    const size_t sms = (size_t)wo.bytes + (size_t)kWarpsPerCta * AgentSmem(S, A, true, true, true).bytes;
+    if (plain && sms <= kMaxSmem)
+      return launch_kernel(dynaq_warp_kernel<A, true, false, true>, grid, kWarpsPerCta * 32, sms, st, p);
   }
-  return launch_kernel(plain ? dynaq_warp_kernel<A, true> : dynaq_warp_kernel<A, false>,
-                       (unsigned)((p.n_agents + kWarpsPerCta - 1) / kWarpsPerCta), kWarpsPerCta * 32, sm, st, p);
+  return launch_kernel(plain ? dynaq_warp_kernel<A, true> : dynaq_warp_kernel<A, false>, grid, kWarpsPerCta * 32, sm,
+                       st, p);
 }
 
 }  // namespace

@@ -277,14 +277,36 @@ COBEL_DEV void eps_cdf_table_init(double* tab, const PolicyTab& pt, int lane) {
   }
   __syncwarp();
 }
+// bit a set = v[a] equals the row maximum m
 template <int A>
-COBEL_DEV int select_action_eps_tab(const double (&v)[A], const double* tab, double u, int lane) {
-  const double m = row_max<A>(v);
+COBEL_DEV uint32_t tie_pattern(const double (&v)[A], double m) {
   uint32_t ties = 0;
 #pragma unroll
   for (int a = 0; a < A; ++a) ties |= (v[a] == m ? 1u : 0u) << a;
+  return ties;
+}
+template <int A>
+COBEL_DEV int select_action_eps_pattern(uint32_t ties, const double* tab, double u, int lane) {
   const double mine = tab[ties * 4 + (lane & 3)];
   return __popc(__ballot_sync(kFull, lane < A - 1 && mine <= u));
+}
+template <int A>
+COBEL_DEV int select_action_eps_tab(const double (&v)[A], const double* tab, double u, int lane) {
+  return select_action_eps_pattern<A>(tie_pattern<A>(v, row_max<A>(v)), tab, u, lane);
+}
+
+// ---------------------------------------------------------------------------
+// Row summaries of an on-chip Q table (the PLAIN Dyna-Q kernel, A <= 4): V[s] = row_max(Q[s,:]) and
+// P[s] = tie_pattern(Q[s,:]), computed with exactly the per-step operations, so reading them is bit-identical to
+// recomputing them from the row.  Whoever writes Q[s,:] refreshes them before the next warp barrier.
+// ---------------------------------------------------------------------------
+template <int A>
+COBEL_DEV void refresh_row_summary(const double* Q, double* V, uint8_t* P, int s) {
+  double row[A];
+  load_row<A>(Q + s * A, row);
+  const double m = row_max<A>(row);
+  V[s] = m;
+  P[s] = (uint8_t)tie_pattern<A>(row, m);
 }
 
 // ---------------------------------------------------------------------------
@@ -317,24 +339,36 @@ COBEL_DEV int select_action_eps_tab(const double (&v)[A], const double* tab, dou
 // `mbits` (optional) holds one byte per state with bit a set = action a may enter the max over
 // Q[s2,:] (SFMA.update_q honours the action mask, agent/sfma.py:440-449; DynaQ / QAgent do not).
 // `td_out` (optional): receives this lane's TD error (SFMA accumulates |td|, agent/sfma.py:456).
-template <int A>
+// SUM: the table keeps row summaries `V`/`P` (refresh_row_summary).  The speculative pass reads V[s2] (one LDS.64)
+// instead of the row; the rounds keep reading rows, because V is stale in the middle of a batch.  The first round's
+// commit stays exact: its read-after-write predecessors were all dropped as null, so the pre-batch V[s2] is the
+// maximum of the row it reads.  After the last round every kept lane refreshes the summaries of its row s (lanes
+// that share a state write identical values).
+template <int A, bool SUM = false>
 COBEL_DEV void td_batch_level_parallel(double* Q, uint32_t* wm, uint32_t* rm, int S, int lane, bool active,
                                        int s, int a, double r, int s2, int nt, double lr, double gamma,
-                                       const uint8_t* mbits = nullptr, double* td_out = nullptr) {
+                                       const uint8_t* mbits = nullptr, double* td_out = nullptr,
+                                       double* V = nullptr, uint8_t* P = nullptr) {
+  static_assert(!SUM || A <= 4, "row summaries hold a tie pattern of at most 4 actions");
   const double g = nt ? gamma : 0.0;
   // this lane's update on the current table: returns Q[s,a] + lr*td, sets q = Q[s,a]
-  auto evaluate = [&](double& q) -> double {
-    double row[A];
-    load_row<A>(Q + s2 * A, row);
-    q = Q[s * A + a];
+  auto evaluate = [&](double& q, bool from_summary) -> double {
     double mx;
-    if (mbits) {
-      const uint32_t mb = mbits[s2];
-      mx = -__longlong_as_double(0x7FF0000000000000ll);
-#pragma unroll
-      for (int x = 0; x < A; ++x) mx = (mb >> x & 1u) ? xmax(mx, row[x]) : mx;
+    if (SUM && from_summary) {
+      q = Q[s * A + a];
+      mx = V[s2];
     } else {
-      mx = row_max<A>(row);
+      double row[A];
+      load_row<A>(Q + s2 * A, row);
+      q = Q[s * A + a];
+      if (mbits) {
+        const uint32_t mb = mbits[s2];
+        mx = -__longlong_as_double(0x7FF0000000000000ll);
+#pragma unroll
+        for (int x = 0; x < A; ++x) mx = (mb >> x & 1u) ? xmax(mx, row[x]) : mx;
+      } else {
+        mx = row_max<A>(row);
+      }
     }
     double td = xadd(r, xmul(g, mx));
     td = xsub(td, q);
@@ -346,7 +380,7 @@ COBEL_DEV void td_batch_level_parallel(double* Q, uint32_t* wm, uint32_t* rm, in
   bool null = true;                                                 // inactive lanes count as null
   if (active) {
     double q;
-    qn = evaluate(q);
+    qn = evaluate(q, true);
     null = __double_as_longlong(qn) == __double_as_longlong(q);
   }
   unsigned bad = __ballot_sync(kFull, !null);
@@ -391,9 +425,13 @@ COBEL_DEV void td_batch_level_parallel(double* Q, uint32_t* wm, uint32_t* rm, in
     // so a lane writes straight after its reads; one barrier per round orders the rounds
     if (ready) {
       double q;
-      Q[s * A + a] = first ? qn : evaluate(q);
+      Q[s * A + a] = first ? qn : evaluate(q, false);
     }
     __syncwarp();
     done |= R;
+  }
+  if constexpr (SUM) {
+    if (bad >> lane & 1u) refresh_row_summary<A>(Q, V, P, s);
+    __syncwarp();
   }
 }
