@@ -6,8 +6,8 @@
 //
 // Mapping: ONE WARP PER AGENT, agent tables resident in shared memory for the whole launch
 // (HBM is touched once: coalesced stage-in / stage-out).  Per environment step the warp
-//   * takes the step's 34 uniforms from the agent's stream window (one Philox block per lane per refill;
-//     the PLAIN kernel keeps 256 draws in shared memory, i.e. seven steps per refill),
+//   * takes the step's 33 uniforms from the agent's stream window (one Philox block per lane per refill;
+//     the PLAIN kernel keeps a ring of 256 draws in shared memory and appends 192 per refill),
 //   * selects the action and steps the environment warp-uniformly (PLAIN: tie-pattern CDF table),
 //   * draws the 32 replay indices one per lane, gathers the 32 experiences in parallel and
 //     applies the 32 TD updates in dependency levels (td_batch_level_parallel): one speculative
@@ -65,13 +65,18 @@ struct WorldSmem {      // byte offsets of the CTA-shared environment tables
 // SUM (PLAIN, A <= 4): the agent keeps the row summaries V[s] = row_max(Q[s,:]) and P[s] = its tie pattern on chip
 // (refresh_row_summary), so the action selection, the online update's target and the replay's speculative pass read
 // one entry instead of a row and its maximum; a step that writes a row refreshes its summaries.
+// The SUM kernel runs one warp per CTA, 28 CTAs per SM: the agent's shared-memory block and its parameters
+// are then CTA-uniform, so the compiler keeps their addresses and the Philox key schedule in uniform registers instead of
+// recomputing them after every window check, and knows the warp converged (no divergence checks before collectives).
+// The world tables are staged once per agent instead of once per four.
 template <int A, bool PLAIN, bool HBM = false, bool SUM = false>
-__global__ void __launch_bounds__(kWarpsPerCta * 32, HBM ? 1 : 7) dynaq_warp_kernel(const __grid_constant__ CobelDynaQParams p) {
+__global__ void __launch_bounds__(SUM ? 32 : kWarpsPerCta * 32, HBM ? 1 : SUM ? 28 : 7)
+dynaq_warp_kernel(const __grid_constant__ CobelDynaQParams p) {
   static_assert(!(PLAIN && HBM), "the HBM path is the generic kernel");
   static_assert(!SUM || (PLAIN && A <= 4), "row summaries go with the tie-pattern table");
   extern __shared__ __align__(16) unsigned char smem[];
   const int S = p.world.n_states, K = p.world.n_starts, SA = S * A;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int lane = threadIdx.x & 31, warp = SUM ? 0 : threadIdx.x >> 5;
   const WorldSmem wo(HBM ? 0 : S, A, HBM ? 0 : K);
   constexpr bool kEpsTab = PLAIN && A <= 4;      // tie-pattern CDF table instead of per-step probabilities
   const AgentSmem ao(S, A, PLAIN, !HBM, SUM);
@@ -91,7 +96,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, HBM ? 1 : 7) dynaq_warp_ker
   auto w_term = [&](int x) -> int { if constexpr (HBM) return __ldg(p.world.terminal + x); else return term_s[x]; };
   auto w_start = [&](int k) -> int { if constexpr (HBM) return __ldg(p.world.starts + k); else return starts_s[k]; };
 
-  const int64_t n = (int64_t)blockIdx.x * blockDim.x / 32 + warp;
+  const int64_t n = SUM ? (int64_t)blockIdx.x : (int64_t)blockIdx.x * blockDim.x / 32 + warp;
   if (n >= p.n_agents) return;                      // whole warp leaves; no block-wide sync below
 
   unsigned char* blk = smem + wo.bytes + (size_t)warp * ao.bytes;
@@ -183,7 +188,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, HBM ? 1 : 7) dynaq_warp_ker
       // before the action selection and the store, so its shared-memory latency overlaps theirs, and the lane whose
       // index is the stored (s,a) takes the stored values -- what the sequential order reads.
       for (;; ++step) {
-        win.ensure(34, lane);
+        win.ensure(33, lane);                       // the action's draw and the 32 replay indices
         const int i = draw_integer(win.peek(1 + lane), SA);
         double rr = Mr[i];
         int rs2, rnt;
@@ -215,15 +220,14 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, HBM ? 1 : 7) dynaq_warp_ker
         const double qn = xadd(q, xmul(lr, td));
         if (i == sa) { rr = m1; rs2 = s2; rnt = nt; }
         const int rs = i / A, ra = i - rs * A;
-        __syncwarp();
-        if (lane == 0) {
-          Mr[sa] = m1;
-          m_set(sa, s2, nt);
-          Q[sa] = qn;
-          // warp-uniform: 7 % of C2's online updates change Q[s,a]
-          if (SUM && __double_as_longlong(qn) != __double_as_longlong(q)) refresh_row_summary<A>(Q, V, P, s);
-        }
-        __syncwarp();
+        __syncwarp();                               // every lane has read Mr, Mx (gather) and Q, V, P before the commit
+        // every lane holds the same values and writes them: no branch on the lane
+        Mr[sa] = m1;
+        m_set(sa, s2, nt);
+        Q[sa] = qn;
+        // 7 % of C2's online updates change Q[s,a]; the vote makes the branch warp-uniform for the compiler
+        if (SUM && __any_sync(kFull, __double_as_longlong(qn) != __double_as_longlong(q))) refresh_row_summary<A>(Q, V, P, s);
+        __syncwarp();                               // the commit is visible to the replay's reads
         td_batch_level_parallel<A, SUM>(Q, wm, rm, S, lane, true, rs, ra, rr, rs2, rnt, lr, gamma, nullptr, nullptr, V, P);
         win.advance(32);
         ++nsteps;
@@ -545,11 +549,12 @@ int launch(const CobelDynaQParams& p, cudaStream_t st) {
       const int64_t per_cta = kPairWarps * 2;
       return launch_kernel(dynaq_pair_kernel<A>, (unsigned)((p.n_agents + per_cta - 1) / per_cta), kPairWarps * 32, smp, st, p);
     }
-    // the row summaries (9 bytes per state and agent) where they fit; otherwise the PLAIN kernel without them, so
-    // that the largest world on chip stays the same
-    const size_t sms = (size_t)wo.bytes + (size_t)kWarpsPerCta * AgentSmem(S, A, true, true, true).bytes;
-    if (plain && sms <= kMaxSmem)
-      return launch_kernel(dynaq_warp_kernel<A, true, false, true>, grid, kWarpsPerCta * 32, sms, st, p);
+    // the row summaries (9 bytes per state and agent) where four agents' blocks and the world fit in one CTA;
+    // otherwise the PLAIN kernel without them, so that the largest world on chip stays the same
+    const int sum_bytes = AgentSmem(S, A, true, true, true).bytes;
+    if (plain && (size_t)wo.bytes + (size_t)kWarpsPerCta * sum_bytes <= kMaxSmem)
+      return launch_kernel(dynaq_warp_kernel<A, true, false, true>, (unsigned)p.n_agents, 32,
+                           (size_t)wo.bytes + sum_bytes, st, p);
   }
   return launch_kernel(plain ? dynaq_warp_kernel<A, true> : dynaq_warp_kernel<A, false>, grid, kWarpsPerCta * 32, sm,
                        st, p);

@@ -125,45 +125,58 @@ struct DrawWindowT {
 using DrawWindow = DrawWindowT<true>;
 
 // ---------------------------------------------------------------------------
-// SmemDrawWindow: the same interface over a window of kSmemDraws draws in shared memory (the PLAIN
-// kernels).  A refill costs one Philox block per lane per 64 draws whatever is consumed, and a Dyna-Q
-// step consumes 34: a 64-draw window serves one step per refill (53 % of the generated draws used), a
-// 256-draw window seven (93 %); reading a draw is one LDS.64 instead of four shuffles.
+// SmemDrawWindow: the same interface over a ring of kSmemDraws draws in shared memory (the PLAIN
+// kernels); reading a draw is one LDS.64 instead of four shuffles.  Draw k of the stream lives in slot
+// k % NDRAWS, so Philox block b (draws 2b, 2b+1) fills the aligned slot pair b % (NDRAWS/2).  A refill
+// appends the next NDRAWS - 64 draws after the last generated one: one Philox block per lane and 64
+// draws, each draw generated once (a Dyna-Q step consumes 33, so a 256-draw ring serves 5.8 steps per
+// refill).  The refill overwrites draws [gen - NDRAWS, gen - 64), all read since fewer than `need` <= 64
+// were left.  The Philox key schedule is warp-uniform and computed once, at init.
 // ---------------------------------------------------------------------------
 constexpr int kSmemDraws = 256;
 template <int NDRAWS>
 struct SmemDrawWindowT {
+  static_assert(NDRAWS % 64 == 0 && (NDRAWS & (NDRAWS - 1)) == 0, "a power of two of whole refill chunks");
+  static constexpr int kBlocks = NDRAWS / 64 - 1;   // Philox blocks per lane and refill
   uint64_t agent;
-  uint32_t key0, key1;
-  uint64_t base;          // stream index of buf[0] (even)
-  int off;                // buf slot of the next draw: k = base + off
-  int cap;                // slots filled (0 = empty)
+  uint32_t ks0[10], ks1[10];  // the key of each Philox round
+  uint64_t gen;           // stream index one past the last generated draw (even)
+  uint32_t rd;            // low 32 bits of the stream index of the next draw
   double* buf;            // [NDRAWS], 16-byte aligned, this agent's
 
   COBEL_DEV void attach(double* b) { buf = b; }
   COBEL_DEV void init(const CobelStream& s, int64_t local_agent, uint64_t k) {
     agent = (uint64_t)(s.agent_id_base + local_agent);
-    key0 = (uint32_t)s.seed; key1 = (uint32_t)(s.seed >> 32);
-    base = k; off = 0; cap = 0;
-  }
-  COBEL_DEV uint64_t position() const { return base + (uint64_t)off; }
-  COBEL_DEV void ensure(int need, int lane) {
-    if (off + need <= cap) return;
-    const uint64_t k = base + (uint64_t)off;
-    base = k & ~1ull; off = (int)(k & 1ull); cap = NDRAWS;
-    __syncwarp();                                   // every lane has read what it needed of the old window
+    const uint32_t key0 = (uint32_t)s.seed, key1 = (uint32_t)(s.seed >> 32);
 #pragma unroll
-    for (int j = 0; j < NDRAWS / 64; ++j) {
-      const uint64_t b = (base >> 1) + (uint64_t)(j * 32 + lane);
-      uint32_t o[4];
-      philox4x32_10((uint32_t)b, (uint32_t)(b >> 32), (uint32_t)agent, (uint32_t)(agent >> 32), key0, key1, o);
-      reinterpret_cast<double2*>(buf)[j * 32 + lane] = make_double2(u53(o[0], o[1]), u53(o[2], o[3]));
-    }
-    __syncwarp();
+    for (int r = 0; r < 10; ++r) { ks0[r] = key0 + (uint32_t)r * 0x9E3779B9u; ks1[r] = key1 + (uint32_t)r * 0xBB67AE85u; }
+    gen = k & ~1ull; rd = (uint32_t)k;              // nothing generated: gen - k is 0 or -1
   }
-  COBEL_DEV double peek(int ahead) const { return buf[off + ahead]; }
-  COBEL_DEV void advance(int n) { off += n; }
-  COBEL_DEV double next() { return buf[off++]; }
+  COBEL_DEV uint64_t position() const { return gen - (uint64_t)(int64_t)(int)((uint32_t)gen - rd); }
+  // make the next `need` draws available (need <= 64); warp-uniform
+  COBEL_DEV void ensure(int need, int lane) {
+    if ((int)((uint32_t)gen - rd) >= need) return;
+    __syncwarp();                                   // every lane has read the draws this refill overwrites
+    const uint64_t b0 = gen >> 1;
+#pragma unroll
+    for (int j = 0; j < kBlocks; ++j) {
+      const uint64_t b = b0 + (uint64_t)(j * 32 + lane);
+      uint32_t c0 = (uint32_t)b, c1 = (uint32_t)(b >> 32), c2 = (uint32_t)agent, c3 = (uint32_t)(agent >> 32);
+#pragma unroll
+      for (int r = 0; r < 10; ++r) {                // philox4x32_10 with the precomputed key schedule
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
+        const uint32_t n0 = hi1 ^ c1 ^ ks0[r], n2 = hi0 ^ c3 ^ ks1[r];
+        c0 = n0; c1 = lo1; c2 = n2; c3 = lo0;
+      }
+      reinterpret_cast<double2*>(buf)[(uint32_t)b & (NDRAWS / 2 - 1)] = make_double2(u53(c0, c1), u53(c2, c3));
+    }
+    gen += 64 * kBlocks;
+    __syncwarp();                                   // the new draws are visible to every lane
+  }
+  COBEL_DEV double peek(int ahead) const { return buf[(rd + (uint32_t)ahead) & (NDRAWS - 1)]; }
+  COBEL_DEV void advance(int n) { rd += (uint32_t)n; }
+  COBEL_DEV double next() { const double u = peek(0); ++rd; return u; }
 };
 using SmemDrawWindow = SmemDrawWindowT<kSmemDraws>;
 template <bool PLAIN, int NDRAWS = kSmemDraws> struct WindowFor { using type = DrawWindowT<true>; };
