@@ -33,7 +33,7 @@ class Trace(C.Structure):
     _fields_ = [('trial_steps', c_ptr), ('trial_reward', c_ptr), ('n_steps', c_ptr), ('n_replay', c_ptr),
                 ('step_sa', c_ptr), ('step_cap', C.c_int64), ('replay_idx', c_ptr), ('replay_cap', C.c_int64),
                 ('replay_len', c_ptr), ('replay_calls_cap', C.c_int64), ('flags', c_ptr), ('step_next', c_ptr),
-                ('step_td', c_ptr), ('reserved', c_ptr)]
+                ('step_td', c_ptr), ('replay_td', c_ptr)]
 
 
 class DynaQParams(C.Structure):

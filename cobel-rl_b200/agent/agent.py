@@ -11,7 +11,8 @@ agents, so per-step Python callbacks cannot run inside the loop.  What is kept:
   session into several launches;
 * per-step information is available from the recorded trajectory buffers
   (``agent.record = True`` -> ``agent.last_run``): ``step_sa``, ``step_next`` and, for the
-  Q-learning agents when the call learns, ``step_td`` (the TD error of each step's online update).
+  Q-learning agents when the call learns, ``step_td`` (the TD error of each step's online update)
+  and, when it also replays, ``replay_td`` (the TD error of each replayed update).
 This is the one intentional API deviation (SURVEY.md section 7.2).
 """
 import abc
@@ -56,6 +57,11 @@ class RunResult(dict):
     -1 behind ``n_steps``; ``replay_idx`` and ``replay_len``.  With ``agent.record`` in a call that learns (Dyna-Q,
     QAgent, SFMA, PMA ``train()``, also with ``no_replay=True``): ``step_td`` ``[N, trials*steps]`` fp64, the TD error
     that each step's online update added to ``Q[s,a]`` (scaled by the learning rate), NaN behind ``n_steps``.
+    With ``agent.record`` in a call that learns with replays (Dyna-Q, QAgent, SFMA, PMA ``train()`` without
+    ``no_replay``): ``replay_td`` fp64, shaped and aligned like ``replay_idx``: entry j is the TD error of the update
+    that applied the agent's j-th replayed experience, the value that feeds ``Q[s,a] += lr * td`` at that moment of
+    the batch.  PMA: the td of the element that ``replay_idx`` names (the last one of its n-step sequence), NaN where
+    the n-step update aborted.  SFMA: NaN for the trace-only replay at trial start.  NaN behind ``n_replay``.
     Entry k of every per-step buffer belongs to the agent's k-th step.  Every buffer keeps its leading agent axis,
     also for a single-agent stream."""
     __getattr__ = dict.__getitem__
@@ -69,7 +75,7 @@ class Agent(abc.ABC):
         self.current_trial = 0
         self.stop = False
         # batched-path extras
-        self.record = False            # record per-step (s,a), next state, TD error and replay indices of each call
+        self.record = False            # record per-step (s,a), next state, TD error, replay indices and replay TD errors
         self.trials_per_launch = None  # split a session into launches of this many trials
         self.last_run = None
         self._stream = None
@@ -102,9 +108,11 @@ class Agent(abc.ABC):
         dst.copy_(v.reshape(dst.shape) if v.numel() == dst.numel() else v.expand_as(dst))
 
     # ---- trace plumbing --------------------------------------------------------
-    def _make_trace(self, trials, steps, replay_per_step, replay_calls_per_trial, replay_len_max, keep, td=False):
+    def _make_trace(self, trials, steps, replay_per_step, replay_calls_per_trial, replay_len_max, keep, td=False,
+                    replay_td=False):
         """CobelTrace of one launch and the RunResult that owns its buffers; ``td`` = the launch performs online
-        Q updates whose TD errors are recorded (``step_td``) when ``agent.record`` is set."""
+        Q updates whose TD errors are recorded (``step_td``) when ``agent.record`` is set; ``replay_td`` = it also
+        replays, and the TD errors of the replayed updates are recorded (``replay_td``)."""
         st = self._stream
         n, dev = st.n_agents, st.device
         res = RunResult()
@@ -123,12 +131,15 @@ class Agent(abc.ABC):
             if td:
                 res['step_td'] = torch.full((n, max(step_cap, 1)), float('nan'), dtype=torch.float64, device=dev)
             res['replay_idx'] = torch.full((n, max(replay_cap, 1)), -1, dtype=torch.int32, device=dev)
+            if replay_td:
+                res['replay_td'] = torch.full((n, max(replay_cap, 1)), float('nan'), dtype=torch.float64, device=dev)
             res['replay_len'] = torch.full((n, max(calls_cap, 1)), -1, dtype=torch.int32, device=dev)
         keep.append(res)
         tr = _lib.Trace(res['trial_steps'].data_ptr(), res['trial_reward'].data_ptr(), res['n_steps'].data_ptr(),
                         res['n_replay'].data_ptr(), _lib.ptr(res.get('step_sa')), step_cap,
                         _lib.ptr(res.get('replay_idx')), replay_cap, _lib.ptr(res.get('replay_len')), calls_cap,
-                        res['flags'].data_ptr(), _lib.ptr(res.get('step_next')), _lib.ptr(res.get('step_td')))
+                        res['flags'].data_ptr(), _lib.ptr(res.get('step_next')), _lib.ptr(res.get('step_td')),
+                        _lib.ptr(res.get('replay_td')))
         return tr, res
 
     def _mask_args(self, keep):
@@ -145,7 +156,8 @@ class Agent(abc.ABC):
         ``replay_calls = (calls at trial start, calls at trial end)`` additionally fires
         ``on_replay_begin`` / ``on_replay_end`` (agent/pma.py:112-135, agent/sfma.py:139-187) with
         ``logs['replay']`` = dict of padded ``[N, L]`` tensors (flat index, state, action; -1 = no
-        experience) when the run was recorded (``agent.record``), else ``None``."""
+        experience; ``td``, the TD error of each replayed update, NaN where ``index`` is -1, when the run recorded
+        ``replay_td``) when the run was recorded (``agent.record``), else ``None``."""
         cbs = self.callbacks.custom_callbacks
         if not any(k in cbs for k in Callbacks.HOOKS):
             return
@@ -170,7 +182,11 @@ class Agent(abc.ABC):
             A = int(self.action_space.n)
             state = torch.where(valid, idx % S if flat_order == 'F' else idx // A, idx)
             action = torch.where(valid, idx // S if flat_order == 'F' else idx % A, idx)
-            return {'index': idx, 'state': state, 'action': action, 'length': ln}
+            out = {'index': idx, 'state': state, 'action': action, 'length': ln}
+            if 'replay_td' in res:
+                td = torch.gather(res['replay_td'], 1, (off.unsqueeze(1) + pos).clamp(max=res['replay_td'].shape[1] - 1))
+                out['td'] = torch.where(valid, td, torch.full_like(td, float('nan')))
+            return out
 
         for t in range(trials):
             steps_t, rew_t = res['trial_steps'][:, t], res['trial_reward'][:, t]
@@ -200,7 +216,7 @@ class Agent(abc.ABC):
     @staticmethod
     def _merge(results):
         """One RunResult for a session that ran as several launches (``trials_per_launch``).  Per-trial arrays are
-        concatenated; the recorded per-step / per-replay buffers of a launch are padded (-1, NaN for ``step_td``)
+        concatenated; the recorded per-step / per-replay buffers of a launch are padded (-1, NaN for the TD errors)
         behind the data of each agent, so they are compacted per agent (the merged buffer is addressed by cumulative
         counts, exactly like the buffer of a single launch)."""
         if len(results) == 1:
@@ -234,6 +250,8 @@ class Agent(abc.ABC):
                 out[k] = compact_cat([r[k] for r in results], [r['n_steps'] for r in results], float('nan'))
             elif k == 'replay_idx':
                 out[k] = compact_cat([r[k] for r in results], [r['n_replay'] for r in results])
+            elif k == 'replay_td':
+                out[k] = compact_cat([r[k] for r in results], [r['n_replay'] for r in results], float('nan'))
             elif k == 'replay_len':
                 out[k] = compact_cat([r[k] for r in results], [(r[k] >= 0).sum(dim=1) for r in results])
             else:

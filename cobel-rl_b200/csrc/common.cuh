@@ -182,5 +182,8 @@ int launch_kernel(void (*kernel)(Params...), dim3 grid, dim3 block, size_t smem,
 // Checks shared by the fused train()/test() entry points (util.cu).
 int cobel_validate_common(int64_t n_agents, const CobelWorld& w, const CobelStream& s, const CobelPolicy& pol,
                           const CobelTrace& tr, int trials, int steps);
+// replay_td is recorded entry for entry with replay_idx, so it needs that buffer: checked by every train()/test() entry
+// point after its other argument checks, before a zero-trial call returns (util.cu).
+int cobel_validate_replay_td(const CobelTrace& tr);
 // carry[n, 0] = state[n], carry[n, 1..stride) = 0: the per-agent state a stand-alone replay starts from (util.cu).
 int cobel_set_carry(int64_t* carry, int stride, const int32_t* state, int64_t n_agents, cudaStream_t st);

@@ -167,7 +167,15 @@ dynaq_warp_kernel(const __grid_constant__ CobelDynaQParams p) {
           else flags |= COBEL_FLAG_TRACE_OVERFLOW;
         }
       }
-      td_batch_level_parallel<A>(Q, wm, rm, S, lane, active, rs, ra, rr, rs2, rnt, lr, gamma);
+      // replay_td: the lane's sequential td -- the speculative one for the updates dropped as null or committed in the
+      // first round (their inputs are the pre-batch values), the one of its round for the others
+      double rtd = 0.0;
+      td_batch_level_parallel<A>(Q, wm, rm, S, lane, active, rs, ra, rr, rs2, rnt, lr, gamma, nullptr,
+                                 PLAIN ? nullptr : &rtd);
+      if (!PLAIN && tr.replay_td && active) {
+        if (nrep + lane < tr.replay_cap) tr.replay_td[n * tr.replay_cap + nrep + lane] = rtd;
+        else flags |= COBEL_FLAG_TRACE_OVERFLOW;
+      }
       nrep += nb;
     }
     if (!PLAIN && tr.replay_len && lane == 0) {
@@ -569,6 +577,7 @@ extern "C" int cobel_dynaq_run(const CobelDynaQParams* pp, void* stream) {
   if (rc) return rc;
   COBEL_REQUIRE(p.Q && p.Mr && p.Ms && p.Mt && p.lr && p.gamma && p.mem_lr, COBEL_EINVAL, "agent tables missing");
   COBEL_REQUIRE(p.batch >= 0, COBEL_EINVAL, "batch must be >= 0");
+  if ((rc = cobel_validate_replay_td(p.trace))) return rc;
   if (p.trials == 0) return COBEL_OK;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   COBEL_DISPATCH_A(p.world.n_actions, return launch<A>(p, st));

@@ -1404,8 +1404,13 @@ __global__ void __launch_bounds__(kMainWarps * 32, BIG ? 1 : 4) pma_main_kernel(
           ok = !__any_sync(kFull, bad);
         }
         ndst = 0;
+        // replay_td of this update (slot nrep + count of replay_idx) is the td of the sequence's last element, the
+        // experience that replay_idx names; NaN when the n-step update aborts (no element is updated then).  The
+        // elements return their td instead of storing it, so the lambda captures nothing new: capturing the trace or
+        // the counters by reference there made the compiler keep the BIG kernel's locals in a local-memory frame.
+        double last_td = __longlong_as_double(0x7FF8000000000000ll);
         if (ok) {
-          auto update_element = [&](int j) {
+          auto update_element = [&](int j) -> double {
             const int i = sq[j];
             const int a = act_of(i), s = i - a * S;
             double r = 0.0;
@@ -1416,17 +1421,26 @@ __global__ void __launch_bounds__(kMainWarps * 32, BIG ? 1 : 4) pma_main_kernel(
             td = xsub(td, q);
             Q[s * A + a] = xadd(q, xmul(lrq, td));
             dst[j] = (uint16_t)s;
+            return td;
           };
           if (opt & COBEL_PMA_OPT_ALLOW_LOOPS) {      // a sequence may revisit (s, a): in order, like the reference's loop
             if (lane == 0) {
 #pragma unroll 1
-              for (int j = 0; j < nseq5; ++j) update_element(j);
+              for (int j = 0; j < nseq5; ++j) last_td = update_element(j);
             }
           } else {                                    // the states of a sequence are distinct: one element per lane
 #pragma unroll 1
-            for (int j = lane; j < nseq5; j += 32) update_element(j);
+            for (int j = lane; j < nseq5; j += 32) last_td = update_element(j);
           }
           ndst = nseq5;
+        }
+        if constexpr (!PLAIN) {
+          // the lane that updated the last element (lane 0 for the in-order loop and for an aborted update)
+          const int owner = (ok && !(opt & COBEL_PMA_OPT_ALLOW_LOOPS)) ? (nseq5 - 1) & 31 : 0;
+          if (tr.replay_td && lane == owner) {
+            if (nrep + count < tr.replay_cap) tr.replay_td[n * tr.replay_cap + nrep + count] = last_td;
+            else flags |= COBEL_FLAG_TRACE_OVERFLOW;
+          }
         }
         ++count;
         const int cs = st_of(chosen);
@@ -1758,6 +1772,7 @@ extern "C" int cobel_pma_run(const CobelPMAParams* pp, void* stream) {
   COBEL_REQUIRE(p.batch >= 0 && p.batch <= kMaxSeq, COBEL_EUNSUPPORTED, "PMA replay batch must be in 0..%d", kMaxSeq);
   COBEL_REQUIRE(p.sr_band < 0 || (p.sr_band <= 31 && p.band_scratch), COBEL_EINVAL,
                 "sr_band must be < 0 (dense update_sr) or 0..31 with band_scratch[N, S*(2*sr_band+1)]");
+  if ((rc = cobel_validate_replay_td(p.trace))) return rc;
   if (p.trials == 0) return COBEL_OK;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   COBEL_DISPATCH_A(p.world.n_actions, return run<A>(p, st));
@@ -1765,7 +1780,8 @@ extern "C" int cobel_pma_run(const CobelPMAParams* pp, void* stream) {
 
 extern "C" int cobel_pma_replay(const CobelPMAParams* pp, const int32_t* state, int update_sr, void* stream) {
   COBEL_REQUIRE(pp != nullptr && state != nullptr, COBEL_EINVAL, "null params");
-  const CobelPMAParams& p = *pp;
+  CobelPMAParams p = *pp;
+  p.trace.replay_td = nullptr;                         // recorded by the fused train() only
   COBEL_REQUIRE(p.n_agents > 0 && p.stream.draw_count && p.trace.n_steps && p.trace.n_replay, COBEL_EINVAL, "stream / trace missing");
   COBEL_REQUIRE(p.Q && p.Mr && p.Ms && p.Mt && p.T && p.SR && p.update_mask && p.lr && p.gamma && p.mem_lr && p.lr_q &&
                 p.gamma_q && p.gamma_sr && p.pow_gamma_sr && p.pow_gamma_q && p.mem_policy.param && p.policy.param && p.carry &&

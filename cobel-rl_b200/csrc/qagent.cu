@@ -163,7 +163,13 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, HBM ? 1 : 7) q_warp_kernel(
               else flags |= COBEL_FLAG_TRACE_OVERFLOW;
             }
           }
-          td_batch_level_parallel<A>(Q, wm, rm, NK, lane, active, es, ea, er, es2, ent, lr, gamma);
+          double rtd = 0.0;                       // the update's sequential td (see dynaq.cu)
+          td_batch_level_parallel<A>(Q, wm, rm, NK, lane, active, es, ea, er, es2, ent, lr, gamma, nullptr,
+                                     PLAIN ? nullptr : &rtd);
+          if (!PLAIN && tr.replay_td && active) {
+            if (nrep + lane < tr.replay_cap) tr.replay_td[n * tr.replay_cap + nrep + lane] = rtd;
+            else flags |= COBEL_FLAG_TRACE_OVERFLOW;
+          }
           nrep += nb;
         }
         if (!PLAIN && tr.replay_len && lane == 0) {  // one replay call per step, also for batch 0 (q.py:216)
@@ -226,6 +232,7 @@ extern "C" int cobel_q_run(const CobelQParams* pp, void* stream) {
   COBEL_REQUIRE(p.Q && p.lr && p.gamma, COBEL_EINVAL, "agent tables missing");
   COBEL_REQUIRE(p.n_keys > 0 && p.n_keys <= 65535, COBEL_EINVAL, "n_keys must be in 1..65535");
   COBEL_REQUIRE(p.batch >= 0, COBEL_EINVAL, "batch must be >= 0");
+  if ((rc = cobel_validate_replay_td(p.trace))) return rc;
   if (p.trials == 0) return COBEL_OK;                  // a zero-trial session is a no-op (no log needed)
   COBEL_REQUIRE(!p.learn || (p.log && p.log_len && p.log_cap > 0), COBEL_EINVAL, "experience log missing");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);

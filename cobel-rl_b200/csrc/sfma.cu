@@ -385,11 +385,13 @@ __global__ void __launch_bounds__(256, SFMA_REPLAY_MINB) sfma_replay_kernel(cons
     for (int l = 0; l < 32 && (act >> l & 1u); ++l) tdacc = xadd(tdacc, fabs(shfl_f64(tdl, l)));
   };
   // the replayed TD updates, in order, on the Q table in HBM (agent/sfma.py:416-419); warp 0
+  // apply_batch follows log_replay, which has counted the batch: its replay_td entries start at nrep - count
   auto apply_batch = [&](int count) {
 #pragma unroll 1
     for (int e = tid; e < 2 * S; e += T) wm[e] = 0;                        // wm, rm alias R
     __syncthreads();
     if (warp == 0 && apply_updates) {
+      const int64_t at = nrep - count;
 #pragma unroll 1
       for (int b0 = 0; b0 < count; b0 += 32) {
         const bool active = b0 + lane < count;
@@ -405,6 +407,10 @@ __global__ void __launch_bounds__(256, SFMA_REPLAY_MINB) sfma_replay_kernel(cons
         td_batch_level_parallel<A>(Q, wm, rm, S, lane, active, es, ea, er, es2, ent, lr, gamma,
                                    masked ? mbits : nullptr, &tdl);
         acc_td(tdl, active);
+        if (tr.replay_td && active) {
+          if (at + b0 + lane < tr.replay_cap) tr.replay_td[n * tr.replay_cap + at + b0 + lane] = tdl;
+          else flags |= COBEL_FLAG_TRACE_OVERFLOW;
+        }
       }
     }
   };
@@ -880,6 +886,10 @@ __global__ void __launch_bounds__(256) sfma_kernel(const __grid_constant__ Cobel
           td_batch_level_parallel<A>(Q, wm, rm, S, lane, active, es, ea, er, es2, ent, lr, gamma,
                                      masked ? mbits : nullptr, &tdl);
           acc_td(tdl, active);
+          if (tr.replay_td && active) {                      // the update's slot of replay_idx
+            if (nrep + b0 + lane < tr.replay_cap) tr.replay_td[n * tr.replay_cap + nrep + b0 + lane] = tdl;
+            else flags |= COBEL_FLAG_TRACE_OVERFLOW;
+          }
         }
       }
       if (tr.replay_len && tid == 0) {
@@ -1035,6 +1045,10 @@ __global__ void __launch_bounds__(256) sfma_kernel(const __grid_constant__ Cobel
         td_batch_level_parallel<A>(Q, wm, rm, S, lane, active, es, ea, er, es2, ent, lr, gamma,
                                    masked ? mbits : nullptr, &tdl);
         acc_td(tdl, active);
+        if (tr.replay_td && active) {                        // the update's slot of replay_idx
+          if (nrep + b0 + lane < tr.replay_cap) tr.replay_td[n * tr.replay_cap + nrep + b0 + lane] = tdl;
+          else flags |= COBEL_FLAG_TRACE_OVERFLOW;
+        }
       }
     }
     if (tr.replay_len && tid == 0) {
@@ -1324,6 +1338,7 @@ extern "C" int cobel_sfma_run(const CobelSFMAParams* pp, void* stream) {
   COBEL_REQUIRE(p.carry, COBEL_EINVAL, "carry scratch missing");
   COBEL_REQUIRE(p.batch >= 0 && p.nb_replays >= 0, COBEL_EINVAL, "batch and nb_replays must be >= 0");
   COBEL_REQUIRE(p.mode >= MODE_DEFAULT && p.mode <= MODE_SWEEPING, COBEL_EINVAL, "unknown replay mode %d", p.mode);
+  if ((rc = cobel_validate_replay_td(p.trace))) return rc;
   if (p.trials == 0) return COBEL_OK;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   COBEL_DISPATCH_A(p.world.n_actions, return launch<A>(p, st));
@@ -1331,7 +1346,8 @@ extern "C" int cobel_sfma_run(const CobelSFMAParams* pp, void* stream) {
 
 extern "C" int cobel_sfma_replay(const CobelSFMAParams* pp, const int32_t* state, int apply_updates, void* stream) {
   COBEL_REQUIRE(pp != nullptr && state != nullptr, COBEL_EINVAL, "null params");
-  const CobelSFMAParams& p = *pp;
+  CobelSFMAParams p = *pp;
+  p.trace.replay_td = nullptr;                         // recorded by the fused train() only
   COBEL_REQUIRE(p.n_agents > 0 && p.stream.draw_count && p.trace.n_replay && p.trace.replay_idx && p.trace.replay_len && p.carry,
                 COBEL_EINVAL, "cobel_sfma_replay needs the stream, trace.replay_idx / replay_len / n_replay and the carry scratch");
   COBEL_REQUIRE(p.Mr && p.Ms && p.Mt && p.C && p.I && p.D, COBEL_EINVAL, "memory tables missing");

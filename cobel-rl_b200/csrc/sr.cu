@@ -464,6 +464,7 @@ extern "C" int cobel_sr_run(const CobelSRParams* pp, void* stream) {
   int rc = cobel_validate_common(p.n_agents, p.world, p.stream, p.policy, p.trace, p.trials, p.steps);
   if (rc) return rc;
   COBEL_REQUIRE(p.SR && p.rewards && p.model && p.lr && p.gamma, COBEL_EINVAL, "agent tables missing");
+  if ((rc = cobel_validate_replay_td(p.trace))) return rc;
   if (p.trials == 0) return COBEL_OK;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   COBEL_DISPATCH_A(p.world.n_actions, return launch<A>(p, st));

@@ -655,6 +655,7 @@ extern "C" int cobel_sr_compact_run(const CobelSRCompactParams* pp, void* stream
   COBEL_REQUIRE(p.SRc && p.rewards && p.model && p.visited && p.n_visited && p.lr && p.gamma, COBEL_EINVAL,
                 "agent tables missing");
   COBEL_REQUIRE(p.max_visited >= 2 && p.max_visited <= 65535, COBEL_EINVAL, "max_visited must be in 2..65535");
+  if ((rc = cobel_validate_replay_td(p.trace))) return rc;
   if (p.trials == 0) return COBEL_OK;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   COBEL_DISPATCH_A(p.world.n_actions, return launch<A>(p, st));

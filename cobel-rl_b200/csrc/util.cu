@@ -48,6 +48,11 @@ int cobel_validate_common(int64_t n_agents, const CobelWorld& w, const CobelStre
   return COBEL_OK;
 }
 
+int cobel_validate_replay_td(const CobelTrace& tr) {
+  COBEL_REQUIRE(!tr.replay_td || tr.replay_idx, COBEL_EINVAL, "trace.replay_td needs trace.replay_idx");
+  return COBEL_OK;
+}
+
 int cobel_set_carry(int64_t* carry, int stride, const int32_t* state, int64_t n_agents, cudaStream_t st) {
   return launch_kernel(set_carry_kernel, (unsigned)((n_agents + 127) / 128), 128, 0, st, carry, stride, state, n_agents);
 }

@@ -351,7 +351,9 @@ COBEL_DEV void refresh_row_summary(const double* Q, double* V, uint8_t* P, int s
 // ---------------------------------------------------------------------------
 // `mbits` (optional) holds one byte per state with bit a set = action a may enter the max over
 // Q[s2,:] (SFMA.update_q honours the action mask, agent/sfma.py:440-449; DynaQ / QAgent do not).
-// `td_out` (optional): receives this lane's TD error (SFMA accumulates |td|, agent/sfma.py:456).
+// `td_out` (optional): receives this lane's TD error, the value the sequential loop computes for its update: the
+// speculative pass writes it (exact for the dropped lanes and the first round, whose inputs are pre-batch values) and a
+// later round overwrites it (SFMA accumulates |td|, agent/sfma.py:456; the replay_td trace records it).
 // SUM: the table keeps row summaries `V`/`P` (refresh_row_summary).  The speculative pass reads V[s2] (one LDS.64)
 // instead of the row; the rounds keep reading rows, because V is stale in the middle of a batch.  The first round's
 // commit stays exact: its read-after-write predecessors were all dropped as null, so the pre-batch V[s2] is the

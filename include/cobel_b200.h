@@ -100,13 +100,19 @@ typedef struct CobelTrace {
   double*  step_td;          /* optional [N, step_cap]: TD error of the online update of every step, the value
                                 that feeds Q[s,a] += lr * td (Dyna-Q, QAgent, SFMA, PMA; ignored by the SR agents
                                 and by runs that do not learn) */
-  void*    reserved;         /* NULL.  Pads the struct to a multiple of 16 bytes: the members that follow an embedded
-                                CobelTrace keep their 16-byte alignment in the kernel parameter block, so kernels
-                                that do not read step_td compile to the same instructions as before it existed */
+  double*  replay_td;        /* optional [N, replay_cap], needs replay_idx: TD error of every replayed update, entry for
+                                entry with replay_idx, the value that feeds Q[s,a] += lr * td (cobel_dynaq_run,
+                                cobel_q_run, cobel_sfma_run, cobel_pma_run in a call that replays; PMA: the td of the
+                                element that replay_idx names in its n-step update, NaN where that update aborted).
+                                Entries of replays that update nothing (SFMA's trace-only replay at trial start) are
+                                left untouched, as are all entries in the stand-alone entry points and the SR agents:
+                                fill it with NaN to tell them apart.  NULL = not recorded.  It also pads the struct to
+                                a multiple of 16 bytes: the members that follow an embedded CobelTrace keep their
+                                16-byte alignment in the kernel parameter block */
 } CobelTrace;
 
 enum {
-  COBEL_FLAG_TRACE_OVERFLOW = 1,  /* a step_sa / step_td / replay_idx / replay_len buffer was too small */
+  COBEL_FLAG_TRACE_OVERFLOW = 1,  /* a step_sa / step_td / replay_idx / replay_td / replay_len buffer was too small */
   COBEL_FLAG_CDF_NEAR_TIE   = 2,  /* an inverse-CDF draw fell within rounding distance of a bin edge */
   COBEL_FLAG_LOG_OVERFLOW   = 4,  /* QAgent experience log full */
   COBEL_FLAG_SINGULAR       = 8,  /* PMA: (I - gamma T) pivot underflow */
